@@ -3,7 +3,7 @@
 bench.py -- MH chain-steps/sec and min-ESS/sec of the B200 engine on BASELINE.json's metric, next to the
 CPU sampler timed on the same box.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
                     [--workload NAME [--precision P] [--chains C] [--iters T]] [--no-configs] [--no-cpu]
 
 The line printed by the default invocation (the one the driver runs):
@@ -25,6 +25,9 @@ The line printed by the default invocation (the one the driver runs):
   row-sharded data mode replaying the reference-stream fixtures with the rows split over the N ranks.
 
 `--workload NAME` prints the line of that single workload (profiling, DESIGN.md tables).
+
+`--dump-outputs DIR` writes what the headline workload's last timed step computed (`dump_outputs`) as float64 .npy
+files, so that two builds can be compared output for output: inputs, seeds and step counts depend on the arguments only.
 
 Timing: W untimed warm-up steps, then K steps each bracketed by CUDA events on the launching stream, L2 flushed
 (256 MiB write) between steps outside the event pairs, barrier + synchronize on both sides, MAX over ranks.
@@ -65,17 +68,17 @@ ALGO_FLOP = {"changepoint": 350.0, "gauss2d_rw": 40.0, "gauss1000_mala": 2.0e6,
              "logistic_mala": 4.0e8, "logistic_mmala": 4.4e8, "gauss2d_pt": 40.0}
 ALGO_COMPARES = {"changepoint": 300.0}
 
-# The `configs` array of the default line: (key, workload, precision, sharding, iters/step, steps).
+# The `configs` array of the default line: (key, workload, precision, sharding, iters/step); each is timed over --steps.
 #   sharding "strong": BASELINE's total chain count split over the ranks; "weak": per-GPU count; "replica": K = 1.
 SUBCONFIGS = [
-    ("gauss2d_rw_k1", "gauss2d_rw", "f64", "replica", 10000, 5),
-    ("gauss2d_rw", "gauss2d_rw", "f64", "weak", 2000, 5),
-    ("gauss1000_mala_f64", "gauss1000_mala", "f64", "strong", 20, 5),
-    ("gauss1000_mala_tf32x3", "gauss1000_mala", "tf32x3", "strong", 20, 5),
-    ("logistic_mala_f64", "logistic_mala", "f64", "strong", 2, 4),
-    ("logistic_mala_tf32x3", "logistic_mala", "tf32x3", "strong", 4, 4),
-    ("logistic_mmala_f64", "logistic_mmala", "f64", "strong", 2, 4),
-    ("logistic_mmala_tf32x3", "logistic_mmala", "tf32x3", "strong", 4, 4),
+    ("gauss2d_rw_k1", "gauss2d_rw", "f64", "replica", 10000),
+    ("gauss2d_rw", "gauss2d_rw", "f64", "weak", 2000),
+    ("gauss1000_mala_f64", "gauss1000_mala", "f64", "strong", 20),
+    ("gauss1000_mala_tf32x3", "gauss1000_mala", "tf32x3", "strong", 20),
+    ("logistic_mala_f64", "logistic_mala", "f64", "strong", 2),
+    ("logistic_mala_tf32x3", "logistic_mala", "tf32x3", "strong", 4),
+    ("logistic_mmala_f64", "logistic_mmala", "f64", "strong", 2),
+    ("logistic_mmala_tf32x3", "logistic_mmala", "tf32x3", "strong", 4),
 ]
 
 # From the committed ncu captures (`ncu --set full`, one launch of the dominant kernel): DRAM bytes per launch and
@@ -565,9 +568,43 @@ def roofline_for(ctx, wl, precision, Kg, T, steps, kt, ms):
     return roof
 
 
-def measure(ctx, wl, precision, Kg, T, steps, warmup, burn, chain_offset, K_total, scaling, cpu_seconds=0.0, e2e=True):
+DUMP_BYTES = 60 << 20                                   # below 64 MB with the .npy headers
+
+
+def dump_outputs(out_dir, s, blk, rank, world):
+    """What the last timed step computed, as a caller of the sampler receives it: every chain's state and log-posterior
+    and the all-reduced diagnostics block, as float64 DIR/<name>.npy (DIR/<name>_rank<r>.npy on several ranks).  The
+    unused lanes of a changepoint state (cpx beyond k, cpv beyond k + 1) are 0, whatever the kernels left there, so
+    every value is finite and the shapes are fixed.  Where the per-chain arrays exceed DUMP_BYTES in all, a fixed seeded
+    sample of chains is written, their indices in chain_index.npy."""
+    if s._is_cp:
+        (k, cpx, cpv, sig), lp = s._download_state()
+        lane = np.arange(cpx.shape[1])[None, :]
+        out = {"k": k, "cpx": np.where(lane < k[:, None], cpx, 0.0), "cpv": np.where(lane <= k[:, None], cpv, 0.0),
+               "sig": sig, "logpost": lp}
+    else:
+        th, lp = s._download_state()
+        out = {"theta": th, "logpost": lp}
+    out = {n: np.asarray(a, dtype=np.float64) for n, a in out.items()}
+    diag = blk.cpu().numpy().astype(np.float64)
+    K = len(lp)
+    per_chain = sum(a.nbytes for a in out.values()) // K + 8          # + 8: its entry in chain_index
+    n = min(K, (DUMP_BYTES - diag.nbytes) // per_chain)
+    if n < K:
+        idx = np.sort(np.random.default_rng(SEED).choice(K, n, replace=False))
+        out = {name: a[idx] for name, a in out.items()}
+        out["chain_index"] = idx.astype(np.float64)
+    out["diagnostics"] = diag
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, (name if world == 1 else "%s_rank%d" % (name, rank)) + ".npy"), a)
+
+
+def measure(ctx, wl, precision, Kg, T, steps, warmup, burn, chain_offset, K_total, scaling, cpu_seconds=0.0, e2e=True,
+            dump_dir=None):
     """One workload on this rank's shard: burn-in, warm-up, `steps` timed launches (CUDA events, L2 flush between
-    them), split-chain diagnostics over the two halves of the timed region, the end-to-end leg, roofline."""
+    them), split-chain diagnostics over the two halves of the timed region, the end-to-end leg, roofline.  dump_dir:
+    dump_outputs() of the last timed step, before the roofline and end-to-end legs run the chains further."""
     torch = ctx.torch
     from riemann_b200 import _lib
     from riemann_b200.distributed import reduce_block, summarize_block, summarize_split
@@ -610,9 +647,10 @@ def measure(ctx, wl, precision, Kg, T, steps, warmup, burn, chain_offset, K_tota
     w1 = time.time()
     launches = s.launch_count - launches0
     ms = ctx.max_over_ranks(ms)
+    if dump_dir:
+        dump_outputs(dump_dir, s, blk, ctx.rank, ctx.world)
     # roofline pass: the same launches with the dominant kernel's own CUDA events
-    roof_steps = max(2, min(steps, 6))
-    ms_roof, _, _ = timed_region(roof_steps, True, False)
+    ms_roof, _, _ = timed_region(steps, True, False)
     kt = s.kernel_timing()                         # dominant kernel only: total ms / launches in the roofline pass
     s.enable_kernel_timing(False)
     ms_roof = ctx.max_over_ranks(ms_roof)
@@ -643,10 +681,10 @@ def measure(ctx, wl, precision, Kg, T, steps, warmup, burn, chain_offset, K_tota
                                                "the window is shorter than ~10 tau of the slowest functional"
                                                % (rhat, diag["steps"]) if rhat is not None else "no finite R-hat")
     if ctx.rank == 0:
-        out["roofline"] = roofline_for(ctx, wl, precision, Kg, T, roof_steps, kt, ms_roof)
+        out["roofline"] = roofline_for(ctx, wl, precision, Kg, T, steps, kt, ms_roof)
         out["roofline"]["timed_in"] = ("a second pass of %d steps (%.3f ms/step) with CUDA events around every launch of the "
                                        "kernel on the launching stream; the `value` region runs without them"
-                                       % (roof_steps, ms_roof / roof_steps))
+                                       % (steps, ms_roof / steps))
     out["_sampler"] = s
     return out
 
@@ -659,7 +697,6 @@ def run_e2e(ctx, s, T, Kg, nworld, steps):
     upload -> run -> download -> synchronize, nothing overlapped."""
     torch = ctx.torch
     from riemann_b200.pipeline import HostJobRunner
-    steps = max(4, min(steps, 10))
     if s._is_cp:
         (k, cpx, cpv, sig), _ = s._download_state()
         job = tuple(torch.from_numpy(a).pin_memory() for a in (k, cpx, cpv, sig))
@@ -873,7 +910,8 @@ def run_engine(args):
         sharding = "strong"
     Kg, off, Ktot, scaling = shard_for(ctx, wl, sharding, args.chains)
     burn = args.burn if args.burn is not None else {"changepoint": 50000}.get(wl, 2 * T)
-    head = measure(ctx, wl, args.precision, Kg, T, args.steps, args.warmup, burn, off, Ktot, scaling)
+    head = measure(ctx, wl, args.precision, Kg, T, args.steps, args.warmup, burn, off, Ktot, scaling,
+                   dump_dir=args.dump_outputs)
     s = head.pop("_sampler")
 
     ess = sokal = None
@@ -887,12 +925,12 @@ def run_engine(args):
     configs, pending_cpu = [], []
     if not single and not args.no_configs:
         only = set(args.only.split(",")) if args.only else None
-        for key, w, prec, shd, Tn, steps in SUBCONFIGS:
+        for key, w, prec, shd, Tn in SUBCONFIGS:
             if only and key not in only and w not in only:
                 continue
             Kg2, off2, Kt2, sc2 = shard_for(ctx, w, shd)
             try:
-                r = measure(ctx, w, prec, Kg2, Tn, steps, 3, 2 * Tn if shd != "replica" else 1000, off2, Kt2, sc2)
+                r = measure(ctx, w, prec, Kg2, Tn, args.steps, 3, 2 * Tn if shd != "replica" else 1000, off2, Kt2, sc2)
             except Exception as e:                       # a config that cannot run must not take the line down
                 configs.append({"key": key, "workload": w, "precision": prec, "error": "%s: %s" % (type(e).__name__, e)})
                 torch.cuda.empty_cache()
@@ -1018,7 +1056,16 @@ def main():
     ap.add_argument("--only", default=None, help="comma-separated keys / workloads of the configs array to run")
     ap.add_argument("--precision", default="f64", choices=["f64", "tf32x3", "tf32-metric"],
                     help="single workload: tf32x3 = tcgen05 tensor-core modes; tf32-metric = tcgen05 Fisher-metric GEMM")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write what the headline workload's last timed step computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the engine arm")
+    # the tree may be read-only: no bytecode caches next to the sources, in this process or the spawned CPU-arm workers
+    sys.dont_write_bytecode = True
+    os.environ["PYTHONDONTWRITEBYTECODE"] = "1"
     if args.impl == "reference":
         run_reference(args)
     else:
