@@ -108,26 +108,20 @@ __device__ __forceinline__ void shift_next(const T (&a)[Geo<GL>::EPL], T (&out)[
     }
 }
 
-// value of element e + off, off in {-1, 0, +1} chosen per chain (birth: -1 above the insertion point,
-// death: +1 from the removed element on, everything else 0); elements -1 and LANES read `pad`.
-// Two shuffles per row: the row itself and the neighbouring row the wrap-around lane reads from.
+// value of element e + off of row j (a live row, see ROW_ON), off in {-1, 0, +1} chosen per chain (birth: -1 above
+// the insertion point, death: +1 from the removed element on, everything else 0); elements -1 and LANES read `pad`.
+// Two shuffles: the row itself and the neighbouring row the wrap-around lane reads from.  One row at a time, so that
+// the caller can merge it into the proposal before the next row is shifted.
 template <int GL, typename T>
-__device__ __forceinline__ void shift_by(const T (&a)[Geo<GL>::EPL], T (&out)[Geo<GL>::EPL], T pad, int lane,
-                                         int dir, const int (&off)[Geo<GL>::EPL], int kw) {
+__device__ __forceinline__ T shift_row(const T (&a)[Geo<GL>::EPL], int j, T pad, int lane, int dir, int off) {
     constexpr int EPL = Geo<GL>::EPL;
-#pragma unroll
-    for (int j = 0; j < EPL; ++j) {
-        out[j] = a[j];
-        if (ROW_ON(j)) {
-            const int src = (lane + off[j]) & (GL - 1);
-            const T lo = (j > 0) ? a[j > 0 ? j - 1 : 0] : pad;            // row below (read by lane 0 when off = -1)
-            const T hi = (j + 1 < EPL) ? a[j + 1 < EPL ? j + 1 : j] : pad; // row above (read by lane GL-1 when off = +1)
-            const T m = __shfl_sync(0xffffffffu, a[j], src, GL);
-            const T w = __shfl_sync(0xffffffffu, (dir < 0) ? lo : hi, src, GL);
-            const bool wrap = (off[j] < 0 && lane == 0) || (off[j] > 0 && lane == GL - 1);
-            out[j] = wrap ? w : m;
-        }
-    }
+    const int src = (lane + off) & (GL - 1);
+    const T lo = (j > 0) ? a[j > 0 ? j - 1 : 0] : pad;            // row below (read by lane 0 when off = -1)
+    const T hi = (j + 1 < EPL) ? a[j + 1 < EPL ? j + 1 : j] : pad; // row above (read by lane GL-1 when off = +1)
+    const T m = __shfl_sync(0xffffffffu, a[j], src, GL);
+    const T w = __shfl_sync(0xffffffffu, (dir < 0) ? lo : hi, src, GL);
+    const bool wrap = (off < 0 && lane == 0) || (off > 0 && lane == GL - 1);
+    return wrap ? w : m;
 }
 
 // a[idx] for a per-chain element index idx in [0, LANES)
@@ -238,12 +232,16 @@ __device__ __forceinline__ void log4(int lane, double a0, double a1, double a2, 
     l3 = __shfl_sync(0xffffffffu, lres, 3, GL);
 }
 
-// which: 0 = log posterior (model.py:43-55), 1 = log likelihood, 2 = log prior
-__device__ __forceinline__ double cp_assemble(const CPParams& P, int kk, double ss, double vt, double lg, double nsig,
+// ss / sigma^2, the residual term of the likelihood (changepoint.py:118-120); taken before the logarithms of the step
+// so that their results are not live across the division
+__device__ __forceinline__ double cp_ss_over_s2(double ss, double nsig) { return __ddiv_rn(ss, __dmul_rn(nsig, nsig)); }
+
+// which: 0 = log posterior (model.py:43-55), 1 = log likelihood, 2 = log prior; sss = cp_ss_over_s2(ss, nsig)
+__device__ __forceinline__ double cp_assemble(const CPParams& P, int kk, double sss, double vt, double lg, double nsig,
                                               double log_s2, int which) {
     const double s2v = __dmul_rn(nsig, nsig);
     const int ks = kk + 1;                                     // number of steps
-    double logl = -0.5 * __dadd_rn(__fma_rn((double)P.M, log_s2, __ddiv_rn(ss, s2v)), P.Mlog2pi);   // :118-120
+    double logl = -0.5 * __dadd_rn(__fma_rn((double)P.M, log_s2, sss), P.Mlog2pi);   // :118-120
     if (isnan(logl)) logl = -INFINITY;                         // :124-125
     double lsig = (s2v < 5.562684646268003e-309) ? INFINITY : -log_s2;      // log(1/sigma^2), :148
     if (nsig < 0.0) lsig = NAN;                                // :146-147
@@ -264,12 +262,17 @@ __device__ __forceinline__ double cp_logpost_rows(const CPParams& P, const doubl
                                                   double& ss, double& vt, double& lg, double& log_s2) {
     double gp, d2, d3;
     cp_terms<GL>(P, cy, cyy, lane, kw, kk, nx, nv, nbu, true, true, true, ss, vt, gp);
+    const double sss = cp_ss_over_s2(ss, nsig);
     log4<GL>(lane, gp, __dmul_rn(nsig, nsig), 1.0, 1.0, lg, log_s2, d2, d3);
-    return cp_assemble(P, kk, ss, vt, lg, nsig, log_s2, which);
+    return cp_assemble(P, kk, sss, vt, lg, nsig, log_s2, which);
 }
 
+// resident blocks of 128 threads per SM the register allocation targets (GL = 4 and 8), DESIGN.md 4.1
 #ifndef RMN_CP_MINBLOCKS
-#define RMN_CP_MINBLOCKS 4   /* 128 regs, 16 warps/SM, no spills: best of 4, 5, 6 with the move-specific guards (gpurun r2e) */
+#define RMN_CP_MINBLOCKS 4          /* one-slice kernel (traced, injected, short or whole-wave runs) */
+#endif
+#ifndef RMN_CP_MINBLOCKS_SLICED
+#define RMN_CP_MINBLOCKS_SLICED 5   /* time-sliced kernel: 96 registers, 20 warps/SM */
 #endif
 #ifndef RMN_CP_FASTPATHS
 #define RMN_CP_FASTPATHS 1   /* move-specific paths for warps whose chains all drew the same move type */
@@ -333,12 +336,29 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
     }
     double sig = __ldcg(st.sig + c);
     double lp = __ldcg(st.lp + c);
-    double ss_c, vt_c, lg_c, ls2_c;               // pieces of lp (see cp_terms / cp_assemble)
-    cp_logpost_rows<GL>(P, cy, cyy, lane, LANES, k, cx, cv, bu, sig, 0, ss_c, vt_c, lg_c, ls2_c);
-    int nacc = 0, novf = 0;
-    double s1[NS], s2[NS];                        // lane l, slot s accumulates functional l + GL*s
+    // pieces of lp (see cp_terms / cp_assemble), one slot per chain of the block in shared memory: only the moves that
+    // leave a piece alone read them, so they take no registers across the T loop.  Every lane of a group writes the
+    // same values and reads back its own writes.
+    __shared__ double s_ss[128 / GL], s_vt[128 / GL], s_lg[128 / GL];
+    const int g = threadIdx.x / GL;
+    {
+        double ss0, vt0, lg0, ls20;
+        cp_logpost_rows<GL>(P, cy, cyy, lane, LANES, k, cx, cv, bu, sig, 0, ss0, vt0, lg0, ls20);
+        s_ss[g] = ss0; s_vt[g] = vt0; s_lg[g] = lg0;
+    }
+    // diagnostics sums: lane l, slot s holds functional l + GL*s of the chain.  They stay in shared memory for the
+    // launch (no registers across the T loop) and every sample is added to the running sum in time order, so the sums
+    // do not depend on how the launch is sliced.
+    __shared__ double s_S1[NS][128], s_S2[NS][128];
 #pragma unroll
-    for (int s = 0; s < NS; ++s) { s1[s] = 0.0; s2[s] = 0.0; }
+    for (int s = 0; s < NS; ++s) {
+        const int64_t i = (int64_t)(lane + GL * s) * K + c;
+        const bool on = lane + GL * s < RMN_CP_NDIAG;
+        s_S1[s][threadIdx.x] = on ? __ldcg(st.S1 + i) : 0.0;
+        s_S2[s][threadIdx.x] = on ? __ldcg(st.S2 + i) : 0.0;
+    }
+    __shared__ int s_nacc[128], s_novf[128];        // accept / overflow counts of the launch, one per thread
+    s_nacc[threadIdx.x] = 0; s_novf[threadIdx.x] = 0;
     const RngKey rk(seed, (uint64_t)(chain_offset + c_raw));
     const TraceSel ts{tr.first, tr.thin > 0 ? tr.thin : 1};
     const bool tracing = tr.d_k || tr.d_cpx || tr.d_cpv || tr.d_sig || tr.d_logpost;
@@ -411,6 +431,33 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
         const bool skip = RMN_CP_FASTPATHS && GUARD && (INJ || shared_mv);   // per-chain Philox mode keeps ONE instruction stream
         const bool need_xi = !skip || __any_sync(FULL, mv != 3);
 
+        // ---- birth / death: the chain-level numbers (position, heights, |J|) first, while the proposal's rows are not
+        //      yet live -- the divisions and the square root are the step's widest point
+        int kk = k, nb = 0;
+        double jarg = 1.0, hnew = 0.0;
+        bool ovf = false, td = false;
+        if (any3) {                                                     // warp-uniform
+            nb = count_below<GL>(cx, lane, k, snew, kw);                // searchsorted(cpx, s), :206
+            const double hb = elem_at<GL>(cv, nb, kw);
+            const double h1d = elem_at<GL>(cv, nrand, kw);
+            const double h2d = elem_at<GL>(cv, nrand + 1, kw);
+            // birth (changepoint.py:57,61,72-74) and death (:67-68,76-78) share one instruction
+            // stream: the operands of each division / square root are selected per chain
+            const double q1 = birth ? du / P.sqrtM : h2d / h1d;
+            const double ub = 0.5 + q1;                                 // birth: u, :61
+            const double q2 = birth ? (1.0 - ub) / ub : 1.0 / (1.0 + q1);       // birth: f^2; death: u, :68
+            const double u = birth ? ub : q2;
+            const double rr = sqrt(birth ? q2 : h1d * h2d);             // birth: f, :57; death: h, :67
+            jarg = fabs((birth ? hb : rr) / (u * (1.0 - u)));           // |J| resp. 1/|J^-1|
+            // the new height this lane holds: birth, element nb: hb / f, element nb + 1: hb f (the two are on
+            // neighbouring lanes); death, element nrand: h
+            hnew = birth ? ((lane == (nb & (GL - 1))) ? hb / rr : hb * rr) : rr;
+            ovf = (mv == 3) && birth && (k + 1 > LANES - 1);
+            td = (mv == 3) && !ovf;
+            if (!(mv == 3)) jarg = 1.0;
+            if (td) kk = birth ? k + 1 : k - 1;
+        }
+
         // normals of the block moves: rows 0,1 from this step's block, rows 2,3 (only when some chain of the
         // warp has an element there and a location / height move is being made) from a second block
         double xi[EPL];
@@ -432,9 +479,8 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
         }
 
         // ---- build the proposal by selection (the chains of a warp never diverge on mv)
-        int kk = k, nbu[EPL];
-        double nx[EPL], nv[EPL], nsig = sig, jarg = 1.0;
-        bool ovf = false;
+        int nbu[EPL];
+        double nx[EPL], nv[EPL], nsig = sig;
         const double sxk = P.sx[k];
 #pragma unroll
         for (int j = 0; j < EPL; ++j) {
@@ -447,54 +493,30 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
         }
         const double xi0 = __shfl_sync(FULL, xi[0], 0, GL);
         if (mv == 2) nsig = __dadd_rn(sig, __dmul_rn(P.ss, xi0));
-        int nb = 0;
-        if (any3) {                                                     // warp-uniform
-            nb = count_below<GL>(cx, lane, k, snew, kw);                // searchsorted(cpx, s), :206
-            const double hb = elem_at<GL>(cv, nb, kw);
-            const double h1d = elem_at<GL>(cv, nrand, kw);
-            const double h2d = elem_at<GL>(cv, nrand + 1, kw);
-            // birth (changepoint.py:57,61,72-74) and death (:67-68,76-78) share one instruction
-            // stream: the operands of each division / square root are selected per chain
-            const double q1 = birth ? du / P.sqrtM : h2d / h1d;
-            const double ub = 0.5 + q1;                                 // birth: u, :61
-            const double q2 = birth ? (1.0 - ub) / ub : 1.0 / (1.0 + q1);       // birth: f^2; death: u, :68
-            const double u = birth ? ub : q2;
-            const double rr = sqrt(birth ? q2 : h1d * h2d);             // birth: f, :57; death: h, :67
-            jarg = fabs((birth ? hb : rr) / (u * (1.0 - u)));           // |J| resp. 1/|J^-1|
-            const double hbf = hb / rr;
-            ovf = (mv == 3) && birth && (k + 1 > LANES - 1);
-            const bool td = (mv == 3) && !ovf;
-            if (!(mv == 3)) jarg = 1.0;
+        if (any3) {
             // insert / delete = every element reads its neighbour below (birth, above the insertion
             // point) or above (death, from the removed element on); other chains read themselves
             const int dir = birth ? -1 : 1;
             const int pivot = birth ? nb : nrand - 1;                   // elements <= pivot stay
-            int off[EPL];
-#pragma unroll
-            for (int j = 0; j < EPL; ++j) off[j] = (td && lane + GL * j > pivot) ? dir : 0;
-            double sx_[EPL], sv_[EPL];
-            int sb_[EPL];
-            shift_by<GL, double>(cx, sx_, 0.0, lane, dir, off, kw);
-            shift_by<GL, double>(cv, sv_, 0.0, lane, dir, off, kw);
-            shift_by<GL, int>(bu, sb_, P.M, lane, dir, off, kw);
-            if (td) {
-                kk = birth ? k + 1 : k - 1;
-#pragma unroll
-                for (int j = 0; j < EPL; ++j) {
-                    const int e = lane + GL * j;
-                    nx[j] = sx_[j]; nv[j] = sv_[j]; nbu[j] = sb_[j];
-                    if (birth) {
-                        if (e == nb) { nx[j] = snew; nv[j] = hbf; nbu[j] = bu[j]; }   // boundary searched below
-                        if (e == nb + 1) nv[j] = hb * rr;
-                    } else if (e == nrand) {
-                        nv[j] = rr;
-                    }
-                }
-            }
-            // elements beyond the new extent hold zeros (canonical padding)
 #pragma unroll
             for (int j = 0; j < EPL; ++j) {
                 const int e = lane + GL * j;
+                if (ROW_ON(j)) {                                        // rows above hold the padding: nothing moves
+                    const int off = (td && e > pivot) ? dir : 0;
+                    const double sx = shift_row<GL, double>(cx, j, 0.0, lane, dir, off);
+                    const double sv = shift_row<GL, double>(cv, j, 0.0, lane, dir, off);
+                    const int sb = shift_row<GL, int>(bu, j, P.M, lane, dir, off);
+                    if (td) { nx[j] = sx; nv[j] = sv; nbu[j] = sb; }
+                }
+                if (td) {
+                    if (birth) {
+                        if (e == nb) { nx[j] = snew; nv[j] = hnew; nbu[j] = bu[j]; }   // boundary searched below
+                        if (e == nb + 1) nv[j] = hnew;
+                    } else if (e == nrand) {
+                        nv[j] = hnew;
+                    }
+                }
+                // elements beyond the new extent hold zeros (canonical padding)
                 if (e >= kk) { nx[j] = 0.0; nbu[j] = P.M; }
                 if (e > kk) nv[j] = 0.0;
             }
@@ -522,12 +544,15 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
         // ---- log-posterior of the proposal from the pieces that changed (a sigma move: none of the three sums;
         //      a height move: ss, vt; a location move: ss, gp; birth / death: all), every fp64 log of the step in
         //      one call.  A chain whose move leaves a piece alone recomputes the cached value bit for bit.
-        double nss = ss_c, nvt = vt_c, gp = 1.0, nlg, nls2, logu, ljac;
+        double nss = 0.0, nvt = 0.0, gp = 1.0, nlg, nls2, logu, ljac;
         const bool wss = !skip || any0 || any1 || any3, wvt = !skip || any1 || any3, wgp = !skip || any0 || any3;
         cp_terms<GL>(P, cy, cyy, lane, kw, kk, nx, nv, nbu, wss, wvt, wgp, nss, nvt, gp);
+        if (!wss) nss = s_ss[g];
+        if (!wvt) nvt = s_vt[g];
+        const double sss = cp_ss_over_s2(nss, nsig);
         log4<GL>(lane, gp, __dmul_rn(nsig, nsig), uacc, jarg, nlg, nls2, logu, ljac);
-        if (!wgp) nlg = lg_c;
-        const double lpn = cp_assemble(P, kk, nss, nvt, nlg, nsig, nls2, 0);
+        if (!wgp) nlg = s_lg[g];
+        const double lpn = cp_assemble(P, kk, sss, nvt, nlg, nsig, nls2, 0);
         const double lqr = (mv == 3) ? (birth ? ljac : -ljac) : 0.0;
 
         // sampler.py:83-84 with Python's min(0, nan) == 0
@@ -537,12 +562,12 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
         trace_prop(t, lpn, acc, lqr, kk, nsig, nx, nv);
         if (acc) {
             k = kk; sig = nsig; lp = lpn;
-            ss_c = nss; vt_c = nvt; lg_c = nlg; ls2_c = nls2;
+            s_ss[g] = nss; s_vt[g] = nvt; s_lg[g] = nlg;
 #pragma unroll
             for (int j = 0; j < EPL; ++j) { cx[j] = nx[j]; cv[j] = nv[j]; bu[j] = nbu[j]; }
         }
-        nacc += acc ? 1 : 0;
-        novf += ovf ? 1 : 0;
+        if (acc) s_nacc[threadIdx.x] += 1;
+        if (ovf) s_novf[threadIdx.x] += 1;
 
         if ((step % RMN_CP_DIAG_EVERY) == 0) {              // thinned accumulation (warp-uniform)
             const int kd = __reduce_max_sync(FULL, k);      // (an accepted birth may have raised the extent)
@@ -558,8 +583,10 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
                 if (lane == (2 + q) % GL) f[(2 + q) / GL] = yq;
             }
 #pragma unroll
-            for (int s = 0; s < NS; ++s)
-                if (lane + GL * s < RMN_CP_NDIAG) { s1[s] += f[s]; s2[s] += f[s] * f[s]; }
+            for (int s = 0; s < NS; ++s) {
+                s_S1[s][threadIdx.x] = __dadd_rn(s_S1[s][threadIdx.x], f[s]);
+                s_S2[s][threadIdx.x] = __fma_rn(f[s], f[s], s_S2[s][threadIdx.x]);
+            }
         }
 
         if (live && tracing) {
@@ -591,15 +618,19 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
             st.k[c] = k;
             st.sig[c] = sig;
             st.lp[c] = lp;
-            st.dacc[c] = __ldcg(st.dacc + c) + nacc;
-            st.dovf[c] = __ldcg(st.dovf + c) + novf;
+            st.dacc[c] = __ldcg(st.dacc + c) + s_nacc[threadIdx.x];
+            st.dovf[c] = __ldcg(st.dovf + c) + s_novf[threadIdx.x];
         }
+        // the same addresses as the loads at entry, computed again: keeping them live across the T loop would cost
+        // registers the loop needs (the empty asm hides that they are equal)
+        int64_t c2 = c;
+        asm volatile("" : "+l"(c2));
 #pragma unroll
         for (int s = 0; s < NS; ++s) {
-            const int i = lane + GL * s;
-            if (i < RMN_CP_NDIAG) {
-                st.S1[(int64_t)i * K + c] = __ldcg(st.S1 + (int64_t)i * K + c) + s1[s];
-                st.S2[(int64_t)i * K + c] = __ldcg(st.S2 + (int64_t)i * K + c) + s2[s];
+            const int64_t i = (int64_t)(lane + GL * s) * K + c2;
+            if (lane + GL * s < RMN_CP_NDIAG) {
+                st.S1[i] = s_S1[s][threadIdx.x];
+                st.S2[i] = s_S2[s][threadIdx.x];
             }
         }
     }
@@ -624,14 +655,14 @@ changepoint_kernel(const __grid_constant__ CPParams P, const double* __restrict_
 }
 
 // Time-sliced form of the same run (plain Philox runs without traces).  A launch of B blocks that do not fit the SMs'
-// resident-block slots S in a whole number of waves ends with a partly filled wave (2,048 blocks on 592 slots = 3.46 waves
-// at the bench shape: 4.5 % of the launch).  Here S persistent blocks take the items (time slice j, block b), index
+// resident-block slots S in a whole number of waves ends with a partly filled wave (2,048 blocks on 740 slots = 2.77 waves
+// at the bench shape).  Here S persistent blocks take the items (time slice j, block b), index
 // j B + b, from an atomic counter in increasing order: every persistent block gets the same amount of work to within one
 // item, the state of a slice's chains travels through global memory, and a flag per chain block orders the slices of the
 // same chains (the predecessor is B >> S items earlier, so the wait is almost never taken).  Philox is keyed by
 // (step, chain), so the chains are bit-identical to the one-slice launch.
 template <int DATA, int GL, bool GUARD = true>
-__global__ void __launch_bounds__(128, (GL == 16) ? 8 : RMN_CP_MINBLOCKS)
+__global__ void __launch_bounds__(128, (GL == 16) ? 8 : RMN_CP_MINBLOCKS_SLICED)
 changepoint_sliced_kernel(const __grid_constant__ CPParams P, const double* __restrict__ gdata, CPState st,
                           int64_t K, int64_t T, int64_t step0, uint64_t seed, int64_t chain_offset, int shared_mv,
                           int nblk, int slice, int nslice, int* __restrict__ done) {
@@ -787,23 +818,31 @@ struct ChangepointSampler : SamplerImpl {
         st.S1 = (double*)p; p += align256(RMN_CP_NDIAG * K * 8);
         st.S2 = (double*)p; p += align256(RMN_CP_NDIAG * K * 8);
         RMN_CUDA(cudaMemset(ws, 0, workspace_bytes()));
-        if (use_smem && smem_bytes > 48 * 1024) {
+        if (use_smem) {
             RMN_CUDA(set_smem_attr<4>());
             RMN_CUDA(set_smem_attr<8>());
             RMN_CUDA(set_smem_attr<16>());
         }
         return RMN_OK;
     }
+    // without the attribute a kernel may take 48 KB minus its STATIC shared memory (the diagnostics sums, counts and
+    // cached pieces of cp_block: 4-7 KB) as dynamic shared memory
+    cudaError_t raise_smem(const void* kernel) const {
+        cudaFuncAttributes a{};
+        cudaError_t e = cudaFuncGetAttributes(&a, kernel);
+        if (e != cudaSuccess) return e;
+        return (smem_bytes + a.sharedSizeBytes > 48 * 1024) ? rmn_raise_dyn_smem(kernel, smem_bytes) : cudaSuccess;
+    }
     template <int GL> cudaError_t set_smem_attr() {
-        cudaError_t e = rmn_raise_dyn_smem((const void*)changepoint_kernel<false, 1, GL>, smem_bytes);
+        cudaError_t e = raise_smem((const void*)changepoint_kernel<false, 1, GL>);
         if (e != cudaSuccess) return e;
-        e = rmn_raise_dyn_smem((const void*)changepoint_kernel<true, 1, GL>, smem_bytes);
+        e = raise_smem((const void*)changepoint_kernel<true, 1, GL>);
         if (e != cudaSuccess || GL != 4) return e;
-        e = rmn_raise_dyn_smem((const void*)changepoint_kernel<false, 1, 4, false>, smem_bytes);
+        e = raise_smem((const void*)changepoint_kernel<false, 1, 4, false>);
         if (e != cudaSuccess) return e;
-        e = rmn_raise_dyn_smem((const void*)changepoint_sliced_kernel<1, 4, false>, smem_bytes);
+        e = raise_smem((const void*)changepoint_sliced_kernel<1, 4, false>);
         if (e != cudaSuccess) return e;
-        return rmn_raise_dyn_smem((const void*)changepoint_sliced_kernel<1, 4>, smem_bytes);
+        return raise_smem((const void*)changepoint_sliced_kernel<1, 4>);
     }
     unsigned grid(int gl = LANES) const { return (unsigned)((s->K * gl + 127) / 128); }
     // grid of the T-step kernel: schedule groups are aligned to global chain ids, so up to 32/gl - 1 leading
