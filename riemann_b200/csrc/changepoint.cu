@@ -171,7 +171,11 @@ __device__ __forceinline__ void cp_terms(const CPParams& P, const double* __rest
                                          const double (&nx)[Geo<GL>::EPL], const double (&nv)[Geo<GL>::EPL],
                                          const int (&nbu)[Geo<GL>::EPL], bool wss, bool wvt, bool wgp,
                                          double& ss, double& vt, double& gp) {
-    // wss / wvt / wgp are WARP-UNIFORM: which of the three sums any chain of the warp needs recomputed
+    // wss / wvt / wgp are WARP-UNIFORM: which of the three sums any chain of the warp needs recomputed.
+    // Inside a live row every lane computes its element's term; elements beyond the chain's extent (e > kk, canonical
+    // padding: cpx = 0, cpv = 0, boundary = M) contribute an exact identity instead of being branched around, so the
+    // rows are straight-line code.  Each sum starts at +0.0 and a round-to-nearest sum that starts at +0.0 is never -0.0,
+    // so adding +0.0 changes no bit of it; multiplying by 1.0 changes no bit of the product.
     constexpr int EPL = Geo<GL>::EPL;
     if (wss) {
         int pb[EPL];
@@ -179,7 +183,12 @@ __device__ __forceinline__ void cp_terms(const CPParams& P, const double* __rest
         double a = 0.0;
 #pragma unroll
         for (int j = 0; j < EPL; ++j) {
-            if (ROW_ON(j) && lane + GL * j <= kk) {
+            if (ROW_ON(j)) {
+                // taken as computed: a padding element has bu = bl = M (its predecessor is padding or the last step,
+                // whose boundary is M too), so n = 0 and s1 = s2 = +0.0 exactly, and with cpv = 0 the finite vc gives
+                // (-2 vc) s1 + s2 = +0.0 and (n vc) vc + 0.0 = +0.0.  This needs finite data: vc = -ycenter, cy[M] and
+                // cyy[M] finite.  With non-finite data the term is NaN and can turn an infinite ss into NaN; the
+                // log-likelihood is -inf either way (cp_assemble maps NaN to -inf), so no chain changes.
                 const int bu = nbu[j], bl = pb[j];
                 const double n = (double)(bu - bl);
                 const double s1 = __dsub_rn(cy[bu], cy[bl]);
@@ -197,9 +206,10 @@ __device__ __forceinline__ void cp_terms(const CPParams& P, const double* __rest
 #pragma unroll
         for (int j = 0; j < EPL; ++j) {
             const int e = lane + GL * j;
-            if (ROW_ON(j) && e <= kk) {
+            if (ROW_ON(j)) {
+                // a padding gap is 0 - 0 = 0, which would zero the product: it takes the factor 1.0 instead
                 const double gap = __dsub_rn((e < kk) ? nx[j] : P.xmax, px[j]);           // changepoint.py:142-143
-                g = __dmul_rn(g, (gap < 0.0) ? NAN : gap);
+                g = __dmul_rn(g, (e > kk) ? 1.0 : ((gap < 0.0) ? NAN : gap));
             }
         }
         gp = gprod<GL>(g);
@@ -208,11 +218,14 @@ __device__ __forceinline__ void cp_terms(const CPParams& P, const double* __rest
         double b = 0.0;
 #pragma unroll
         for (int j = 0; j < EPL; ++j) {
-            if (ROW_ON(j) && lane + GL * j <= kk) {
+            if (ROW_ON(j)) {
+                // a padding height is 0 and log(0) = -inf: the term is selected to 0.0 before it is added (and the log
+                // takes 1.0 there, so that it stays on its fast path)
+                const bool on = lane + GL * j <= kk;
                 double t = __fma_rn(-P.beta, nv[j], P.cv);                                // changepoint.py:18-19,136
-                if (!P.alpha_is_one) t = __fma_rn(P.alpha - 1.0, log(nv[j]), t);
+                if (!P.alpha_is_one) t = __fma_rn(P.alpha - 1.0, log(on ? nv[j] : 1.0), t);
                 else if (!(nv[j] > 0.0)) t = NAN;                                         // 0 * log(v<=0) is nan in numpy
-                b = __dadd_rn(b, t);
+                b = __dadd_rn(b, on ? t : 0.0);
             }
         }
         vt = gsum<GL>(b);
@@ -478,17 +491,33 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
             }
         }
 
-        // ---- build the proposal by selection (the chains of a warp never diverge on mv)
+        // ---- build the proposal by selection (the chains of a warp never diverge on mv).  Only live rows (ROW_ON) are
+        //      touched: a row above holds the canonical padding in the state and in the proposal alike (every element
+        //      of it is beyond k + 1), so its proposal IS the state's row and needs no copy.  Inside a row, per-lane
+        //      predicates select between values that are all computed (no divergent branches).
         int nbu[EPL];
         double nx[EPL], nv[EPL], nsig = sig;
-        const double sxk = P.sx[k];
 #pragma unroll
-        for (int j = 0; j < EPL; ++j) {
-            const int e = lane + GL * j;
-            nx[j] = cx[j]; nv[j] = cv[j]; nbu[j] = bu[j];
-            if (ROW_ON(j)) {
-                if (mv == 0 && e < k) nx[j] = __dadd_rn(cx[j], __dmul_rn(sxk, xi[j]));   // randomwalk.py:26, scale = 1
-                if (mv == 1 && e <= k) nv[j] = __dadd_rn(cv[j], __dmul_rn(P.sv, xi[j]));
+        for (int j = 0; j < EPL; ++j) { nx[j] = cx[j]; nv[j] = cv[j]; nbu[j] = bu[j]; }
+        if (!skip || any0) {
+            const double sxk = P.sx[k];
+#pragma unroll
+            for (int j = 0; j < EPL; ++j) {
+                const int e = lane + GL * j;
+                if (ROW_ON(j)) {
+                    const double x1 = __dadd_rn(cx[j], __dmul_rn(sxk, xi[j]));           // randomwalk.py:26, scale = 1
+                    nx[j] = (mv == 0 && e < k) ? x1 : cx[j];
+                }
+            }
+        }
+        if (!skip || any1) {
+#pragma unroll
+            for (int j = 0; j < EPL; ++j) {
+                const int e = lane + GL * j;
+                if (ROW_ON(j)) {
+                    const double v1 = __dadd_rn(cv[j], __dmul_rn(P.sv, xi[j]));
+                    nv[j] = (mv == 1 && e <= k) ? v1 : cv[j];
+                }
             }
         }
         const double xi0 = __shfl_sync(FULL, xi[0], 0, GL);
@@ -534,10 +563,10 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
 #pragma unroll
             for (int j = 0; j < EPL; ++j) {
                 const int e = lane + GL * j;
-                int sb = 0;
-                if (j < NA) sb = sa[j < NA ? j : 0];
-                else if (ROW_ON(j)) sb = upper_bound<LOGP2>(xs, P.P2, nx[j]);
-                if (moved_x && e < kk && (mv == 0 || e == nb)) nbu[j] = sb;
+                if (ROW_ON(j)) {                                        // no element of a row above moves
+                    const int sb = (j < NA) ? sa[j < NA ? j : 0] : upper_bound<LOGP2>(xs, P.P2, nx[j]);
+                    nbu[j] = (moved_x && e < kk && (mv == 0 || e == nb)) ? sb : nbu[j];
+                }
             }
         }
         if (!INJ) rA = rk.block(step + 1, (uint32_t)lane);
