@@ -2,8 +2,10 @@
 #include <stdarg.h>
 #include <stdio.h>
 #include <string.h>
+#include <algorithm>
 
 #include "common.cuh"
+#include "changepoint.cuh"
 #include <nvtx3/nvToolsExt.h>      // header-only; a no-op unless a profiler injects itself (NVTX_INJECTION64_PATH)
 
 static thread_local char g_err[1024] = "";
@@ -84,19 +86,47 @@ extern "C" int rmn_model_changepoint_create(rmn_model_t** out, int M, const doub
     for (int i = 0; i < M; ++i) mean += h_y[i];
     mean /= (double)M;
     m->ycenter = mean;
+    // run-boundary bucket table (changepoint.cuh: run_boundary): the fewest buckets, a power of two from M up to
+    // BUCKET_GMAX, in which no bucket holds more than BUCKET_W points.  Other data keeps the binary search (G = 0).
+    bool finite = true;
+    for (int i = 0; i < M; ++i) finite = finite && isfinite(h_x[i]);
+    int G = 2;
+    while (G < M) G *= 2;
+    for (std::vector<int> cnt; finite && G <= cp::BUCKET_GMAX; G *= 2) {
+        const double scale = G / (xmax - xmin), off = -xmin * scale;
+        if (!(isfinite(scale) && isfinite(off))) break;
+        cnt.assign(G, 0);
+        int C = 0;
+        for (int i = 0; i < M; ++i) C = std::max(C, ++cnt[cp::bucket_of(h_x[i], scale, off, G)]);
+        if (C <= cp::BUCKET_W) {
+            m->cp_G = G; m->cp_bscale = scale; m->cp_boff = off;
+            break;
+        }
+    }
     int p2 = 1;
     while (p2 * 2 <= M) p2 *= 2;
-    const int XP = 2 * p2;                         // x table padded with NaN (changepoint.cuh: upper_bound)
-    std::vector<double> buf((size_t)XP + 2 * (size_t)M + 2, NAN);
+    const int XP = 2 * p2;                         // x table padded with NaN (changepoint.cuh: run_boundary)
+    std::vector<double> buf((size_t)XP + 2 * (size_t)M + 2 + (size_t)m->cp_G * 5 / 2, NAN);
     double* x = buf.data();
-    double* cy = x + XP;
-    double* cyy = cy + M + 1;
-    cy[0] = 0.0; cyy[0] = 0.0;
+    double* cyc = x + XP;                          // {cy, cyy} pairs
+    cyc[0] = 0.0; cyc[1] = 0.0;
     for (int i = 0; i < M; ++i) {
         x[i] = h_x[i];
         const double r = h_y[i] - mean;
-        cy[i + 1] = cy[i] + r;
-        cyy[i + 1] = cyy[i] + r * r;
+        cyc[2 * i + 2] = cyc[2 * i] + r;
+        cyc[2 * i + 3] = cyc[2 * i + 1] + r * r;
+    }
+    if (m->cp_G > 0) {
+        // bx[b] = {x[s], x[s + 1]}, bstart[b] = s = min(#{i : bucket(x_i) < b}, XP - 2)
+        double* bx = cyc + 2 * (size_t)M + 2;
+        std::vector<int> bstart(m->cp_G);
+        for (int b = 0, i = 0; b < m->cp_G; ++b) {
+            while (i < M && cp::bucket_of(h_x[i], m->cp_bscale, m->cp_boff, m->cp_G) < b) ++i;
+            bstart[b] = std::min(i, XP - 2);
+            bx[2 * b] = x[bstart[b]];
+            bx[2 * b + 1] = x[bstart[b] + 1];
+        }
+        memcpy(bx + 2 * (size_t)m->cp_G, bstart.data(), bstart.size() * sizeof(int));
     }
     cudaGetDevice(&m->device);
     if (cudaMalloc(&m->d_cpdata, buf.size() * 8) != cudaSuccess ||

@@ -13,10 +13,11 @@
 // Likelihood: x is sorted, so the prediction is constant on runs of data points; with
 // prefix sums cy[i] = sum_{m<i} (y_m - c), cyy[i] = sum_{m<i} (y_m - c)^2 the residual
 // sum of squares of segment j is  n_j (v_j-c)^2 - 2 (v_j-c) S1_j + S2_j,  where the run
-// boundaries b_j = #{x_i <= cpx_j} come from a branch-free binary search (equivalent to
-// np.searchsorted(cpx, x), changepoint.py:181).  O(k log M) instead of O(M) per
-// evaluation; all arithmetic fp64 like the reference.  x/cy/cyy are staged in shared
-// memory once per block and reused by all chains and all T iterations.
+// boundaries b_j = #{x_i <= cpx_j} come from a bucket table or a branch-free binary search
+// (changepoint.cuh: run_boundary; equivalent to np.searchsorted(cpx, x), changepoint.py:181).
+// O(k) or O(k log M) instead of O(M) per evaluation; all arithmetic fp64 like the reference.
+// The data tables are staged in shared memory once per block and reused by all chains and
+// all T iterations.
 //
 // Reference behaviours reproduced (SURVEY.md appendix A 10-12): k = number of STEPS in
 // the three k-terms of the prior; constraints enforced only through nan/inf -> -inf;
@@ -166,8 +167,7 @@ __device__ __forceinline__ int count_below(const double (&cx)[Geo<GL>::EPL], int
 // relative (tests: 1e-9).
 // ---------------------------------------------------------------------------------------
 template <int GL>
-__device__ __forceinline__ void cp_terms(const CPParams& P, const double* __restrict__ cy,
-                                         const double* __restrict__ cyy, int lane, int kw, int kk,
+__device__ __forceinline__ void cp_terms(const CPParams& P, const double2* __restrict__ cyc, int lane, int kw, int kk,
                                          const double (&nx)[Geo<GL>::EPL], const double (&nv)[Geo<GL>::EPL],
                                          const int (&nbu)[Geo<GL>::EPL], bool wss, bool wvt, bool wgp,
                                          double& ss, double& vt, double& gp) {
@@ -191,8 +191,9 @@ __device__ __forceinline__ void cp_terms(const CPParams& P, const double* __rest
                 // log-likelihood is -inf either way (cp_assemble maps NaN to -inf), so no chain changes.
                 const int bu = nbu[j], bl = pb[j];
                 const double n = (double)(bu - bl);
-                const double s1 = __dsub_rn(cy[bu], cy[bl]);
-                const double s2 = __dsub_rn(cyy[bu], cyy[bl]);
+                const double2 pu = cyc[bu], pl = cyc[bl];                                 // {cy, cyy}: one load each
+                const double s1 = __dsub_rn(pu.x, pl.x);
+                const double s2 = __dsub_rn(pu.y, pl.y);
                 const double vc = __dsub_rn(nv[j], P.ycenter);
                 a = __dadd_rn(a, __fma_rn(__dmul_rn(n, vc), vc, __fma_rn(-2.0 * vc, s1, s2)));   // n vc^2 - 2 vc s1 + s2
             }
@@ -268,13 +269,13 @@ __device__ __forceinline__ double cp_assemble(const CPParams& P, int kk, double 
 
 // full evaluation (pointwise entry, state caches at kernel entry)
 template <int GL>
-__device__ __forceinline__ double cp_logpost_rows(const CPParams& P, const double* __restrict__ cy,
-                                                  const double* __restrict__ cyy, int lane, int kw, int kk,
+__device__ __forceinline__ double cp_logpost_rows(const CPParams& P, const double2* __restrict__ cyc, int lane,
+                                                  int kw, int kk,
                                                   const double (&nx)[Geo<GL>::EPL], const double (&nv)[Geo<GL>::EPL],
                                                   const int (&nbu)[Geo<GL>::EPL], double nsig, int which,
                                                   double& ss, double& vt, double& lg, double& log_s2) {
     double gp, d2, d3;
-    cp_terms<GL>(P, cy, cyy, lane, kw, kk, nx, nv, nbu, true, true, true, ss, vt, gp);
+    cp_terms<GL>(P, cyc, lane, kw, kk, nx, nv, nbu, true, true, true, ss, vt, gp);
     const double sss = cp_ss_over_s2(ss, nsig);
     log4<GL>(lane, gp, __dmul_rn(nsig, nsig), 1.0, 1.0, lg, log_s2, d2, d3);
     return cp_assemble(P, kk, sss, vt, lg, nsig, log_s2, which);
@@ -326,9 +327,9 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
     constexpr int NS = Geo<GL>::NS;
     constexpr int CPW = 32 / GL;                  // chains per warp = chains per schedule group
     constexpr unsigned FULL = 0xffffffffu;
-    constexpr int LOGP2 = (DATA == 2) ? 6 : -1;
-    const double* cy = xs + P.XP;
-    const double* cyy = cy + P.M + 1;
+    constexpr bool BUCKETS = (DATA == 2);
+    const double2* cyc = (const double2*)(xs + P.XP);
+    const double2* bx = cyc + P.M + 1;                // bucket table (P.G > 0)
 
     const int lane = threadIdx.x & (GL - 1);
     // schedule groups are aligned to GLOBAL chain ids: `head` leading groups of the grid are dead
@@ -345,7 +346,7 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
         const int e = lane + GL * j;
         cx[j] = __ldcg(st.cpx + c * LANES + e);
         cv[j] = __ldcg(st.cpv + c * LANES + e);
-        bu[j] = (e < k) ? upper_bound<LOGP2>(xs, P.P2, cx[j]) : P.M;
+        bu[j] = (e < k) ? run_boundary<BUCKETS>(P, xs, bx, cx[j]) : P.M;
     }
     double sig = __ldcg(st.sig + c);
     double lp = __ldcg(st.lp + c);
@@ -356,7 +357,7 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
     const int g = threadIdx.x / GL;
     {
         double ss0, vt0, lg0, ls20;
-        cp_logpost_rows<GL>(P, cy, cyy, lane, LANES, k, cx, cv, bu, sig, 0, ss0, vt0, lg0, ls20);
+        cp_logpost_rows<GL>(P, cyc, lane, __reduce_max_sync(FULL, k), k, cx, cv, bu, sig, 0, ss0, vt0, lg0, ls20);
         s_ss[g] = ss0; s_vt[g] = vt0; s_lg[g] = lg0;
     }
     // diagnostics sums: lane l, slot s holds functional l + GL*s of the chain.  They stay in shared memory for the
@@ -559,12 +560,12 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
             int sa[NA];
 #pragma unroll
             for (int j = 0; j < NA; ++j) qa[j] = nx[j];
-            upper_bound_rows<LOGP2, NA>(xs, P.P2, qa, sa);
+            run_boundary<BUCKETS, NA>(P, xs, bx, qa, sa);
 #pragma unroll
             for (int j = 0; j < EPL; ++j) {
                 const int e = lane + GL * j;
                 if (ROW_ON(j)) {                                        // no element of a row above moves
-                    const int sb = (j < NA) ? sa[j < NA ? j : 0] : upper_bound<LOGP2>(xs, P.P2, nx[j]);
+                    const int sb = (j < NA) ? sa[j < NA ? j : 0] : run_boundary<BUCKETS>(P, xs, bx, nx[j]);
                     nbu[j] = (moved_x && e < kk && (mv == 0 || e == nb)) ? sb : nbu[j];
                 }
             }
@@ -575,7 +576,7 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
         //      one call.  A chain whose move leaves a piece alone recomputes the cached value bit for bit.
         double nss = 0.0, nvt = 0.0, gp = 1.0, nlg, nls2, logu, ljac;
         const bool wss = !skip || any0 || any1 || any3, wvt = !skip || any1 || any3, wgp = !skip || any0 || any3;
-        cp_terms<GL>(P, cy, cyy, lane, kw, kk, nx, nv, nbu, wss, wvt, wgp, nss, nvt, gp);
+        cp_terms<GL>(P, cyc, lane, kw, kk, nx, nv, nbu, wss, wvt, wgp, nss, nvt, gp);
         if (!wss) nss = s_ss[g];
         if (!wvt) nvt = s_vt[g];
         const double sss = cp_ss_over_s2(nss, nsig);
@@ -666,7 +667,8 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
 }
 
 // DATA: 0 = data tables read from global memory (too large for shared memory), 1 = staged in shared
-// memory, 2 = staged and 64 <= M < 128 (P2 = 64: fully unrolled 7-level search; the bench shape)
+// memory, 2 = staged with the bucket table (P.G > 0: run_boundary's lookup; the bench data).  The table exists only for
+// M <= BUCKET_GMAX, so its data is always staged.
 template <bool INJ, int DATA, int GL, bool GUARD = true>
 __global__ void __launch_bounds__(128, (GL == 16) ? 8 : RMN_CP_MINBLOCKS)
 changepoint_kernel(const __grid_constant__ CPParams P, const double* __restrict__ gdata, CPState st,
@@ -675,7 +677,7 @@ changepoint_kernel(const __grid_constant__ CPParams P, const double* __restrict_
     extern __shared__ double smem[];
     const double* xs = gdata;
     if (DATA != 0) {
-        const int n = P.XP + 2 * P.M + 2;
+        const int n = P.XP + 2 * P.M + 2 + ((DATA == 2) ? P.G * 5 / 2 : 0);
         for (int i = threadIdx.x; i < n; i += blockDim.x) smem[i] = gdata[i];
         __syncthreads();
         xs = smem;
@@ -698,7 +700,7 @@ changepoint_sliced_kernel(const __grid_constant__ CPParams P, const double* __re
     extern __shared__ double smem[];
     const double* xs = gdata;
     if (DATA != 0) {
-        const int n = P.XP + 2 * P.M + 2;
+        const int n = P.XP + 2 * P.M + 2 + ((DATA == 2) ? P.G * 5 / 2 : 0);
         for (int i = threadIdx.x; i < n; i += blockDim.x) smem[i] = gdata[i];
         __syncthreads();
         xs = smem;
@@ -743,16 +745,17 @@ cp_eval_kernel(const __grid_constant__ CPParams P, const double* __restrict__ gd
     const bool live = c_raw < n;
     const int64_t c = live ? c_raw : n - 1;
     const double* xs = gdata;
-    const double* cy = xs + P.XP;
-    const double* cyy = cy + P.M + 1;
+    const double2* cyc = (const double2*)(xs + P.XP);
+    const double2* bx = cyc + P.M + 1;                // bucket table (P.G > 0)
     const int k = kin[c];
     const int kw = LANES;                                        // every row on
     double x1[1] = {cpx[c * LANES + lane]}, v1[1] = {cpv[c * LANES + lane]};
-    int b1[1] = {(lane < k) ? upper_bound<-1>(xs, P.P2, x1[0]) : P.M};
+    int b1[1] = {P.M};
+    if (lane < k) b1[0] = P.G ? run_boundary<true>(P, xs, bx, x1[0]) : run_boundary<false>(P, xs, bx, x1[0]);
     if (lane >= k) x1[0] = 0.0;
     if (lane > k) v1[0] = 0.0;
     double ss, vt, lg, ls2;
-    const double v = cp_logpost_rows<GL>(P, cy, cyy, lane, kw, k, x1, v1, b1, sig[c], which, ss, vt, lg, ls2);
+    const double v = cp_logpost_rows<GL>(P, cyc, lane, kw, k, x1, v1, b1, sig[c], which, ss, vt, lg, ls2);
     if (live && lane == 0) out[c] = v;
 }
 
@@ -781,6 +784,7 @@ static CPParams make_params(const rmn_model* m, const rmn_proposal* p) {
     while (p2 * 2 <= m->M) p2 *= 2;
     P.P2 = (m->M >= 1) ? p2 : 0;
     P.XP = 2 * P.P2;
+    P.G = m->cp_G; P.bscale = m->cp_bscale; P.boff = m->cp_boff;
     P.alpha_is_one = (m->alpha == 1.0);
     P.xmin = m->xmin; P.xmax = m->xmax; P.alpha = m->alpha; P.beta = m->beta;
     P.cv = m->cv;
@@ -826,8 +830,9 @@ struct ChangepointSampler : SamplerImpl {
         if (const char* e = getenv("RMN_CP_SCHEDULE")) shared_mv = (e[0] == 'c' || e[0] == '0') ? 0 : 1;
         if (const char* e = getenv("RMN_CP_SLICED")) sliced = (e[0] == '0') ? 0 : 1;
         if (const char* e = getenv("RMN_CP_GUARD")) force_guard = (e[0] == '1') ? 1 : 0;
-        smem_bytes = (size_t)(P.XP + 2 * P.M + 2) * 8;
-        use_smem = smem_bytes <= 96 * 1024;
+        const size_t tables = (size_t)(P.XP + 2 * P.M + 2) * 8;
+        smem_bytes = tables + (size_t)P.G * 20;     // the bucket table is staged with the data
+        use_smem = tables <= 96 * 1024;
     }
     size_t workspace_bytes() const override {
         const size_t K = (size_t)s->K;
@@ -862,16 +867,18 @@ struct ChangepointSampler : SamplerImpl {
         if (e != cudaSuccess) return e;
         return (smem_bytes + a.sharedSizeBytes > 48 * 1024) ? rmn_raise_dyn_smem(kernel, smem_bytes) : cudaSuccess;
     }
-    template <int GL> cudaError_t set_smem_attr() {
-        cudaError_t e = raise_smem((const void*)changepoint_kernel<false, 1, GL>);
+    // the staged kernels this data launches: DATA = 2 with the bucket table, 1 without
+    template <int GL> cudaError_t set_smem_attr() { return (P.G > 0) ? set_smem_attr<2, GL>() : set_smem_attr<1, GL>(); }
+    template <int DATA, int GL> cudaError_t set_smem_attr() {
+        cudaError_t e = raise_smem((const void*)changepoint_kernel<false, DATA, GL>);
         if (e != cudaSuccess) return e;
-        e = raise_smem((const void*)changepoint_kernel<true, 1, GL>);
+        e = raise_smem((const void*)changepoint_kernel<true, DATA, GL>);
         if (e != cudaSuccess || GL != 4) return e;
-        e = raise_smem((const void*)changepoint_kernel<false, 1, 4, false>);
+        e = raise_smem((const void*)changepoint_kernel<false, DATA, 4, false>);
         if (e != cudaSuccess) return e;
-        e = raise_smem((const void*)changepoint_sliced_kernel<1, 4, false>);
+        e = raise_smem((const void*)changepoint_sliced_kernel<DATA, 4, false>);
         if (e != cudaSuccess) return e;
-        return raise_smem((const void*)changepoint_sliced_kernel<1, 4>);
+        return raise_smem((const void*)changepoint_sliced_kernel<DATA, 4>);
     }
     unsigned grid(int gl = LANES) const { return (unsigned)((s->K * gl + 127) / 128); }
     // grid of the T-step kernel: schedule groups are aligned to global chain ids, so up to 32/gl - 1 leading
@@ -975,10 +982,10 @@ struct ChangepointSampler : SamplerImpl {
         const bool traced = t0.d_k || t0.d_cpx || t0.d_cpv || t0.d_sig || t0.d_logpost || t0.d_prop_logpost || t0.d_accepted ||
                             t0.d_logqratio || t0.d_prop_k || t0.d_prop_sig || t0.d_prop_cpx || t0.d_prop_cpv;
         if constexpr (!INJ && GL == 4) {
-            if (!traced && use_smem && P.P2 == 64) { if (launch_sliced<2, GL, GUARD>(T, g, sh, smem_bytes, stream)) return; }
+            if (!traced && use_smem && P.G > 0) { if (launch_sliced<2, GL, GUARD>(T, g, sh, smem_bytes, stream)) return; }
             else if (!traced && use_smem) { if (launch_sliced<1, GL, GUARD>(T, g, sh, smem_bytes, stream)) return; }
         }
-        if (use_smem && P.P2 == 64)
+        if (use_smem && P.G > 0)
             changepoint_kernel<INJ, 2, GL, GUARD><<<g, 128, smem_bytes, stream>>>(
                 P, s->model->d_cpdata, st, s->K, T, step0, s->seed, s->chain_offset, tape, t0, sh);
         else if (use_smem)

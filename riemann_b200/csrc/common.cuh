@@ -168,7 +168,9 @@ struct rmn_model {
     // changepoint
     int M = 0, kmax = 0;
     double xmin = 0, xmax = 0, lamb = 0, alpha = 0, beta = 0, ycenter = 0;
-    double* d_cpdata = nullptr;          // x[M] | cy[M+1] | cyy[M+1]
+    double* d_cpdata = nullptr;          // x[XP] | {cy, cyy}[M+1] | bucket table int32[cp_G] (changepoint.cuh: CPParams)
+    int cp_G = 0;                        // buckets of the run-boundary table, 0 = none
+    double cp_bscale = 0, cp_boff = 0;
     double tabA[RMN_CP_LANES + 1];       // k log lam - gammaln(k) - lam + gammaln(2k+1), k = #steps
     double cv = 0.0;                     // alpha log beta - gammaln(alpha)
     // logistic

@@ -18,7 +18,7 @@ ANCHORS = {
     "common.cuh": [("__device__ __forceinline__ uint4 philox4x32_10", "Philox4x32-10 rounds"),
                    ("// uniform on (0,1): (x + 0.5)", "Box-Muller normals / uniforms"),
                    ("// Metropolis-Hastings accept rule", "accept rule helpers")],
-    "changepoint.cuh": [("template <int LOGP2>", "binary search of the x table"),
+    "changepoint.cuh": [("// #{i : x_i <= c}", "run boundaries (bucket table / binary search)"),
                         ("// uniform on (0,1) from 32 random bits", "fast uniforms")],
     "changepoint.cu": [("__device__ __forceinline__ unsigned gballot", "group ballot / butterfly sums"),
                        ("// value of element e-1 for every row", "shift_prev / shift_next (neighbour element)"),
