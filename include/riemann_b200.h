@@ -165,7 +165,9 @@ typedef struct {
     const double* d_u;
     const double* d_tape;
     const double* d_usel;   /* tempered samplers: swap-selection uniforms usel[t*K + c] (ptsampler.py:104);
-                             * d_u then holds the accept uniform of a within-chain step or the swap uniform (:121) */
+                             * d_u then holds the accept uniform of a within-chain step or the swap uniform (:121);
+                             * on the changepoint model the tape's RMN_CP_SLOT_ACC slot does, for a swap initiator the
+                             * swap uniform (the other slots of a swap participant's row are not read) */
 } rmn_inject_t;
 
 /* Optional trace.  History index i = 0 is the state at entry, i = t+1 the state after
@@ -232,11 +234,13 @@ int rmn_sampler_destroy(rmn_sampler_t* s);
 /* AdaptCovProposal.L of every chain: d_L[K][d][d] (lower triangular). */
 int rmn_sampler_get_adaptcov(rmn_sampler_t* s, double* d_L, void* stream);
 
-/* PTSampler (riemann/samplers/ptsampler.py:41-127) on the Gaussian models (small-d and dense path, f64) and the logistic
- * model (any precision; the prior is not tempered): chains c = l*nt + i form ladder l,
+/* PTSampler (riemann/samplers/ptsampler.py:41-127) on the Gaussian models (small-d and dense path, f64), the logistic
+ * model (any precision; the prior is not tempered) and the changepoint model (ChangepointRegression1DProp; a ladder
+ * lives inside one warp, so nt <= 8 there; the prior is not tempered): chains c = l*nt + i form ladder l,
  * chain i of a ladder samples TemperedModel(model, h_betas[i]) (likelihood * beta, :33-34); every step each chain either
  * takes a within-chain MH step or, with probability pswap and sequentially along the ladder exactly as :102-125,
- * proposes a swap with its lower neighbour.  K must be a multiple of nt (2..32); non-adaptive RW / pCN proposals.
+ * proposes a swap with its lower neighbour.  K and chain_offset must be multiples of nt (2..32, 2..8 on the changepoint
+ * model); non-adaptive RW / pCN proposals, or the changepoint proposal.
  * Call before rmn_sampler_set_state. */
 int rmn_sampler_set_tempering(rmn_sampler_t* s, int nt, const double* h_betas, double pswap);
 

@@ -314,13 +314,25 @@ __device__ __forceinline__ double cp_logpost_rows(const CPParams& P, const doubl
 //   cpx move    :48-50                      searches, residual sums, gap product; height-prior sum cached
 //   birth/death :57-71                      the general path
 // ---------------------------------------------------------------------------------------
+// Parallel tempering (rmn_sampler_set_tempering, ptsampler.py:41-127): chains c = l*nt + i form ladder l, rung i samples
+// log_prior + betas[i] * log_likelihood.  Given only to cp_tempered_kernel; see there for the layout.
+struct CPTemper {
+    double betas[8];
+    double pswap;
+    int nt;                     // temperatures, 2..8
+    int S;                      // groups a ladder occupies: the power of two >= nt
+};
+
 // GUARD = false: the instantiation for per-chain move schedules in Philox mode -- the warp executes the union of the
 // moves every step, so the votes and the guards that a uniform warp would use are compiled out (same arithmetic, same bits).
-template <bool INJ, int DATA, int GL, bool GUARD>
+// TEMPER: the ladder layout and the swap moves of cp_tempered_kernel (tp, usel_tape); every addition sits under
+// `if constexpr`, so the untempered instantiations are unchanged.
+template <bool INJ, int DATA, int GL, bool GUARD, bool TEMPER = false>
 __device__ __forceinline__ void cp_block(const CPParams& P, const double* __restrict__ xs, CPState st,
                                          int64_t K, int64_t t_begin, int64_t t_end, int64_t step0, uint64_t seed,
                                          int64_t chain_offset, const double* __restrict__ tape, const rmn_trace_t& tr,
-                                         int shared_mv, int64_t blk) {
+                                         int shared_mv, int64_t blk, const CPTemper* tp = nullptr,
+                                         const double* __restrict__ usel_tape = nullptr) {
     // iterations [t_begin, t_end) of the launch for the 128 / GL chains of block `blk`; the chain state is read from and
     // written back to global memory (L2-coherent loads: in the time-sliced kernel another SM wrote it)
     constexpr int EPL = Geo<GL>::EPL;
@@ -332,11 +344,28 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
     const double2* bx = cyc + P.M + 1;                // bucket table (P.G > 0)
 
     const int lane = threadIdx.x & (GL - 1);
-    // schedule groups are aligned to GLOBAL chain ids: `head` leading groups of the grid are dead
-    const int head = shared_mv ? (int)(chain_offset & (CPW - 1)) : 0;
-    const int64_t c_raw = (blk * (int64_t)blockDim.x + threadIdx.x) / GL - head;
-    const bool live = c_raw >= 0 && c_raw < K;
-    const int64_t c = c_raw < 0 ? 0 : (c_raw < K ? c_raw : K - 1);   // dead groups shadow a live chain, never store
+    int64_t c_raw, c;
+    bool live;
+    int ti = 0;                                       // tempered: this group's rung
+    if constexpr (TEMPER) {
+        // ladder slot q of the grid = S consecutive groups of one warp, rung ti = group index within the slot; with a
+        // shared move schedule the warp's CPW / S ladders are aligned to GLOBAL ladder ids (`head` dead leading slots)
+        const int64_t L = K / tp->nt;
+        const int head = shared_mv ? (int)((chain_offset / tp->nt) & (CPW / tp->S - 1)) : 0;
+        const int64_t grp = (blk * (int64_t)blockDim.x + threadIdx.x) / GL;
+        const int64_t lad = grp / tp->S - head;
+        ti = (int)(grp & (tp->S - 1));
+        live = lad >= 0 && lad < L && ti < tp->nt;
+        c_raw = lad * tp->nt + ti;                    // global id chain_offset + c_raw keys Philox
+        // dead slots and idle rungs (ti >= nt) shadow a live chain for the shuffles and never store
+        c = (lad < 0 ? 0 : (lad < L ? lad : L - 1)) * tp->nt + min(ti, tp->nt - 1);
+    } else {
+        // schedule groups are aligned to GLOBAL chain ids: `head` leading groups of the grid are dead
+        const int head = shared_mv ? (int)(chain_offset & (CPW - 1)) : 0;
+        c_raw = (blk * (int64_t)blockDim.x + threadIdx.x) / GL - head;
+        live = c_raw >= 0 && c_raw < K;
+        c = c_raw < 0 ? 0 : (c_raw < K ? c_raw : K - 1);   // dead groups shadow a live chain, never store
+    }
 
     int k = __ldcg(st.k + c);
     double cx[EPL], cv[EPL];
@@ -354,12 +383,21 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
     // leave a piece alone read them, so they take no registers across the T loop.  Every lane of a group writes the
     // same values and reads back its own writes.
     __shared__ double s_ss[128 / GL], s_vt[128 / GL], s_lg[128 / GL];
+    // tempered: the untempered log-likelihood and log-prior of the state, which the swap test reads for both partners
+    __shared__ double s_ll[TEMPER ? 128 / GL : 1], s_lpr[TEMPER ? 128 / GL : 1];
     const int g = threadIdx.x / GL;
     {
         double ss0, vt0, lg0, ls20;
-        cp_logpost_rows<GL>(P, cyc, lane, __reduce_max_sync(FULL, k), k, cx, cv, bu, sig, 0, ss0, vt0, lg0, ls20);
+        const double v0 = cp_logpost_rows<GL>(P, cyc, lane, __reduce_max_sync(FULL, k), k, cx, cv, bu, sig, TEMPER ? 1 : 0,
+                                              ss0, vt0, lg0, ls20);
         s_ss[g] = ss0; s_vt[g] = vt0; s_lg[g] = lg0;
+        if constexpr (TEMPER) {
+            s_ll[g] = v0;
+            s_lpr[g] = cp_assemble(P, k, cp_ss_over_s2(ss0, sig), vt0, lg0, sig, ls20, 2);
+        }
     }
+    double beta = 1.0;                                // this rung's inverse temperature
+    if constexpr (TEMPER) beta = tp->betas[min(ti, tp->nt - 1)];
     // diagnostics sums: lane l, slot s holds functional l + GL*s of the chain.  They stay in shared memory for the
     // launch (no registers across the T loop) and every sample is added to the running sum in time order, so the sums
     // do not depend on how the launch is sliced.
@@ -437,6 +475,23 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
             uacc = u01_fast(w3);
         }
         nrand = max(0, min(nrand, k - 1));
+        // Tempered: swap roles (ptsampler.py:102-112).  Rung i initiates a swap with i+1 iff it was not itself swapped by
+        // i-1, !(usel > pswap) and i < nt-1 -- sequential along the ladder: a ballot of lane 0 of every group, then at most
+        // nt-1 iterations.  Every decision reads start-of-step states (participants make no within-chain move), so all
+        // swaps of the step are decided at once.  Philox: usel from block (step, 2 GL + lane), read by lane 0.
+        bool is_init = false, is_part = false, regular = true;
+        if constexpr (TEMPER) {
+            const double usel = INJ ? usel_tape[t * K + c] : u01_fast(rk.block(step, (uint32_t)(2 * GL + lane)).x);
+            const bool want = live && lane == 0 && ti < tp->nt - 1 && !(usel > tp->pswap);
+            const int base = ((threadIdx.x & 31) / GL) & ~(tp->S - 1);      // the ladder's first group in the warp
+            const unsigned wb = __ballot_sync(FULL, want) >> (base * GL);
+            unsigned init = 0;
+            for (int b = 0; b < tp->nt - 1; ++b)
+                if (((wb >> (b * GL)) & 1u) && !(b > 0 && ((init >> (b - 1)) & 1u))) init |= 1u << b;
+            is_init = live && ((init >> ti) & 1u);
+            is_part = live && ti > 0 && ((init >> (ti - 1)) & 1u);
+            regular = !is_init && !is_part;
+        }
         // What the warp as a whole needs this step (warp-uniform).  With a shared move schedule all chains of the
         // warp drew the same move, so most of the step's blocks are skipped by real branches; with per-chain move types
         // the guards are almost always taken and the warp executes the union, selecting per chain.
@@ -582,22 +637,78 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
         const double sss = cp_ss_over_s2(nss, nsig);
         log4<GL>(lane, gp, __dmul_rn(nsig, nsig), uacc, jarg, nlg, nls2, logu, ljac);
         if (!wgp) nlg = s_lg[g];
-        const double lpn = cp_assemble(P, kk, sss, nvt, nlg, nsig, nls2, 0);
+        double lpn, nll = 0.0, nlpr = 0.0;
+        if constexpr (TEMPER) {
+            // TemperedModel (ptsampler.py:33-37): combine(log_prior, beta * log_likelihood); beta = 0 times -inf is nan -> -inf
+            nll = cp_assemble(P, kk, sss, nvt, nlg, nsig, nls2, 1);
+            nlpr = cp_assemble(P, kk, sss, nvt, nlg, nsig, nls2, 2);
+            lpn = combine_logpost(nlpr, __dmul_rn(beta, nll));
+        } else {
+            lpn = cp_assemble(P, kk, sss, nvt, nlg, nsig, nls2, 0);
+        }
         const double lqr = (mv == 3) ? (birth ? ljac : -ljac) : 0.0;
 
         // sampler.py:83-84 with Python's min(0, nan) == 0
         const double delta = lpn - lp - lqr;
         const double mh = (delta < 0.0) ? delta : 0.0;
-        const bool acc = !ovf && (logu < mh);
+        const bool acc = regular && !ovf && (logu < mh);
         trace_prop(t, lpn, acc, lqr, kk, nsig, nx, nv);
         if (acc) {
             k = kk; sig = nsig; lp = lpn;
             s_ss[g] = nss; s_vt[g] = nvt; s_lg[g] = nlg;
+            if constexpr (TEMPER) { s_ll[g] = nll; s_lpr[g] = nlpr; }
 #pragma unroll
             for (int j = 0; j < EPL; ++j) { cx[j] = nx[j]; cv[j] = nv[j]; bu[j] = nbu[j]; }
         }
         if (acc) s_nacc[threadIdx.x] += 1;
-        if (ovf) s_novf[threadIdx.x] += 1;
+        if (ovf && regular) s_novf[threadIdx.x] += 1;
+
+        if constexpr (TEMPER) {
+            // ---- swaps (ptsampler.py:113-125), only in warps where one is proposed.  The initiator (group g) sees its
+            //      partner in group g+1, GL lanes up; the state rows, k, sig, lp and the shared-memory slots of both move.
+            if (__any_sync(FULL, is_init)) {
+                __syncwarp();                                 // the partner's slots as its lanes last wrote them
+                const int go = is_init ? g + 1 : (is_part ? g - 1 : g);         // the partner's slot
+                const double ll_i = s_ll[g], lpr_i = s_lpr[g];
+                const double ll_o = s_ll[go], lpr_o = s_lpr[go], ss_o = s_ss[go], vt_o = s_vt[go], lg_o = s_lg[go];
+                const double beta_o = tp->betas[min(ti + 1, tp->nt - 1)];
+                const double lp_jj = __shfl_down_sync(FULL, lp, GL);
+                const double lp_ij = combine_logpost(lpr_o, __dmul_rn(beta, ll_o));      // model_i at theta_j
+                const double lp_ji = combine_logpost(lpr_i, __dmul_rn(beta_o, ll_i));    // model_j at theta_i
+                const double x = exp((lp_ji + lp_ij) - (lp + lp_jj));
+                const double mhr = (x < 1.0) ? x : 1.0;                                  // Python min(1, x): nan -> 1
+                const bool sw = is_init && (uacc < mhr);                                 // :121
+                const bool sw_prev = __shfl_up_sync(FULL, (int)sw, GL) != 0;
+                const double lp_ji_prev = __shfl_up_sync(FULL, lp_ji, GL);
+                const bool take = is_init ? sw : (is_part && sw_prev);
+                const double lp_o = is_init ? lp_ij : lp_ji_prev;
+                double ox[EPL], ov[EPL];
+                int ob[EPL];
+#pragma unroll
+                for (int j = 0; j < EPL; ++j) {
+                    ox[j] = cx[j]; ov[j] = cv[j]; ob[j] = bu[j];
+                    if (ROW_ON(j)) {                          // rows above hold the padding in both partners
+                        const double xd = __shfl_down_sync(FULL, cx[j], GL), xu = __shfl_up_sync(FULL, cx[j], GL);
+                        const double vd = __shfl_down_sync(FULL, cv[j], GL), vu = __shfl_up_sync(FULL, cv[j], GL);
+                        const int bd = __shfl_down_sync(FULL, bu[j], GL), bup = __shfl_up_sync(FULL, bu[j], GL);
+                        ox[j] = is_init ? xd : xu; ov[j] = is_init ? vd : vu; ob[j] = is_init ? bd : bup;
+                    }
+                }
+                const int kd = __shfl_down_sync(FULL, k, GL), ku = __shfl_up_sync(FULL, k, GL);
+                const double sd = __shfl_down_sync(FULL, sig, GL), su = __shfl_up_sync(FULL, sig, GL);
+                const int ko = is_init ? kd : ku;
+                const double so = is_init ? sd : su;
+                // a participant's proposal record is its partner's state, with logqratio = 0
+                if (is_init || is_part) trace_prop(t, lp_o, take, 0.0, ko, so, ox, ov);
+                __syncwarp();                                 // every lane has read its partner's slots
+                if (take) {
+                    k = ko; sig = so; lp = lp_o;
+                    s_ss[g] = ss_o; s_vt[g] = vt_o; s_lg[g] = lg_o; s_ll[g] = ll_o; s_lpr[g] = lpr_o;
+#pragma unroll
+                    for (int j = 0; j < EPL; ++j) { cx[j] = ox[j]; cv[j] = ov[j]; bu[j] = ob[j]; }
+                }
+            }
+        }
 
         if ((step % RMN_CP_DIAG_EVERY) == 0) {              // thinned accumulation (warp-uniform)
             const int kd = __reduce_max_sync(FULL, k);      // (an accepted birth may have raised the extent)
@@ -733,12 +844,45 @@ changepoint_sliced_kernel(const __grid_constant__ CPParams P, const double* __re
     }
 }
 
-// evaluate n states given in the canonical layout (pointwise parity entry + set_state)
-__global__ void __launch_bounds__(128)
-cp_eval_kernel(const __grid_constant__ CPParams P, const double* __restrict__ gdata, int which,
-               int64_t n, const int32_t* __restrict__ kin, const double* __restrict__ cpx,
-               const double* __restrict__ cpv, const double* __restrict__ sig,
-               double* __restrict__ out) {
+// Tempered form of changepoint_kernel's one-slice launch (rmn_sampler_set_tempering, GL = 4).
+//
+// Layout.  Ladder l occupies S = next_pow2(nt) consecutive 4-lane groups of one warp, rung i in group i of the slot, so
+// a warp holds 8 / S ladders and a ladder never straddles a warp; the S - nt idle groups shadow a live chain for the
+// shuffles and never store.  nt <= 8 (a larger ladder would need a cross-warp exchange through shared memory).
+// Swap exchange.  Partners are adjacent groups, GL lanes apart: one __shfl_down / __shfl_up pair per live register row of
+// cx, cv and the cached run boundaries, then k, sig and lp, selected for initiator, partner and neither; the per-chain
+// shared-memory slots (ss, vt, lg and the untempered log-likelihood / log-prior the swap test needs) move with the state.
+// The exchange sits under a warp-uniform __any_sync: a warp without a swap this step pays only the ballot.
+// Random numbers.  The untempered counters: block (step, lane) for the main words, (step, GL + lane) for rows 2-3; plus
+// (step, 2 GL + lane) for the swap-selection uniform, read by lane 0 of the group.  A swap initiator's swap uniform is
+// its accept word (w3), which its within-chain test does not use that step.  Philox stays keyed by the global chain id,
+// and with the "group" move schedule the schedule group is the warp's ladders aligned to global ladder ids, so a shard
+// reproduces its slice of the full run bit for bit.  Injected mode: usel[t*K + c] and the tape's ACC slot.
+template <bool INJ, int DATA>
+__global__ void __launch_bounds__(128, RMN_CP_MINBLOCKS)
+cp_tempered_kernel(const __grid_constant__ CPParams P, const __grid_constant__ CPTemper TP,
+                   const double* __restrict__ gdata, CPState st, int64_t K, int64_t T, int64_t step0, uint64_t seed,
+                   int64_t chain_offset, const double* __restrict__ tape, const double* __restrict__ usel,
+                   rmn_trace_t tr, int shared_mv) {
+    extern __shared__ double smem[];
+    const double* xs = gdata;
+    if (DATA != 0) {
+        const int n = P.XP + 2 * P.M + 2 + ((DATA == 2) ? P.G * 5 / 2 : 0);
+        for (int i = threadIdx.x; i < n; i += blockDim.x) smem[i] = gdata[i];
+        __syncthreads();
+        xs = smem;
+    }
+    cp_block<INJ, DATA, 4, true, true>(P, xs, st, K, 0, T, step0, seed, chain_offset, tape, tr, shared_mv, blockIdx.x,
+                                       &TP, usel);
+}
+
+// evaluate n states given in the canonical layout (pointwise parity entry + set_state); tempered (tp != nullptr): the
+// carried log-posterior combine(log_prior, betas[c % nt] * log_likelihood)
+template <bool TEMPER>
+__device__ __forceinline__ void cp_eval_body(const CPParams& P, const double* __restrict__ gdata, int which,
+                                             int64_t n, const int32_t* __restrict__ kin, const double* __restrict__ cpx,
+                                             const double* __restrict__ cpv, const double* __restrict__ sig,
+                                             double* __restrict__ out, const CPTemper* tp) {
     constexpr int GL = 16;
     const int lane = threadIdx.x & (GL - 1);
     const int64_t c_raw = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) / GL;
@@ -755,8 +899,29 @@ cp_eval_kernel(const __grid_constant__ CPParams P, const double* __restrict__ gd
     if (lane >= k) x1[0] = 0.0;
     if (lane > k) v1[0] = 0.0;
     double ss, vt, lg, ls2;
-    const double v = cp_logpost_rows<GL>(P, cyc, lane, kw, k, x1, v1, b1, sig[c], which, ss, vt, lg, ls2);
+    double v = cp_logpost_rows<GL>(P, cyc, lane, kw, k, x1, v1, b1, sig[c], TEMPER ? 1 : which, ss, vt, lg, ls2);
+    if constexpr (TEMPER) {
+        const double lpr = cp_assemble(P, k, cp_ss_over_s2(ss, sig[c]), vt, lg, sig[c], ls2, 2);
+        v = combine_logpost(lpr, __dmul_rn(tp->betas[c % tp->nt], v));
+    }
     if (live && lane == 0) out[c] = v;
+}
+
+__global__ void __launch_bounds__(128)
+cp_eval_kernel(const __grid_constant__ CPParams P, const double* __restrict__ gdata, int which,
+               int64_t n, const int32_t* __restrict__ kin, const double* __restrict__ cpx,
+               const double* __restrict__ cpv, const double* __restrict__ sig,
+               double* __restrict__ out) {
+    cp_eval_body<false>(P, gdata, which, n, kin, cpx, cpv, sig, out, nullptr);
+}
+
+// the chains' carried log-posterior on a ladder (chain_offset is a multiple of nt, so chain c is rung c % nt)
+__global__ void __launch_bounds__(128)
+cp_eval_tempered_kernel(const __grid_constant__ CPParams P, const __grid_constant__ CPTemper TP,
+                        const double* __restrict__ gdata, int64_t n, const int32_t* __restrict__ kin,
+                        const double* __restrict__ cpx, const double* __restrict__ cpv,
+                        const double* __restrict__ sig, double* __restrict__ out) {
+    cp_eval_body<true>(P, gdata, 0, n, kin, cpx, cpv, sig, out, &TP);
 }
 
 __global__ void cp_copy_state_kernel(int64_t K, const int32_t* k_in, const double* cpx_in,
@@ -878,6 +1043,10 @@ struct ChangepointSampler : SamplerImpl {
         if (e != cudaSuccess) return e;
         e = raise_smem((const void*)changepoint_sliced_kernel<DATA, 4, false>);
         if (e != cudaSuccess) return e;
+        e = raise_smem((const void*)cp_tempered_kernel<false, DATA>);
+        if (e != cudaSuccess) return e;
+        e = raise_smem((const void*)cp_tempered_kernel<true, DATA>);
+        if (e != cudaSuccess) return e;
         return raise_smem((const void*)changepoint_sliced_kernel<DATA, 4>);
     }
     unsigned grid(int gl = LANES) const { return (unsigned)((s->K * gl + 127) / 128); }
@@ -893,14 +1062,39 @@ struct ChangepointSampler : SamplerImpl {
         return RMN_OK;
     }
 
+    // parallel tempering (PTSampler, ptsampler.py:41-81): chains c = l*nt + i form ladder l with betas[i]; call before
+    // set_state.  A ladder lives inside one warp (cp_tempered_kernel), hence nt <= 8.
+    CPTemper tp{};
+    bool tempered = false;
+    int set_tempering(int nt, const double* betas, double pswap) override {
+        RMN_REQUIRE(nt >= 2 && nt <= 8 && betas,
+                    "set_tempering: the changepoint model takes ladders of 2 <= nt <= 8 temperatures (got %d)", nt);
+        RMN_REQUIRE(pswap > 0.0 && pswap < 1.0, "Pswap must be a number between 0 and 1");
+        RMN_REQUIRE(s->K % nt == 0, "set_tempering: the number of chains (%lld) must be a multiple of nt = %d", (long long)s->K, nt);
+        RMN_REQUIRE(s->chain_offset % nt == 0, "set_tempering: chain_offset must be a multiple of nt");
+        CPTemper t{};
+        for (int i = 0; i < nt; ++i) {
+            RMN_REQUIRE(betas[i] >= 0.0 && betas[i] <= 1.0, "beta = %g must be a number between 0 and 1", betas[i]);
+            t.betas[i] = betas[i];
+        }
+        t.nt = nt; t.pswap = pswap; t.S = 1;
+        while (t.S < nt) t.S *= 2;
+        tp = t; tempered = true;
+        return RMN_OK;
+    }
+
     int cp_set_state(const int32_t* d_k, const double* d_cpx, const double* d_cpv,
                      const double* d_sig, cudaStream_t stream) override {
         const int64_t n = s->K * LANES;
         cp_copy_state_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(
             s->K, d_k, d_cpx, d_cpv, d_sig, st.k, st.cpx, st.cpv, st.sig, nullptr, nullptr);
         RMN_KERNEL_CHECK();
-        cp_eval_kernel<<<grid(), 128, 0, stream>>>(P, s->model->d_cpdata, 0, s->K, st.k, st.cpx,
-                                                   st.cpv, st.sig, st.lp);
+        if (tempered)
+            cp_eval_tempered_kernel<<<grid(), 128, 0, stream>>>(P, tp, s->model->d_cpdata, s->K, st.k, st.cpx,
+                                                                st.cpv, st.sig, st.lp);
+        else
+            cp_eval_kernel<<<grid(), 128, 0, stream>>>(P, s->model->d_cpdata, 0, s->K, st.k, st.cpx,
+                                                       st.cpv, st.sig, st.lp);
         RMN_KERNEL_CHECK();
         launches += 2;
         return RMN_OK;
@@ -995,13 +1189,36 @@ struct ChangepointSampler : SamplerImpl {
             changepoint_kernel<INJ, 0, GL, GUARD><<<g, 128, 0, stream>>>(
                 P, s->model->d_cpdata, st, s->K, T, step0, s->seed, s->chain_offset, tape, t0, sh);
     }
+    // tempered runs: the one-slice launch at GL = 4 (RMN_CP_GL does not apply); one ladder slot of S groups per ladder
+    template <bool INJ>
+    void launch_tempered(int64_t T, const rmn_inject_t* inj, const rmn_trace_t& t0, cudaStream_t stream) {
+        const int sh = INJ ? 0 : shared_mv;
+        const int64_t L = s->K / tp.nt;
+        const int64_t head = sh ? ((s->chain_offset / tp.nt) & (int64_t)(8 / tp.S - 1)) : 0;
+        const unsigned g = (unsigned)(((L + head) * tp.S * 4 + 127) / 128);
+        const double* tape = INJ ? inj->d_tape : nullptr;
+        const double* usel = INJ ? inj->d_usel : nullptr;
+        if (use_smem && P.G > 0)
+            cp_tempered_kernel<INJ, 2><<<g, 128, smem_bytes, stream>>>(
+                P, tp, s->model->d_cpdata, st, s->K, T, step0, s->seed, s->chain_offset, tape, usel, t0, sh);
+        else if (use_smem)
+            cp_tempered_kernel<INJ, 1><<<g, 128, smem_bytes, stream>>>(
+                P, tp, s->model->d_cpdata, st, s->K, T, step0, s->seed, s->chain_offset, tape, usel, t0, sh);
+        else
+            cp_tempered_kernel<INJ, 0><<<g, 128, 0, stream>>>(
+                P, tp, s->model->d_cpdata, st, s->K, T, step0, s->seed, s->chain_offset, tape, usel, t0, sh);
+    }
     int run(int64_t T, const rmn_inject_t* inj, const rmn_trace_t* tr, cudaStream_t stream) override {
         rmn_trace_t t0{};
         if (tr) t0 = *tr;
         if (t0.thin <= 0) t0.thin = 1;
-        ktimer.begin("changepoint_kernel", stream);
-        if (inj) {
-            RMN_REQUIRE(inj->d_tape, "injected changepoint run needs d_tape");
+        if (inj) RMN_REQUIRE(inj->d_tape, "injected changepoint run needs d_tape");
+        if (inj && tempered) RMN_REQUIRE(inj->d_usel, "injected tempered run needs d_usel (selection uniforms)");
+        ktimer.begin(tempered ? "cp_tempered_kernel" : "changepoint_kernel", stream);
+        if (tempered) {
+            if (inj) launch_tempered<true>(T, inj, t0, stream);
+            else launch_tempered<false>(T, nullptr, t0, stream);
+        } else if (inj) {
             launch<true>(T, inj->d_tape, t0, stream);
         } else {
             launch<false>(T, nullptr, t0, stream);

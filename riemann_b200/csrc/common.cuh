@@ -280,7 +280,7 @@ struct SamplerImpl {
     virtual int get_adaptcov(double*, cudaStream_t) { return unsupported("get_adaptcov (small-d AdaptCovRandomWalk samplers only)"); }
     virtual int get_pooled_cov(double*, double*, double*, cudaStream_t) { return unsupported("get_pooled_cov (dense Gaussian samplers with PooledAdaptCovRandomWalk only)"); }
     virtual int set_row_comm(const void*, size_t, int, int) { return unsupported("row-sharded data mode (logistic samplers in f64 precision only)"); }
-    virtual int set_tempering(int, const double*, double) { return unsupported("parallel tempering (Gaussian and logistic samplers with RW / pCN proposals)"); }
+    virtual int set_tempering(int, const double*, double) { return unsupported("parallel tempering (Gaussian and logistic samplers with RW / pCN proposals, changepoint samplers)"); }
     virtual int get_adapt(double*, int64_t*, int64_t*, cudaStream_t) { return unsupported("get_adapt"); }
     virtual int set_adapt(const double*, const int64_t*, const int64_t*, cudaStream_t) { return unsupported("set_adapt"); }
     virtual int set_move_schedule(int) { return unsupported("move schedule (changepoint samplers only)"); }

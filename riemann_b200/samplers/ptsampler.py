@@ -8,7 +8,11 @@ lies along the chain axis of the device engine: chains l*Nt .. l*Nt+Nt-1 are lad
 inside the MH kernel on the small-d path (riemann_b200/csrc/small_gauss.cu) and an exchange of the two chain rows by the
 initiator's warp on the dense-Gaussian path (d > 8, riemann_b200/csrc/dense.cu) and on the logistic model
 (riemann_b200/csrc/logistic.cu; the prior is not tempered, :33-37) -- `rmn_sampler_set_tempering` -- and
-`K` independent ladders run side by side.
+`K` independent ladders run side by side.  On the changepoint model (ChangepointRegression1D with the shared,
+non-adaptive ChangepointRegression1DProp) a ladder of at most 8 temperatures lives inside one warp of the changepoint
+kernel (riemann_b200/csrc/changepoint.cu, cp_tempered_kernel) and a swap exchanges the two chains' register rows by
+shuffle; `theta0` is then a ChangepointParams (every chain), a list of K (one per ladder) or of K*Nt, and the
+histories are lists of ChangepointParams (K = 1) or ChangepointTrace objects [record, ladder] (K > 1).
 
 Reference behaviours kept: the default ladder `0.5**arange(5)`; the selection uniform is drawn for every chain,
 swapped or not (:104); the last chain never initiates (:107); `mhratio = min(1, exp(...))` with Python's `min`
@@ -17,13 +21,15 @@ chain as `_chain_thetas` / `_chain_logpost` (:83-90).  Reference defects not rep
 in the reference (`isinstance(betas, np.array)`, :62) -- here an explicit ladder is used as given, which is what
 that branch intends; `sample()` returns `np.array(zip(...))` there (:127) and the states here.
 The reference shares ONE proposal object between all temperatures (:81), so only non-adaptive proposals make
-sense; the device engine enforces that (MetropolisRandomWalk, pCN; Gaussian models of any dimension, logistic model).
+sense; the device engine enforces that (MetropolisRandomWalk, pCN; Gaussian models of any dimension, logistic model;
+ChangepointRegression1DProp on the changepoint model).
 """
 import numpy as np
 
+from ..models.changepoint import ChangepointParams, ChangepointRegression1D, unpack_state
 from ..models.model import Model
 from ..sampling_errors import ParameterError
-from .sampler import Sampler
+from .sampler import ChangepointTrace, Sampler
 
 
 class TemperedModel(Model):
@@ -66,9 +72,11 @@ class _TemperatureView(object):
 
 
 class PTSampler(object):
-    """Same constructor as the reference (ptsampler.py:47) plus `K` = number of independent ladders."""
+    """Same constructor as the reference (ptsampler.py:47) plus `K` = number of independent ladders, the Philox seed,
+    the global id of the first ladder (`chain_offset`, in ladders) and, on the changepoint model, the move schedule
+    (`Sampler`'s `move_schedule`; with "group" the ladders of a warp share the move-type draws)."""
 
-    def __init__(self, model, proposal, theta0, betas=None, Pswap=0.1, K=1, seed=0, chain_offset=0):
+    def __init__(self, model, proposal, theta0, betas=None, Pswap=0.1, K=1, seed=0, chain_offset=0, move_schedule=None):
         self.betas = 0.5 ** np.arange(5) if betas is None else np.asarray(betas, dtype=np.float64)
         if self.betas.ndim != 1 or not (2 <= len(self.betas) <= 32):
             raise ParameterError("betas must be a 1-d ladder of 2..32 temperatures")
@@ -76,25 +84,54 @@ class PTSampler(object):
             raise ParameterError("Pswap must be a number between 0 and 1")
         self.Pswap, self.model, self.proposal = Pswap, model, proposal
         self.K, self.Nt = int(K), len(self.betas)
-        th0 = np.atleast_1d(np.asarray(theta0, dtype=np.float64))
-        if th0.ndim == 1:
-            th0 = np.tile(th0, (self.K * self.Nt, 1))                  # every temperature starts at theta0 (:80-81)
-        elif th0.shape[0] == self.K:
-            th0 = np.repeat(th0, self.Nt, axis=0)
-        elif th0.shape[0] != self.K * self.Nt:
-            raise ParameterError("theta0 must be (d,), (K, d) or (K*Nt, d)")
-        self._sampler = Sampler(model, proposal, th0, seed=seed, chain_offset=chain_offset * self.Nt,
-                                _tempering=(self.betas, Pswap))
+        self._is_cp = isinstance(model, ChangepointRegression1D)
+        if self._is_cp:
+            if isinstance(theta0, ChangepointParams):
+                th0 = [theta0] * (self.K * self.Nt)                    # every temperature starts at theta0 (:80-81)
+            else:
+                th0 = list(theta0)
+                if len(th0) == self.K:
+                    th0 = [th for th in th0 for _ in range(self.Nt)]
+                elif len(th0) != self.K * self.Nt:
+                    raise ParameterError("theta0 must be a ChangepointParams or a list of K or K*Nt of them")
+        else:
+            th0 = np.atleast_1d(np.asarray(theta0, dtype=np.float64))
+            if th0.ndim == 1:
+                th0 = np.tile(th0, (self.K * self.Nt, 1))              # every temperature starts at theta0 (:80-81)
+            elif th0.shape[0] == self.K:
+                th0 = np.repeat(th0, self.Nt, axis=0)
+            elif th0.shape[0] != self.K * self.Nt:
+                raise ParameterError("theta0 must be (d,), (K, d) or (K*Nt, d)")
+        self._sampler = Sampler(model, proposal, th0, K=self.K * self.Nt, seed=seed, chain_offset=chain_offset * self.Nt,
+                                _tempering=(self.betas, Pswap), move_schedule=move_schedule)
         self.d = self._sampler.d
-        self._thetas = [np.asarray(self._sampler._chain_thetas[0]).reshape(self.K, self.Nt, self.d)]
-        self._logpost = [np.asarray(self._sampler._chain_logpost[0]).reshape(self.K, self.Nt)]
+        self._thetas, self._logpost = [], []
+        self._take_record(0)
         self.samplers = [_TemperatureView(self, i) for i in range(self.Nt)]
         self._publish()
 
+    def _take_record(self, r):
+        """Append record r of the flat sampler's history as [ladder][temperature] arrays (the changepoint model: a
+        tuple k, cpx, cpv, sig)."""
+        th, lp = self._sampler._chain_thetas, np.asarray(self._sampler._chain_logpost)
+        shape = (self.K, self.Nt)
+        if self._is_cp:
+            self._thetas.append(tuple(getattr(th, n)[r].reshape(shape + getattr(th, n).shape[2:])
+                                      for n in ("k", "cpx", "cpv", "sig")))
+        else:
+            self._thetas.append(np.asarray(th[r]).reshape(shape + (self.d,)))
+        self._logpost.append(lp[r].reshape(shape))
+
     # history [record][ladder][temperature]
     def _history_of(self, i):
+        lp = np.stack([l[:, i] for l in self._logpost])                # [rec, K]
+        if self._is_cp:
+            k, cpx, cpv, sig = (np.stack([t[n][:, i] for t in self._thetas]) for n in range(4))
+            if self.K == 1:
+                return [unpack_state(k[r, 0], cpx[r, 0], cpv[r, 0], sig[r, 0]) for r in range(k.shape[0])], \
+                    list(lp[:, 0])
+            return ChangepointTrace(k, cpx, cpv, sig), lp
         th = np.stack([t[:, i] for t in self._thetas])                 # [rec, K, d]
-        lp = np.stack([l[:, i] for l in self._logpost])
         if self.K == 1:
             return list(th[:, 0]), list(lp[:, 0])
         return th, lp
@@ -103,13 +140,8 @@ class PTSampler(object):
         self._chain_thetas, self._chain_logpost = self._history_of(0)
 
     def _absorb(self, ex=None):
-        th = np.asarray(self._sampler._chain_thetas)
-        lp = np.asarray(self._sampler._chain_logpost)
-        if th.ndim == 2:                                               # a single chain comes back as [rec, d]
-            th, lp = th[:, None, :], lp[:, None]
-        for r in range(1, th.shape[0]):                                # record 0 is the state we already hold
-            self._thetas.append(th[r].reshape(self.K, self.Nt, self.d))
-            self._logpost.append(lp[r].reshape(self.K, self.Nt))
+        for r in range(1, len(self._sampler._chain_logpost)):         # record 0 is the state we already hold
+            self._take_record(r)
         self._publish()
         return ex
 
@@ -121,13 +153,18 @@ class PTSampler(object):
             self._absorb()
         else:
             self._sampler.run(int(Nsamples), trace=False)
-            self._thetas = [np.asarray(self._sampler._chain_thetas[-1]).reshape(self.K, self.Nt, self.d)]
-            self._logpost = [np.asarray(self._sampler._chain_logpost[-1]).reshape(self.K, self.Nt)]
+            self._thetas, self._logpost = [], []
+            self._take_record(-1)
             self._publish()
 
-    def run_injected(self, usel, xi, u):
-        """Parity mode: usel[T, K*Nt], xi[T, K*Nt, d], u[T, K*Nt] in the reference's per-chain draw order."""
-        ex = self._sampler.run_injected(xi=xi, u=u, usel=usel)
+    def run_injected(self, usel, xi=None, u=None, tape=None):
+        """Parity mode: usel[T, K*Nt], xi[T, K*Nt, d], u[T, K*Nt] in the reference's per-chain draw order; the
+        changepoint model takes tape[T, K*Nt, NSLOT] instead of xi and u (a swap initiator's swap uniform in the
+        RMN_CP_SLOT_ACC slot)."""
+        if self._is_cp:
+            ex = self._sampler.run_injected(tape=tape, usel=usel)
+        else:
+            ex = self._sampler.run_injected(xi=xi, u=u, usel=usel)
         return self._absorb(ex)
 
     def sample(self):

@@ -358,7 +358,8 @@ class Sampler(object):
     def run_injected(self, xi=None, u=None, tape=None, Nburn=0, Nthin=1, usel=None):
         """
         Replay a given noise stream instead of Philox (parity mode):
-        fixed-d: xi[T, K, d] (or [T, d] for K = 1) and u[T, K]; changepoint: tape[T, K, NSLOT].
+        fixed-d: xi[T, K, d] (or [T, d] for K = 1) and u[T, K]; changepoint: tape[T, K, NSLOT].  Tempered samplers
+        also take usel[T, K], the swap-selection uniforms.
         Returns the per-step proposal record: 'prop_theta' [T,K,d] (or prop_k/cpx/cpv/sig),
         'logqratio', 'prop_logpost', 'accepted' [T,K].
         """
@@ -369,6 +370,13 @@ class Sampler(object):
             if tape.shape[1:] != (self.K, _lib.CP_NSLOT):
                 raise ParameterError("tape must have shape [T, K, {}]".format(_lib.CP_NSLOT))
             T, inj = tape.shape[0], {"tape": tape}
+            if usel is not None:                       # tempered samplers: swap-selection uniforms
+                usel = np.asarray(usel, dtype=np.float64)
+                if usel.ndim == 1:
+                    usel = usel[:, None]
+                if usel.shape != tape.shape[:2]:
+                    raise ParameterError("usel must be [T, K] like the tape")
+                inj["usel"] = usel
         else:
             xi = np.asarray(xi, dtype=np.float64)
             u = np.asarray(u, dtype=np.float64)
