@@ -1,8 +1,8 @@
 // riemann_b200 -- fused T-step MH kernel for the changepoint regression model.
 //
-// RMN_CP_LANES (=16) lanes cooperate on one chain: lane j holds cpx[j] and cpv[j] in
-// registers, so the variable-dimension state (k <= LANES-1 changepoints) needs no
-// dynamic indexing; insert/delete are warp shuffles.  Per iteration the kernel replaces
+// GL lanes cooperate on one chain; the variable-dimension state (k <= LANES-1 changepoints)
+// is held in shared-memory slots of the group's lanes, so insert/delete are loads of the
+// neighbouring element's slot.  Per iteration the kernel replaces
 //   Sampler.sample                                riemann/samplers/sampler.py:72-90
 //   ChangepointRegression1DProp.propose           examples/test_changepoint.py:44-73
 //   MetropolisRandomWalk.propose (3 block moves)  riemann/proposals/randomwalk.py:21-26
@@ -35,9 +35,10 @@ namespace {
 using namespace cp;
 
 // ---------------------------------------------------------------------------------------
-// Group geometry.  GL lanes cooperate on one chain (32/GL chains per warp); lane l holds the
+// Group geometry.  GL lanes cooperate on one chain (32/GL chains per warp); lane l owns the
 // EPL = LANES/GL elements e = l + GL*j, j = 0..EPL-1 ("row" j) of cpx, cpv and of the cached
-// run boundaries in registers, statically indexed.  Rows beyond the warp's largest extent hold
+// run boundaries (shared-memory slots for the state, registers for the proposal, statically
+// indexed).  Rows beyond the warp's largest extent hold
 // the canonical padding (cpx = 0, cpv = 0, boundary = M) and are skipped by a warp-uniform
 // guard, so with the typical 3..8 changepoints a GL = 4 warp spends its instructions on 8
 // chains and two rows instead of on 2 chains and ten idle lanes.
@@ -109,43 +110,34 @@ __device__ __forceinline__ void shift_next(const T (&a)[Geo<GL>::EPL], T (&out)[
     }
 }
 
-// value of element e + off of row j (a live row, see ROW_ON), off in {-1, 0, +1} chosen per chain (birth: -1 above
-// the insertion point, death: +1 from the removed element on, everything else 0); elements -1 and LANES read `pad`.
-// Two shuffles: the row itself and the neighbouring row the wrap-around lane reads from.  One row at a time, so that
-// the caller can merge it into the proposal before the next row is shifted.
+// The accepted state's rows live in shared memory for the duration of cp_block: slot [j][t] holds row j of thread t, so
+// element e of the chain of the group whose first thread is gb sits in slot [e / GL][gb + e % GL], and every thread
+// reads and writes its own slots in consecutive (conflict-free) words.  Reading another lane's slot needs a __syncwarp
+// after that lane's last write (see cp_block).
 template <int GL, typename T>
-__device__ __forceinline__ T shift_row(const T (&a)[Geo<GL>::EPL], int j, T pad, int lane, int dir, int off) {
-    constexpr int EPL = Geo<GL>::EPL;
-    const int src = (lane + off) & (GL - 1);
-    const T lo = (j > 0) ? a[j > 0 ? j - 1 : 0] : pad;            // row below (read by lane 0 when off = -1)
-    const T hi = (j + 1 < EPL) ? a[j + 1 < EPL ? j + 1 : j] : pad; // row above (read by lane GL-1 when off = +1)
-    const T m = __shfl_sync(0xffffffffu, a[j], src, GL);
-    const T w = __shfl_sync(0xffffffffu, (dir < 0) ? lo : hi, src, GL);
-    const bool wrap = (off < 0 && lane == 0) || (off > 0 && lane == GL - 1);
-    return wrap ? w : m;
+using Rows = T[Geo<GL>::EPL][128];
+
+// element e of the chain, e in [0, LANES)
+template <int GL, typename T>
+__device__ __forceinline__ T elem_at(const Rows<GL, T>& a, int e) {
+    return a[e >> Geo<GL>::LOG][(threadIdx.x & ~(GL - 1)) + (e & (GL - 1))];
 }
 
-// a[idx] for a per-chain element index idx in [0, LANES)
-template <int GL>
-__device__ __forceinline__ double elem_at(const double (&a)[Geo<GL>::EPL], int idx, int kw) {
-    double r = 0.0;
-#pragma unroll
-    for (int j = 0; j < Geo<GL>::EPL; ++j) {
-        if (ROW_ON(j)) {
-            const double t = __shfl_sync(0xffffffffu, a[j], idx & (GL - 1), GL);
-            if ((idx >> Geo<GL>::LOG) == j) r = t;
-        }
-    }
-    return r;
+// element e + off of the chain, off in {-1, 0, +1} chosen per chain (birth: -1 above the insertion point, death: +1
+// from the removed element on, everything else 0); elements -1 and LANES read `pad`
+template <int GL, typename T>
+__device__ __forceinline__ T shifted(const Rows<GL, T>& a, int e, int off, T pad) {
+    const int s = e + off;
+    return ((unsigned)s < (unsigned)LANES) ? elem_at<GL, T>(a, s) : pad;
 }
 
 // #{e < k : cpx[e] < s}   (np.searchsorted(cpx, s), changepoint.py:206)
 template <int GL>
-__device__ __forceinline__ int count_below(const double (&cx)[Geo<GL>::EPL], int lane, int k, double s, int kw) {
+__device__ __forceinline__ int count_below(const Rows<GL, double>& cx, int lane, int k, double s, int kw) {
     int n = 0;
 #pragma unroll
     for (int j = 0; j < Geo<GL>::EPL; ++j)
-        if (ROW_ON(j)) n += __popc(gballot<GL>(lane + GL * j < k && cx[j] < s));
+        if (ROW_ON(j)) n += __popc(gballot<GL>(lane + GL * j < k && cx[j][threadIdx.x] < s));
     return n;
 }
 
@@ -286,7 +278,7 @@ __device__ __forceinline__ double cp_logpost_rows(const CPParams& P, const doubl
 #define RMN_CP_MINBLOCKS 4          /* one-slice kernel (traced, injected, short or whole-wave runs) */
 #endif
 #ifndef RMN_CP_MINBLOCKS_SLICED
-#define RMN_CP_MINBLOCKS_SLICED 5   /* time-sliced kernel: 96 registers, 20 warps/SM */
+#define RMN_CP_MINBLOCKS_SLICED 6   /* time-sliced kernel: 80 registers, 24 warps/SM */
 #endif
 #ifndef RMN_CP_FASTPATHS
 #define RMN_CP_FASTPATHS 1   /* move-specific paths for warps whose chains all drew the same move type */
@@ -327,13 +319,13 @@ struct CPTemper {
 // moves every step, so the votes and the guards that a uniform warp would use are compiled out (same arithmetic, same bits).
 // TEMPER: the ladder layout and the swap moves of cp_tempered_kernel (tp, usel_tape); every addition sits under
 // `if constexpr`, so the untempered instantiations are unchanged.
-template <bool INJ, int DATA, int GL, bool GUARD, bool TEMPER = false>
+template <bool INJ, int DATA, int GL, bool GUARD, bool TEMPER = false, typename IT = int64_t>
 __device__ __forceinline__ void cp_block(const CPParams& P, const double* __restrict__ xs, CPState st,
-                                         int64_t K, int64_t t_begin, int64_t t_end, int64_t step0, uint64_t seed,
+                                         int64_t K, int64_t t_begin, IT nt, int64_t step0, uint64_t seed,
                                          int64_t chain_offset, const double* __restrict__ tape, const rmn_trace_t& tr,
                                          int shared_mv, int64_t blk, const CPTemper* tp = nullptr,
                                          const double* __restrict__ usel_tape = nullptr) {
-    // iterations [t_begin, t_end) of the launch for the 128 / GL chains of block `blk`; the chain state is read from and
+    // iterations [t_begin, t_begin + nt) of the launch for the 128 / GL chains of block `blk`; the chain state is read from and
     // written back to global memory (L2-coherent loads: in the time-sliced kernel another SM wrote it)
     constexpr int EPL = Geo<GL>::EPL;
     constexpr int NS = Geo<GL>::NS;
@@ -368,15 +360,10 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
     }
 
     int k = __ldcg(st.k + c);
-    double cx[EPL], cv[EPL];
-    int bu[EPL];                                  // cached run boundaries of the state
-#pragma unroll
-    for (int j = 0; j < EPL; ++j) {
-        const int e = lane + GL * j;
-        cx[j] = __ldcg(st.cpx + c * LANES + e);
-        cv[j] = __ldcg(st.cpv + c * LANES + e);
-        bu[j] = (e < k) ? run_boundary<BUCKETS>(P, xs, bx, cx[j]) : P.M;
-    }
+    // the state's rows: cpx, cpv and the cached run boundaries (see Rows).  They take no registers across the T loop;
+    // rows above the warp's extent (ROW_ON) keep the canonical padding they were loaded with.
+    __shared__ double s_cx[EPL][128], s_cv[EPL][128];
+    __shared__ int s_bu[EPL][128];
     double sig = __ldcg(st.sig + c);
     double lp = __ldcg(st.lp + c);
     // pieces of lp (see cp_terms / cp_assemble), one slot per chain of the block in shared memory: only the moves that
@@ -386,7 +373,19 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
     // tempered: the untempered log-likelihood and log-prior of the state, which the swap test reads for both partners
     __shared__ double s_ll[TEMPER ? 128 / GL : 1], s_lpr[TEMPER ? 128 / GL : 1];
     const int g = threadIdx.x / GL;
+    __shared__ int64_t s_chain[128 / GL];             // the chain the group writes back at the end, -1: none
+    s_chain[g] = live ? c : -1;
     {
+        double cx[EPL], cv[EPL];
+        int bu[EPL];
+#pragma unroll
+        for (int j = 0; j < EPL; ++j) {
+            const int e = lane + GL * j;
+            cx[j] = __ldcg(st.cpx + c * LANES + e);
+            cv[j] = __ldcg(st.cpv + c * LANES + e);
+            bu[j] = (e < k) ? run_boundary<BUCKETS>(P, xs, bx, cx[j]) : P.M;
+            s_cx[j][threadIdx.x] = cx[j]; s_cv[j][threadIdx.x] = cv[j]; s_bu[j][threadIdx.x] = bu[j];
+        }
         double ss0, vt0, lg0, ls20;
         const double v0 = cp_logpost_rows<GL>(P, cyc, lane, __reduce_max_sync(FULL, k), k, cx, cv, bu, sig, TEMPER ? 1 : 0,
                                               ss0, vt0, lg0, ls20);
@@ -441,7 +440,9 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
     uint4 rA = make_uint4(0, 0, 0, 0);
     if (!INJ) rA = rk.block((uint64_t)(step0 + t_begin), (uint32_t)lane);
 
-    for (int64_t t = t_begin; t < t_end; ++t) {
+    // IT = int (a time slice): the loop carries a 32-bit count instead of a 64-bit bound
+    int64_t t = t_begin;
+    for (IT n = nt; n > 0; --n, ++t) {
         const uint64_t step = (uint64_t)(step0 + t);
         const int kw = __reduce_max_sync(FULL, k);
         double snew, du, uacc;
@@ -506,10 +507,11 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
         double jarg = 1.0, hnew = 0.0;
         bool ovf = false, td = false;
         if (any3) {                                                     // warp-uniform
-            nb = count_below<GL>(cx, lane, k, snew, kw);                // searchsorted(cpx, s), :206
-            const double hb = elem_at<GL>(cv, nb, kw);
-            const double h1d = elem_at<GL>(cv, nrand, kw);
-            const double h2d = elem_at<GL>(cv, nrand + 1, kw);
+            __syncwarp();                                               // the other lanes' last writes to their slots
+            nb = count_below<GL>(s_cx, lane, k, snew, kw);              // searchsorted(cpx, s), :206
+            const double hb = elem_at<GL, double>(s_cv, nb);            // nb, nrand + 1 <= k: a live row
+            const double h1d = elem_at<GL, double>(s_cv, nrand);
+            const double h2d = elem_at<GL, double>(s_cv, nrand + 1);
             // birth (changepoint.py:57,61,72-74) and death (:67-68,76-78) share one instruction
             // stream: the operands of each division / square root are selected per chain
             const double q1 = birth ? du / P.sqrtM : h2d / h1d;
@@ -549,20 +551,23 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
 
         // ---- build the proposal by selection (the chains of a warp never diverge on mv).  Only live rows (ROW_ON) are
         //      touched: a row above holds the canonical padding in the state and in the proposal alike (every element
-        //      of it is beyond k + 1), so its proposal IS the state's row and needs no copy.  Inside a row, per-lane
+        //      of it is beyond k + 1), so its proposal IS the padding and needs no load.  Inside a row, per-lane
         //      predicates select between values that are all computed (no divergent branches).
         int nbu[EPL];
         double nx[EPL], nv[EPL], nsig = sig;
 #pragma unroll
-        for (int j = 0; j < EPL; ++j) { nx[j] = cx[j]; nv[j] = cv[j]; nbu[j] = bu[j]; }
+        for (int j = 0; j < EPL; ++j) {
+            nx[j] = 0.0; nv[j] = 0.0; nbu[j] = P.M;
+            if (ROW_ON(j)) { nx[j] = s_cx[j][threadIdx.x]; nv[j] = s_cv[j][threadIdx.x]; nbu[j] = s_bu[j][threadIdx.x]; }
+        }
         if (!skip || any0) {
             const double sxk = P.sx[k];
 #pragma unroll
             for (int j = 0; j < EPL; ++j) {
                 const int e = lane + GL * j;
                 if (ROW_ON(j)) {
-                    const double x1 = __dadd_rn(cx[j], __dmul_rn(sxk, xi[j]));           // randomwalk.py:26, scale = 1
-                    nx[j] = (mv == 0 && e < k) ? x1 : cx[j];
+                    const double x1 = __dadd_rn(nx[j], __dmul_rn(sxk, xi[j]));           // randomwalk.py:26, scale = 1
+                    nx[j] = (mv == 0 && e < k) ? x1 : nx[j];
                 }
             }
         }
@@ -571,8 +576,8 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
             for (int j = 0; j < EPL; ++j) {
                 const int e = lane + GL * j;
                 if (ROW_ON(j)) {
-                    const double v1 = __dadd_rn(cv[j], __dmul_rn(P.sv, xi[j]));
-                    nv[j] = (mv == 1 && e <= k) ? v1 : cv[j];
+                    const double v1 = __dadd_rn(nv[j], __dmul_rn(P.sv, xi[j]));
+                    nv[j] = (mv == 1 && e <= k) ? v1 : nv[j];
                 }
             }
         }
@@ -586,16 +591,15 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
 #pragma unroll
             for (int j = 0; j < EPL; ++j) {
                 const int e = lane + GL * j;
-                if (ROW_ON(j)) {                                        // rows above hold the padding: nothing moves
-                    const int off = (td && e > pivot) ? dir : 0;
-                    const double sx = shift_row<GL, double>(cx, j, 0.0, lane, dir, off);
-                    const double sv = shift_row<GL, double>(cv, j, 0.0, lane, dir, off);
-                    const int sb = shift_row<GL, int>(bu, j, P.M, lane, dir, off);
-                    if (td) { nx[j] = sx; nv[j] = sv; nbu[j] = sb; }
+                if (ROW_ON(j) && td) {                                  // rows above hold the padding: nothing moves
+                    const int off = (e > pivot) ? dir : 0;
+                    nx[j] = shifted<GL, double>(s_cx, e, off, 0.0);
+                    nv[j] = shifted<GL, double>(s_cv, e, off, 0.0);
+                    nbu[j] = shifted<GL, int>(s_bu, e, off, P.M);
                 }
                 if (td) {
                     if (birth) {
-                        if (e == nb) { nx[j] = snew; nv[j] = hnew; nbu[j] = bu[j]; }   // boundary searched below
+                        if (e == nb) { nx[j] = snew; nv[j] = hnew; }   // its boundary is searched below
                         if (e == nb + 1) nv[j] = hnew;
                     } else if (e == nrand) {
                         nv[j] = hnew;
@@ -653,12 +657,15 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
         const double mh = (delta < 0.0) ? delta : 0.0;
         const bool acc = regular && !ovf && (logu < mh);
         trace_prop(t, lpn, acc, lqr, kk, nsig, nx, nv);
+        if (any3) __syncwarp();                           // every lane has read the birth / death rows
         if (acc) {
             k = kk; sig = nsig; lp = lpn;
             s_ss[g] = nss; s_vt[g] = nvt; s_lg[g] = nlg;
             if constexpr (TEMPER) { s_ll[g] = nll; s_lpr[g] = nlpr; }
 #pragma unroll
-            for (int j = 0; j < EPL; ++j) { cx[j] = nx[j]; cv[j] = nv[j]; bu[j] = nbu[j]; }
+            for (int j = 0; j < EPL; ++j) {
+                if (ROW_ON(j)) { s_cx[j][threadIdx.x] = nx[j]; s_cv[j][threadIdx.x] = nv[j]; s_bu[j][threadIdx.x] = nbu[j]; }
+            }
         }
         if (acc) s_nacc[threadIdx.x] += 1;
         if (ovf && regular) s_novf[threadIdx.x] += 1;
@@ -682,18 +689,11 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
                 const double lp_ji_prev = __shfl_up_sync(FULL, lp_ji, GL);
                 const bool take = is_init ? sw : (is_part && sw_prev);
                 const double lp_o = is_init ? lp_ij : lp_ji_prev;
+                const int tq = go * GL + lane;                // the partner's slots (its own for a non-participant)
                 double ox[EPL], ov[EPL];
                 int ob[EPL];
 #pragma unroll
-                for (int j = 0; j < EPL; ++j) {
-                    ox[j] = cx[j]; ov[j] = cv[j]; ob[j] = bu[j];
-                    if (ROW_ON(j)) {                          // rows above hold the padding in both partners
-                        const double xd = __shfl_down_sync(FULL, cx[j], GL), xu = __shfl_up_sync(FULL, cx[j], GL);
-                        const double vd = __shfl_down_sync(FULL, cv[j], GL), vu = __shfl_up_sync(FULL, cv[j], GL);
-                        const int bd = __shfl_down_sync(FULL, bu[j], GL), bup = __shfl_up_sync(FULL, bu[j], GL);
-                        ox[j] = is_init ? xd : xu; ov[j] = is_init ? vd : vu; ob[j] = is_init ? bd : bup;
-                    }
-                }
+                for (int j = 0; j < EPL; ++j) { ox[j] = s_cx[j][tq]; ov[j] = s_cv[j][tq]; ob[j] = s_bu[j][tq]; }
                 const int kd = __shfl_down_sync(FULL, k, GL), ku = __shfl_up_sync(FULL, k, GL);
                 const double sd = __shfl_down_sync(FULL, sig, GL), su = __shfl_up_sync(FULL, sig, GL);
                 const int ko = is_init ? kd : ku;
@@ -705,12 +705,16 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
                     k = ko; sig = so; lp = lp_o;
                     s_ss[g] = ss_o; s_vt[g] = vt_o; s_lg[g] = lg_o; s_ll[g] = ll_o; s_lpr[g] = lpr_o;
 #pragma unroll
-                    for (int j = 0; j < EPL; ++j) { cx[j] = ox[j]; cv[j] = ov[j]; bu[j] = ob[j]; }
+                    for (int j = 0; j < EPL; ++j) {
+                        // rows above hold the padding in both partners
+                        if (ROW_ON(j)) { s_cx[j][threadIdx.x] = ox[j]; s_cv[j][threadIdx.x] = ov[j]; s_bu[j][threadIdx.x] = ob[j]; }
+                    }
                 }
             }
         }
 
         if ((step % RMN_CP_DIAG_EVERY) == 0) {              // thinned accumulation (warp-uniform)
+            __syncwarp();                                   // the rows as the other lanes accepted them
             const int kd = __reduce_max_sync(FULL, k);      // (an accepted birth may have raised the extent)
             double f[NS];
 #pragma unroll
@@ -719,8 +723,8 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
             if (lane == 1 % GL) f[1 / GL] = (double)k;
 #pragma unroll
             for (int q = 0; q < NQ; ++q) {
-                const int cnt = count_below<GL>(cx, lane, k, P.xq[q], kd);
-                const double yq = elem_at<GL>(cv, cnt, kd);
+                const int cnt = count_below<GL>(s_cx, lane, k, P.xq[q], kd);
+                const double yq = elem_at<GL, double>(s_cv, cnt);        // cnt <= k
                 if (lane == (2 + q) % GL) f[(2 + q) / GL] = yq;
             }
 #pragma unroll
@@ -728,6 +732,7 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
                 s_S1[s][threadIdx.x] = __dadd_rn(s_S1[s][threadIdx.x], f[s]);
                 s_S2[s][threadIdx.x] = __fma_rn(f[s], f[s], s_S2[s][threadIdx.x]);
             }
+            __syncwarp();                                   // every lane has read the rows before the next step writes
         }
 
         if (live && tracing) {
@@ -736,8 +741,8 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
 #pragma unroll
                 for (int j = 0; j < EPL; ++j) {
                     const int e = lane + GL * j;
-                    if (tr.d_cpx) tr.d_cpx[(rrec * K + c) * LANES + e] = cx[j];
-                    if (tr.d_cpv) tr.d_cpv[(rrec * K + c) * LANES + e] = cv[j];
+                    if (tr.d_cpx) tr.d_cpx[(rrec * K + c) * LANES + e] = s_cx[j][threadIdx.x];
+                    if (tr.d_cpv) tr.d_cpv[(rrec * K + c) * LANES + e] = s_cv[j][threadIdx.x];
                 }
                 if (lane == 0) {
                     if (tr.d_k) tr.d_k[rrec * K + c] = k;
@@ -748,12 +753,16 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
         }
     }
 
-    if (live) {
+    // the chain is read back from its slot: keeping c and `live` in registers across the T loop would cost registers the
+    // loop needs
+    const int64_t cw = s_chain[g];
+    if (cw >= 0) {
+        const int64_t c = cw;
 #pragma unroll
         for (int j = 0; j < EPL; ++j) {
             const int e = lane + GL * j;
-            st.cpx[c * LANES + e] = cx[j];
-            st.cpv[c * LANES + e] = cv[j];
+            st.cpx[c * LANES + e] = s_cx[j][threadIdx.x];
+            st.cpv[c * LANES + e] = s_cv[j][threadIdx.x];
         }
         if (lane == 0) {
             st.k[c] = k;
@@ -762,13 +771,9 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
             st.dacc[c] = __ldcg(st.dacc + c) + s_nacc[threadIdx.x];
             st.dovf[c] = __ldcg(st.dovf + c) + s_novf[threadIdx.x];
         }
-        // the same addresses as the loads at entry, computed again: keeping them live across the T loop would cost
-        // registers the loop needs (the empty asm hides that they are equal)
-        int64_t c2 = c;
-        asm volatile("" : "+l"(c2));
 #pragma unroll
         for (int s = 0; s < NS; ++s) {
-            const int64_t i = (int64_t)(lane + GL * s) * K + c2;
+            const int64_t i = (int64_t)(lane + GL * s) * K + c;
             if (lane + GL * s < RMN_CP_NDIAG) {
                 st.S1[i] = s_S1[s][threadIdx.x];
                 st.S2[i] = s_S2[s][threadIdx.x];
@@ -837,10 +842,12 @@ changepoint_sliced_kernel(const __grid_constant__ CPParams P, const double* __re
         if (it >= items) break;
         const int j = it / nblk, b = it % nblk;
         const int64_t t0 = (int64_t)j * slice, t1 = (t0 + slice < T) ? t0 + slice : T;
-        cp_block<false, DATA, GL, GUARD>(P, xs, st, K, t0, t1, step0, seed, chain_offset, nullptr, tr, shared_mv, b);
+        cp_block<false, DATA, GL, GUARD>(P, xs, st, K, t0, (int)(t1 - t0), step0, seed, chain_offset, nullptr, tr, shared_mv, b);
         __threadfence();
         __syncthreads();
-        if (threadIdx.x == 0) *reinterpret_cast<volatile int*>(done + b) = j + 1;
+        // the item is read again (s_item is not written before the next __syncthreads): keeping it live across the T
+        // loop would cost a register the loop needs
+        if (threadIdx.x == 0) *reinterpret_cast<volatile int*>(done + s_item % nblk) = s_item / nblk + 1;
     }
 }
 
@@ -849,9 +856,9 @@ changepoint_sliced_kernel(const __grid_constant__ CPParams P, const double* __re
 // Layout.  Ladder l occupies S = next_pow2(nt) consecutive 4-lane groups of one warp, rung i in group i of the slot, so
 // a warp holds 8 / S ladders and a ladder never straddles a warp; the S - nt idle groups shadow a live chain for the
 // shuffles and never store.  nt <= 8 (a larger ladder would need a cross-warp exchange through shared memory).
-// Swap exchange.  Partners are adjacent groups, GL lanes apart: one __shfl_down / __shfl_up pair per live register row of
-// cx, cv and the cached run boundaries, then k, sig and lp, selected for initiator, partner and neither; the per-chain
-// shared-memory slots (ss, vt, lg and the untempered log-likelihood / log-prior the swap test needs) move with the state.
+// Swap exchange.  Partners are adjacent groups, GL lanes apart: each lane reads its partner's state slots (rows of cpx, cpv
+// and the cached run boundaries) between two __syncwarp, k, sig and lp come by shuffles, and the per-chain shared-memory
+// slots (ss, vt, lg and the untempered log-likelihood / log-prior the swap test needs) move with the state.
 // The exchange sits under a warp-uniform __any_sync: a warp without a swap this step pays only the ballot.
 // Random numbers.  The untempered counters: block (step, lane) for the main words, (step, GL + lane) for rows 2-3; plus
 // (step, 2 GL + lane) for the swap-selection uniform, read by lane 0 of the group.  A swap initiator's swap uniform is
@@ -1025,7 +1032,7 @@ struct ChangepointSampler : SamplerImpl {
         return RMN_OK;
     }
     // without the attribute a kernel may take 48 KB minus its STATIC shared memory (the diagnostics sums, counts and
-    // cached pieces of cp_block: 4-7 KB) as dynamic shared memory
+    // cached pieces and state rows of cp_block: 6-17 KB) as dynamic shared memory
     cudaError_t raise_smem(const void* kernel) const {
         cudaFuncAttributes a{};
         cudaError_t e = cudaFuncGetAttributes(&a, kernel);
