@@ -46,6 +46,9 @@ def main():
     many = Sampler(model, proposal, theta0, K=K, seed=1)
     many.run(10000, trace=False)
     many.reset_diagnostics()
+    # posterior summaries of the second half on the device: the predictive band on a grid, changepoint locations, k
+    grid = np.linspace(xmin, xmax, 101)
+    many.set_posterior_summary(grid, value_range=(hmin - 1.0, hmax + 1.0), value_bins=200, every=16)
     many.run(10000, trace=False)
     d = many.diagnostics()
     final = many._chain_thetas                      # ChangepointTrace: arrays indexed [record, chain]; one record here
@@ -57,6 +60,15 @@ def main():
     print("           k over the final states: histogram", np.bincount(kfin).tolist())
     first = final[-1, 0]                            # one state as ChangepointParams, like the reference's history items
     print("           chain 0 ends at cpx", np.round(first.cpx, 3), "cpv", np.round(first.cpv, 3))
+    ps = many.posterior_summary()
+    band = ps.yhat_quantiles([0.05, 0.5, 0.95])
+    print("posterior summary: %d sampled chain-steps, posterior over k %s" % (ps.nsamples,
+                                                                           np.round(ps.khist / ps.nsamples, 3).tolist()))
+    for g in range(0, len(grid), 20):
+        print("           predictive band at x = %.2f: 5%% %.3f  50%% %.3f  95%% %.3f" % (grid[g], *band[:, g]))
+    top = np.argsort(ps.cpxhist)[::-1][:5]
+    cells = ["[%.2f, %.2f): %.3f" % (grid[i - 1], grid[i], ps.cpxhist[i] / ps.nsamples) for i in sorted(top) if 0 < i < len(grid)]
+    print("           most likely changepoint cells (changepoints per state):", "; ".join(cells))
 
 
 if __name__ == "__main__":

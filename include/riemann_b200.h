@@ -334,6 +334,28 @@ int rmn_sampler_chain_moments(rmn_sampler_t* s, double* d_mean, double* d_var, v
  * Injected runs always replay the per-chain move types of the tape.  Call before rmn_sampler_run. */
 int rmn_sampler_set_move_schedule(rmn_sampler_t* s, int mode);
 
+/* Posterior summaries of an untempered changepoint sampler, accumulated on the device as 64-bit integer histograms (no
+ * trace needed).  After every MH step whose global index s (rmn_sampler_get_step counts them) satisfies s % every == 0,
+ * the state of every chain adds
+ *   khist[k] += 1                         k = number of changepoints, 0..RMN_CP_LANES-1;
+ *   cpxhist[i] += 1 per changepoint x     i = #{g : h_grid[g] <= x} in 0..G (numpy searchsorted(grid, x, 'right'));
+ *   yhist[g][b] += 1 per grid point g     b = value bin of the prediction y = cpv[searchsorted(cpx[:k], grid[g])]
+ *                                         (ChangepointRegression1D.predict, changepoint.py:181): 1 + floor((y - vlo) * inv)
+ *                                         with inv = H / (vhi - vlo) in fp64 and round-to-nearest products, clamped to
+ *                                         bin 0 (below vlo, and NaN) and bin H + 1 (at or above vhi);
+ * and the count of sampled chain-steps grows by one.  Integer sums do not depend on the order of the additions, so the
+ * counts are identical for any split of a run into calls, time slices or chain shards.  rmn_sampler_reset_diagnostics
+ * also zeroes them.  The chains themselves are unchanged bit for bit.
+ * rmn_sampler_cp_set_summary: 1 <= G <= 1024 strictly increasing finite grid points h_grid (host), finite vlo < vhi,
+ * 1 <= H <= 1024 value bins, 1 <= every <= 2^62; resets the counts.  G = 0 turns the summaries off and frees their
+ * buffers.  Changepoint samplers at 4 lanes per chain only (RMN_CP_GL unset or 4), not tempered: RMN_ERR_UNSUPPORTED.
+ * rmn_sampler_cp_get_summary: d_khist[RMN_CP_LANES], d_cpxhist[G + 1], d_yhist[G][H + 2] (device, int64, any may be
+ * NULL) and *h_nsamples (host, may be NULL), the counts since the last reset; enqueued on `stream`. */
+int rmn_sampler_cp_set_summary(rmn_sampler_t* s, int G, const double* h_grid, double vlo, double vhi, int H,
+                               int64_t every);
+int rmn_sampler_cp_get_summary(rmn_sampler_t* s, int64_t* d_khist, int64_t* d_cpxhist, int64_t* d_yhist,
+                               int64_t* h_nsamples, void* stream);
+
 /* Number of kernel launches this handle has enqueued so far. */
 int64_t rmn_sampler_launch_count(const rmn_sampler_t* s);
 

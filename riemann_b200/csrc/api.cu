@@ -532,6 +532,19 @@ extern "C" int rmn_sampler_set_move_schedule(rmn_sampler_t* s, int mode) {
     return s->impl->set_move_schedule(mode);
 }
 
+extern "C" int rmn_sampler_cp_set_summary(rmn_sampler_t* s, int G, const double* h_grid, double vlo, double vhi, int H,
+                                          int64_t every) {
+    RMN_REQUIRE(s && s->impl, "rmn_sampler_cp_set_summary: null sampler");
+    return s->impl->cp_set_summary(G, h_grid, vlo, vhi, H, every);
+}
+
+extern "C" int rmn_sampler_cp_get_summary(rmn_sampler_t* s, int64_t* d_khist, int64_t* d_cpxhist, int64_t* d_yhist,
+                                          int64_t* h_nsamples, void* stream) {
+    NvtxRange nvtx_("rmn_sampler_cp_get_summary");
+    RMN_REQUIRE(s && s->impl, "rmn_sampler_cp_get_summary: null sampler");
+    return s->impl->cp_get_summary(d_khist, d_cpxhist, d_yhist, h_nsamples, (cudaStream_t)stream);
+}
+
 extern "C" int rmn_sampler_chain_moments(rmn_sampler_t* s, double* d_mean, double* d_var, void* stream) {
     RMN_REQUIRE(s && s->impl, "rmn_sampler_chain_moments: null sampler");
     const double *S1 = nullptr, *S2 = nullptr;

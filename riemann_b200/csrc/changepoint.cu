@@ -25,6 +25,7 @@
 // as logqratio.
 #include "changepoint.cuh"
 #include <stdlib.h>
+#include <algorithm>
 
 #ifndef RMN_CP_DEFAULT_GL
 #define RMN_CP_DEFAULT_GL 4
@@ -280,6 +281,9 @@ __device__ __forceinline__ double cp_logpost_rows(const CPParams& P, const doubl
 #ifndef RMN_CP_MINBLOCKS_SLICED
 #define RMN_CP_MINBLOCKS_SLICED 6   /* time-sliced kernel: 80 registers, 24 warps/SM */
 #endif
+#ifndef RMN_CP_MINBLOCKS_SUMMARY
+#define RMN_CP_MINBLOCKS_SUMMARY 5  /* time-sliced summary kernel: 96 registers (at 80 the sampling spills in the T loop) */
+#endif
 #ifndef RMN_CP_FASTPATHS
 #define RMN_CP_FASTPATHS 1   /* move-specific paths for warps whose chains all drew the same move type */
 #endif
@@ -315,16 +319,82 @@ struct CPTemper {
     int S;                      // groups a ladder occupies: the power of two >= nt
 };
 
+// Posterior summaries (rmn_sampler_cp_set_summary), given only to the cp_summary kernels.  After every step s with
+// s % every == 0 each live chain's state adds, with i_j = #{g : xg[g] <= cpx[j]} and the prediction on the grid
+// yhat(xg[g]) = cpv[#{j < k : cpx[j] < xg[g]}] (ChangepointRegression1D.predict, changepoint.py:181):
+//   khist[k] += 1;  cpxhist[i_j] += 1 for j < k;  yhist[g][bin(yhat(xg[g]))] += 1 for every g,
+// the last one as a difference array over g: segment s = 0..k covers the grid indices [i_{s-1}, i_s) (i_{-1} = 0,
+// i_k = G) at the one bin b_s = bin(cpv[s]), so it adds +1 at D[i_{s-1}][b_s] and -1 at D[i_s][b_s] (nothing for an
+// empty segment or at row G); the prefix sum over g of D is yhist (cp_summary_readout_kernel).  Every counter is a 64-bit
+// integer (the -1 in two's complement), so the counts do not depend on the order of the atomics.  Row 0 of D (every
+// chain's first segment starts there), khist and cpxhist are counted per block in shared memory and flushed at the end of
+// cp_block; the rest of D goes to global memory directly.
+struct CPSummary {
+    const double* xg;            // grid, NaN-padded to 2 * GP2 entries (padded_upper_bound)
+    int G, GP2, H;
+    double vlo, inv;             // inv = H / (vhi - vlo), on the host in fp64
+    long long every;
+    unsigned long long* khist;   // [LANES]
+    unsigned long long* cpxhist; // [G + 1]
+    unsigned long long* D;       // [G][H + 2]
+};
+// the block's shared counters: khist [LANES] | cpxhist [G + 1] | D row 0 [H + 2]
+__host__ __device__ __forceinline__ int summary_counters(int G, int H) { return LANES + (G + 1) + (H + 2); }
+
+// value bin of y: 1 + floor((y - vlo) * inv) clamped to [0, H + 1]; NaN counts in bin 0
+__device__ __forceinline__ int summary_bin(const CPSummary& S, double y) {
+    const double t = __dmul_rn(__dsub_rn(y, S.vlo), S.inv);
+    return (t >= 0.0) ? ((t < (double)S.H) ? 1 + (int)t : S.H + 1) : 0;
+}
+
+// one chain's sampled state (rows as accepted; the caller brackets this with __syncwarp): O(k) searches and atomics
+template <int GL>
+__device__ __forceinline__ void summary_sample(const CPSummary& S, unsigned long long* ssum,
+                                               const Rows<GL, double>& cx, const Rows<GL, double>& cv, int lane, int k,
+                                               bool live) {
+    constexpr int EPL = Geo<GL>::EPL;
+    const int kw = __reduce_max_sync(0xffffffffu, k);
+    unsigned long long* s_khist = ssum;
+    unsigned long long* s_cpxhist = ssum + LANES;
+    unsigned long long* s_d0 = s_cpxhist + S.G + 1;
+    if (live && lane == 0) atomicAdd(s_khist + k, 1ull);
+    double q[EPL];
+    int i[EPL], ip[EPL];
+#pragma unroll
+    for (int j = 0; j < EPL; ++j) q[j] = cx[j][threadIdx.x];
+    padded_upper_bound<EPL>(S.xg, S.GP2, q, i);
+#pragma unroll
+    for (int j = 0; j < EPL; ++j) if (lane + GL * j >= k) i[j] = S.G;      // i_k = G (and the padding beyond)
+    shift_prev<GL, int>(i, ip, 0, lane, kw);                                // i_{e-1}, i_{-1} = 0
+    const int W = S.H + 2;
+#pragma unroll
+    for (int j = 0; j < EPL; ++j) {
+        const int e = lane + GL * j;
+        if (ROW_ON(j) && live && e <= k) {
+            if (e < k) atomicAdd(s_cpxhist + i[j], 1ull);
+            if (ip[j] < i[j]) {                                             // segment e is not empty
+                const int b = summary_bin(S, cv[j][threadIdx.x]);
+                if (ip[j] == 0) atomicAdd(s_d0 + b, 1ull);
+                else atomicAdd(S.D + (size_t)ip[j] * W + b, 1ull);
+                if (i[j] < S.G) atomicAdd(S.D + (size_t)i[j] * W + b, ~0ull);
+            }
+        }
+    }
+}
+
 // GUARD = false: the instantiation for per-chain move schedules in Philox mode -- the warp executes the union of the
 // moves every step, so the votes and the guards that a uniform warp would use are compiled out (same arithmetic, same bits).
 // TEMPER: the ladder layout and the swap moves of cp_tempered_kernel (tp, usel_tape); every addition sits under
 // `if constexpr`, so the untempered instantiations are unchanged.
-template <bool INJ, int DATA, int GL, bool GUARD, bool TEMPER = false, typename IT = int64_t>
+// SUMMARY: the posterior summaries of the cp_summary kernels (sp, and ssum = the block's shared counters, see CPSummary),
+// likewise under `if constexpr`.
+template <bool INJ, int DATA, int GL, bool GUARD, bool TEMPER = false, typename IT = int64_t, bool SUMMARY = false>
 __device__ __forceinline__ void cp_block(const CPParams& P, const double* __restrict__ xs, CPState st,
                                          int64_t K, int64_t t_begin, IT nt, int64_t step0, uint64_t seed,
                                          int64_t chain_offset, const double* __restrict__ tape, const rmn_trace_t& tr,
                                          int shared_mv, int64_t blk, const CPTemper* tp = nullptr,
-                                         const double* __restrict__ usel_tape = nullptr) {
+                                         const double* __restrict__ usel_tape = nullptr, const CPSummary* sp = nullptr,
+                                         unsigned long long* ssum = nullptr) {
     // iterations [t_begin, t_begin + nt) of the launch for the 128 / GL chains of block `blk`; the chain state is read from and
     // written back to global memory (L2-coherent loads: in the time-sliced kernel another SM wrote it)
     constexpr int EPL = Geo<GL>::EPL;
@@ -410,6 +480,14 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
     }
     __shared__ int s_nacc[128], s_novf[128];        // accept / overflow counts of the launch, one per thread
     s_nacc[threadIdx.x] = 0; s_novf[threadIdx.x] = 0;
+    // summaries: the next sampled step, one slot per thread (every thread of the block walks the same steps)
+    __shared__ long long s_snext[SUMMARY ? 128 : 1];
+    if constexpr (SUMMARY) {
+        const long long s0 = step0 + t_begin, r = s0 % sp->every;
+        s_snext[threadIdx.x] = (r == 0) ? s0 : s0 - r + sp->every;
+        for (int i = threadIdx.x; i < summary_counters(sp->G, sp->H); i += blockDim.x) ssum[i] = 0;
+        __syncthreads();
+    }
     const RngKey rk(seed, (uint64_t)(chain_offset + c_raw));
     const TraceSel ts{tr.first, tr.thin > 0 ? tr.thin : 1};
     const bool tracing = tr.d_k || tr.d_cpx || tr.d_cpv || tr.d_sig || tr.d_logpost;
@@ -734,6 +812,14 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
             }
             __syncwarp();                                   // every lane has read the rows before the next step writes
         }
+        if constexpr (SUMMARY) {
+            if ((long long)step == s_snext[threadIdx.x]) {  // warp-uniform
+                s_snext[threadIdx.x] += sp->every;
+                __syncwarp();                               // the rows as the other lanes accepted them
+                summary_sample<GL>(*sp, ssum, s_cx, s_cv, lane, k, s_chain[g] >= 0);
+                __syncwarp();                               // every lane has read the rows before the next step writes
+            }
+        }
 
         if (live && tracing) {
             const long long rrec = ts.slot(t + 1);
@@ -780,6 +866,14 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
             }
         }
     }
+    if constexpr (SUMMARY) {
+        __syncthreads();                                // every warp's last sample is in the shared counters
+        const int n1 = LANES, n2 = LANES + sp->G + 1;
+        for (int i = threadIdx.x; i < summary_counters(sp->G, sp->H); i += blockDim.x) {
+            const unsigned long long v = ssum[i];
+            if (v) atomicAdd((i < n1) ? sp->khist + i : ((i < n2) ? sp->cpxhist + (i - n1) : sp->D + (i - n2)), v);
+        }
+    }
 }
 
 // DATA: 0 = data tables read from global memory (too large for shared memory), 1 = staged in shared
@@ -808,19 +902,12 @@ changepoint_kernel(const __grid_constant__ CPParams P, const double* __restrict_
 // item, the state of a slice's chains travels through global memory, and a flag per chain block orders the slices of the
 // same chains (the predecessor is B >> S items earlier, so the wait is almost never taken).  Philox is keyed by
 // (step, chain), so the chains are bit-identical to the one-slice launch.
-template <int DATA, int GL, bool GUARD = true>
-__global__ void __launch_bounds__(128, (GL == 16) ? 8 : RMN_CP_MINBLOCKS_SLICED)
-changepoint_sliced_kernel(const __grid_constant__ CPParams P, const double* __restrict__ gdata, CPState st,
-                          int64_t K, int64_t T, int64_t step0, uint64_t seed, int64_t chain_offset, int shared_mv,
-                          int nblk, int slice, int nslice, int* __restrict__ done) {
-    extern __shared__ double smem[];
-    const double* xs = gdata;
-    if (DATA != 0) {
-        const int n = P.XP + 2 * P.M + 2 + ((DATA == 2) ? P.G * 5 / 2 : 0);
-        for (int i = threadIdx.x; i < n; i += blockDim.x) smem[i] = gdata[i];
-        __syncthreads();
-        xs = smem;
-    }
+// The body is shared with cp_summary_sliced_kernel (SUMMARY: sp and the block's shared counters ssum, see CPSummary).
+template <int DATA, int GL, bool GUARD, bool SUMMARY>
+__device__ __forceinline__ void cp_sliced_body(const CPParams& P, const double* __restrict__ xs, CPState st, int64_t K,
+                                               int64_t T, int64_t step0, uint64_t seed, int64_t chain_offset,
+                                               int shared_mv, int nblk, int slice, int nslice, int* __restrict__ done,
+                                               const CPSummary* sp, unsigned long long* ssum) {
     rmn_trace_t tr{};
     __shared__ int s_item;
     const int items = nblk * nslice;
@@ -842,12 +929,86 @@ changepoint_sliced_kernel(const __grid_constant__ CPParams P, const double* __re
         if (it >= items) break;
         const int j = it / nblk, b = it % nblk;
         const int64_t t0 = (int64_t)j * slice, t1 = (t0 + slice < T) ? t0 + slice : T;
-        cp_block<false, DATA, GL, GUARD>(P, xs, st, K, t0, (int)(t1 - t0), step0, seed, chain_offset, nullptr, tr, shared_mv, b);
+        if constexpr (SUMMARY)
+            cp_block<false, DATA, GL, GUARD, false, int, true>(P, xs, st, K, t0, (int)(t1 - t0), step0, seed, chain_offset,
+                                                               nullptr, tr, shared_mv, b, nullptr, nullptr, sp, ssum);
+        else
+            cp_block<false, DATA, GL, GUARD>(P, xs, st, K, t0, (int)(t1 - t0), step0, seed, chain_offset, nullptr, tr, shared_mv, b);
         __threadfence();
         __syncthreads();
         // the item is read again (s_item is not written before the next __syncthreads): keeping it live across the T
         // loop would cost a register the loop needs
         if (threadIdx.x == 0) *reinterpret_cast<volatile int*>(done + s_item % nblk) = s_item / nblk + 1;
+    }
+}
+
+template <int DATA, int GL, bool GUARD = true>
+__global__ void __launch_bounds__(128, (GL == 16) ? 8 : RMN_CP_MINBLOCKS_SLICED)
+changepoint_sliced_kernel(const __grid_constant__ CPParams P, const double* __restrict__ gdata, CPState st,
+                          int64_t K, int64_t T, int64_t step0, uint64_t seed, int64_t chain_offset, int shared_mv,
+                          int nblk, int slice, int nslice, int* __restrict__ done) {
+    extern __shared__ double smem[];
+    const double* xs = gdata;
+    if (DATA != 0) {
+        const int n = P.XP + 2 * P.M + 2 + ((DATA == 2) ? P.G * 5 / 2 : 0);
+        for (int i = threadIdx.x; i < n; i += blockDim.x) smem[i] = gdata[i];
+        __syncthreads();
+        xs = smem;
+    }
+    cp_sliced_body<DATA, GL, GUARD, false>(P, xs, st, K, T, step0, seed, chain_offset, shared_mv, nblk, slice, nslice, done,
+                                           nullptr, nullptr);
+}
+
+// Posterior summaries (rmn_sampler_cp_set_summary, GL = 4): the one-slice and the time-sliced launch of the same run with
+// the summary sampling compiled in (cp_block<..., SUMMARY = true>).  Dynamic shared memory: the staged data tables (DATA
+// > 0), then the block's summary counters.  The chains are those of changepoint_kernel / changepoint_sliced_kernel bit
+// for bit: the sampling only reads the accepted rows.
+template <bool INJ, int DATA, bool GUARD>
+__global__ void __launch_bounds__(128, RMN_CP_MINBLOCKS)
+cp_summary_kernel(const __grid_constant__ CPParams P, const __grid_constant__ CPSummary SP,
+                  const double* __restrict__ gdata, CPState st, int64_t K, int64_t T, int64_t step0, uint64_t seed,
+                  int64_t chain_offset, const double* __restrict__ tape, rmn_trace_t tr, int shared_mv) {
+    extern __shared__ double smem[];
+    const double* xs = gdata;
+    const int n = (DATA != 0) ? P.XP + 2 * P.M + 2 + ((DATA == 2) ? P.G * 5 / 2 : 0) : 0;
+    if (DATA != 0) {
+        for (int i = threadIdx.x; i < n; i += blockDim.x) smem[i] = gdata[i];
+        __syncthreads();
+        xs = smem;
+    }
+    cp_block<INJ, DATA, 4, GUARD, false, int64_t, true>(P, xs, st, K, 0, T, step0, seed, chain_offset, tape, tr, shared_mv,
+                                                         blockIdx.x, nullptr, nullptr, &SP,
+                                                         reinterpret_cast<unsigned long long*>(smem + n));
+}
+
+template <int DATA, bool GUARD>
+__global__ void __launch_bounds__(128, RMN_CP_MINBLOCKS_SUMMARY)
+cp_summary_sliced_kernel(const __grid_constant__ CPParams P, const __grid_constant__ CPSummary SP,
+                         const double* __restrict__ gdata, CPState st, int64_t K, int64_t T, int64_t step0,
+                         uint64_t seed, int64_t chain_offset, int shared_mv, int nblk, int slice, int nslice,
+                         int* __restrict__ done) {
+    extern __shared__ double smem[];
+    const int n = P.XP + 2 * P.M + 2 + ((DATA == 2) ? P.G * 5 / 2 : 0);
+    for (int i = threadIdx.x; i < n; i += blockDim.x) smem[i] = gdata[i];
+    __syncthreads();
+    cp_sliced_body<DATA, 4, GUARD, true>(P, smem, st, K, T, step0, seed, chain_offset, shared_mv, nblk, slice, nslice, done,
+                                         &SP, reinterpret_cast<unsigned long long*>(smem + n));
+}
+
+// D [G][W] -> yhist [G][W] by a prefix sum over g, one thread per bin column (int64, exact); khist and cpxhist copied
+__global__ void cp_summary_readout_kernel(const unsigned long long* __restrict__ khist,
+                                          const unsigned long long* __restrict__ cpxhist,
+                                          const unsigned long long* __restrict__ D, int G, int W, int64_t* d_khist,
+                                          int64_t* d_cpxhist, int64_t* d_yhist) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (d_khist && i < LANES) d_khist[i] = (int64_t)khist[i];
+    if (d_cpxhist && i <= G) d_cpxhist[i] = (int64_t)cpxhist[i];
+    if (d_yhist && i < W) {
+        unsigned long long acc = 0;
+        for (int g = 0; g < G; ++g) {
+            acc += D[(size_t)g * W + i];
+            d_yhist[(size_t)g * W + i] = (int64_t)acc;
+        }
     }
 }
 
@@ -1033,12 +1194,13 @@ struct ChangepointSampler : SamplerImpl {
     }
     // without the attribute a kernel may take 48 KB minus its STATIC shared memory (the diagnostics sums, counts and
     // cached pieces and state rows of cp_block: 6-17 KB) as dynamic shared memory
-    cudaError_t raise_smem(const void* kernel) const {
+    cudaError_t raise_smem(const void* kernel, size_t bytes) const {
         cudaFuncAttributes a{};
         cudaError_t e = cudaFuncGetAttributes(&a, kernel);
         if (e != cudaSuccess) return e;
-        return (smem_bytes + a.sharedSizeBytes > 48 * 1024) ? rmn_raise_dyn_smem(kernel, smem_bytes) : cudaSuccess;
+        return (bytes + a.sharedSizeBytes > 48 * 1024) ? rmn_raise_dyn_smem(kernel, bytes) : cudaSuccess;
     }
+    cudaError_t raise_smem(const void* kernel) const { return raise_smem(kernel, smem_bytes); }
     // the staged kernels this data launches: DATA = 2 with the bucket table, 1 without
     template <int GL> cudaError_t set_smem_attr() { return (P.G > 0) ? set_smem_attr<2, GL>() : set_smem_attr<1, GL>(); }
     template <int DATA, int GL> cudaError_t set_smem_attr() {
@@ -1128,9 +1290,12 @@ struct ChangepointSampler : SamplerImpl {
     int done_cap = 0;
     int sliced = 1;                 // RMN_CP_SLICED=0 switches it off (A/B)
     int force_guard = 0;            // RMN_CP_GUARD=1: per-chain schedules through the guarded instantiation (A/B)
-    ~ChangepointSampler() override { if (d_done) cudaFree(d_done); }
+    ~ChangepointSampler() override {
+        if (d_done) cudaFree(d_done);
+        free_summary();
+    }
     bool last_sliced = false;       // which kernel the last plain launch used (the timer label is corrected after the launch)
-    template <int DATA, int GL, bool GUARD>
+    template <int DATA, int GL, bool GUARD, bool SUM = false>
     bool launch_sliced(int64_t T, unsigned nblk, int sh, size_t smem, cudaStream_t stream) {
         constexpr int SLICE_MIN = 100;          // iterations: the state round trip and the entry evaluation cost about one
         last_sliced = false;
@@ -1138,7 +1303,8 @@ struct ChangepointSampler : SamplerImpl {
         int dev = 0, sms = 0, per_sm = 0;
         cudaGetDevice(&dev);
         cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, changepoint_sliced_kernel<DATA, GL, GUARD>, 128, smem) != cudaSuccess || per_sm < 1)
+        const void* kfn = SUM ? (const void*)cp_summary_sliced_kernel<DATA, GUARD> : (const void*)changepoint_sliced_kernel<DATA, GL, GUARD>;
+        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kfn, 128, smem) != cudaSuccess || per_sm < 1)
             return false;
         const unsigned slots = (unsigned)(per_sm * sms);
         if (nblk <= slots || nblk % slots == 0) return false;       // one wave, or whole waves: nothing to gain
@@ -1161,8 +1327,12 @@ struct ChangepointSampler : SamplerImpl {
             done_cap = (int)nblk;
         }
         if (cudaMemsetAsync(d_done, 0, ((size_t)nblk + 1) * sizeof(int), stream) != cudaSuccess) return false;
-        changepoint_sliced_kernel<DATA, GL, GUARD><<<slots, 128, smem, stream>>>(
-            P, s->model->d_cpdata, st, s->K, T, step0, s->seed, s->chain_offset, sh, (int)nblk, slice, nslice, d_done);
+        if constexpr (SUM)
+            cp_summary_sliced_kernel<DATA, GUARD><<<slots, 128, smem, stream>>>(
+                P, sum, s->model->d_cpdata, st, s->K, T, step0, s->seed, s->chain_offset, sh, (int)nblk, slice, nslice, d_done);
+        else
+            changepoint_sliced_kernel<DATA, GL, GUARD><<<slots, 128, smem, stream>>>(
+                P, s->model->d_cpdata, st, s->K, T, step0, s->seed, s->chain_offset, sh, (int)nblk, slice, nslice, d_done);
         last_sliced = true;
         return true;
     }
@@ -1175,13 +1345,16 @@ struct ChangepointSampler : SamplerImpl {
         }
         launch_gl_g<INJ, GL, true>(T, tape, t0, stream);
     }
+    static bool is_traced(const rmn_trace_t& t0) {
+        return t0.d_k || t0.d_cpx || t0.d_cpv || t0.d_sig || t0.d_logpost || t0.d_prop_logpost || t0.d_accepted ||
+               t0.d_logqratio || t0.d_prop_k || t0.d_prop_sig || t0.d_prop_cpx || t0.d_prop_cpv;
+    }
     template <bool INJ, int GL, bool GUARD>
     void launch_gl_g(int64_t T, const double* tape, const rmn_trace_t& t0, cudaStream_t stream) {
         const int sh = INJ ? 0 : shared_mv;
         const unsigned g = run_grid(GL, sh);
         last_sliced = false;
-        const bool traced = t0.d_k || t0.d_cpx || t0.d_cpv || t0.d_sig || t0.d_logpost || t0.d_prop_logpost || t0.d_accepted ||
-                            t0.d_logqratio || t0.d_prop_k || t0.d_prop_sig || t0.d_prop_cpx || t0.d_prop_cpv;
+        const bool traced = is_traced(t0);
         if constexpr (!INJ && GL == 4) {
             if (!traced && use_smem && P.G > 0) { if (launch_sliced<2, GL, GUARD>(T, g, sh, smem_bytes, stream)) return; }
             else if (!traced && use_smem) { if (launch_sliced<1, GL, GUARD>(T, g, sh, smem_bytes, stream)) return; }
@@ -1196,6 +1369,98 @@ struct ChangepointSampler : SamplerImpl {
             changepoint_kernel<INJ, 0, GL, GUARD><<<g, 128, 0, stream>>>(
                 P, s->model->d_cpdata, st, s->K, T, step0, s->seed, s->chain_offset, tape, t0, sh);
     }
+    // ---- posterior summaries (CPSummary; rmn_sampler_cp_set_summary / rmn_sampler_cp_get_summary)
+    CPSummary sum{};
+    bool summary = false;
+    int64_t sum_samples = 0;        // sampled chain-steps since the last reset
+    size_t sum_smem() const { return (size_t)summary_counters(sum.G, sum.H) * 8; }
+    void free_summary() {
+        if (sum.xg) cudaFree((void*)sum.xg);
+        if (sum.khist) cudaFree(sum.khist);
+        sum = CPSummary{}; summary = false; sum_samples = 0;
+    }
+    size_t sum_count_bytes() const { return ((size_t)LANES + sum.G + 1 + (size_t)sum.G * (sum.H + 2)) * 8; }
+    int cp_set_summary(int G, const double* grid, double vlo, double vhi, int H, int64_t every) override {
+        if (G == 0) { free_summary(); return RMN_OK; }
+        if (tempered || gl != 4) {
+            rmn_set_error("posterior summaries run on the untempered changepoint sampler at 4 lanes per chain only%s",
+                          tempered ? " (this sampler is tempered)" : " (RMN_CP_GL selects another width)");
+            return RMN_ERR_UNSUPPORTED;
+        }
+        RMN_REQUIRE(G >= 1 && G <= 1024 && grid, "rmn_sampler_cp_set_summary: need 1 <= G <= 1024 grid points (got %d)", G);
+        for (int i = 0; i < G; ++i) {
+            RMN_REQUIRE(isfinite(grid[i]), "rmn_sampler_cp_set_summary: grid point %d is not finite", i);
+            RMN_REQUIRE(i == 0 || grid[i] > grid[i - 1], "rmn_sampler_cp_set_summary: the grid must be strictly increasing");
+        }
+        RMN_REQUIRE(H >= 1 && H <= 1024, "rmn_sampler_cp_set_summary: need 1 <= H <= 1024 value bins (got %d)", H);
+        const double inv = (double)H / (vhi - vlo);
+        RMN_REQUIRE(isfinite(vlo) && isfinite(vhi) && vlo < vhi && isfinite(inv) && inv > 0.0,
+                    "rmn_sampler_cp_set_summary: need a finite value range vlo < vhi");
+        RMN_REQUIRE(every >= 1 && every <= ((int64_t)1 << 62), "rmn_sampler_cp_set_summary: need 1 <= every <= 2^62");
+        free_summary();
+        CPSummary q{};
+        q.G = G; q.H = H; q.vlo = vlo; q.inv = inv; q.every = every;
+        q.GP2 = 1;
+        while (q.GP2 * 2 <= G) q.GP2 *= 2;
+        std::vector<double> tab(2 * (size_t)q.GP2, NAN);             // padded_upper_bound's table
+        std::copy(grid, grid + G, tab.begin());
+        sum = q;
+        double* d_xg = nullptr;
+        unsigned long long* d_cnt = nullptr;
+        if (cudaMalloc(&d_xg, tab.size() * 8) != cudaSuccess || cudaMalloc(&d_cnt, sum_count_bytes()) != cudaSuccess) {
+            if (d_xg) cudaFree(d_xg);
+            sum = CPSummary{};
+            rmn_set_error("rmn_sampler_cp_set_summary: device allocation failed");
+            return RMN_ERR_CUDA;
+        }
+        sum.xg = d_xg;
+        sum.khist = d_cnt; sum.cpxhist = d_cnt + LANES; sum.D = sum.cpxhist + G + 1;
+        summary = true;
+        RMN_CUDA(cudaMemcpy(d_xg, tab.data(), tab.size() * 8, cudaMemcpyHostToDevice));
+        RMN_CUDA(cudaMemset(d_cnt, 0, sum_count_bytes()));
+        if (use_smem) {
+            const size_t b = smem_bytes + sum_smem();
+            const void* kf[] = {(const void*)cp_summary_kernel<false, 1, true>, (const void*)cp_summary_kernel<false, 1, false>,
+                                (const void*)cp_summary_kernel<true, 1, true>, (const void*)cp_summary_kernel<false, 2, true>,
+                                (const void*)cp_summary_kernel<false, 2, false>, (const void*)cp_summary_kernel<true, 2, true>,
+                                (const void*)cp_summary_sliced_kernel<1, true>, (const void*)cp_summary_sliced_kernel<1, false>,
+                                (const void*)cp_summary_sliced_kernel<2, true>, (const void*)cp_summary_sliced_kernel<2, false>};
+            for (const void* f : kf) RMN_CUDA(raise_smem(f, b));
+        }
+        return RMN_OK;
+    }
+    int cp_get_summary(int64_t* d_khist, int64_t* d_cpxhist, int64_t* d_yhist, int64_t* h_nsamples,
+                       cudaStream_t stream) override {
+        RMN_REQUIRE(summary, "rmn_sampler_cp_get_summary: no summary is set (rmn_sampler_cp_set_summary)");
+        const int W = sum.H + 2, n = std::max(W, sum.G + 1);
+        cp_summary_readout_kernel<<<(unsigned)((n + 127) / 128), 128, 0, stream>>>(sum.khist, sum.cpxhist, sum.D, sum.G, W,
+                                                                                  d_khist, d_cpxhist, d_yhist);
+        RMN_KERNEL_CHECK();
+        launches++;
+        if (h_nsamples) *h_nsamples = sum_samples;
+        return RMN_OK;
+    }
+    template <bool INJ, bool GUARD>
+    void launch_summary(int64_t T, const double* tape, const rmn_trace_t& t0, cudaStream_t stream) {
+        const int sh = INJ ? 0 : shared_mv;
+        const unsigned g = run_grid(4, sh);
+        const size_t ss = sum_smem();
+        last_sliced = false;
+        if constexpr (!INJ) {
+            if (!is_traced(t0) && use_smem && P.G > 0) { if (launch_sliced<2, 4, GUARD, true>(T, g, sh, smem_bytes + ss, stream)) return; }
+            else if (!is_traced(t0) && use_smem) { if (launch_sliced<1, 4, GUARD, true>(T, g, sh, smem_bytes + ss, stream)) return; }
+        }
+        if (use_smem && P.G > 0)
+            cp_summary_kernel<INJ, 2, GUARD><<<g, 128, smem_bytes + ss, stream>>>(
+                P, sum, s->model->d_cpdata, st, s->K, T, step0, s->seed, s->chain_offset, tape, t0, sh);
+        else if (use_smem)
+            cp_summary_kernel<INJ, 1, GUARD><<<g, 128, smem_bytes + ss, stream>>>(
+                P, sum, s->model->d_cpdata, st, s->K, T, step0, s->seed, s->chain_offset, tape, t0, sh);
+        else
+            cp_summary_kernel<INJ, 0, GUARD><<<g, 128, ss, stream>>>(
+                P, sum, s->model->d_cpdata, st, s->K, T, step0, s->seed, s->chain_offset, tape, t0, sh);
+    }
+
     // tempered runs: the one-slice launch at GL = 4 (RMN_CP_GL does not apply); one ladder slot of S groups per ladder
     template <bool INJ>
     void launch_tempered(int64_t T, const rmn_inject_t* inj, const rmn_trace_t& t0, cudaStream_t stream) {
@@ -1221,10 +1486,20 @@ struct ChangepointSampler : SamplerImpl {
         if (t0.thin <= 0) t0.thin = 1;
         if (inj) RMN_REQUIRE(inj->d_tape, "injected changepoint run needs d_tape");
         if (inj && tempered) RMN_REQUIRE(inj->d_usel, "injected tempered run needs d_usel (selection uniforms)");
-        ktimer.begin(tempered ? "cp_tempered_kernel" : "changepoint_kernel", stream);
+        if (summary && tempered) {
+            rmn_set_error("posterior summaries run on the untempered changepoint sampler only");
+            return RMN_ERR_UNSUPPORTED;
+        }
+        ktimer.begin(tempered ? "cp_tempered_kernel" : (summary ? "cp_summary_kernel" : "changepoint_kernel"), stream);
         if (tempered) {
             if (inj) launch_tempered<true>(T, inj, t0, stream);
             else launch_tempered<false>(T, nullptr, t0, stream);
+        } else if (summary) {
+            // GL = 4 (cp_set_summary refuses other widths); per-chain move schedules without the guards as in launch_gl
+            if (inj) launch_summary<true, true>(T, inj->d_tape, t0, stream);
+            else if (!shared_mv && !force_guard) launch_summary<false, false>(T, nullptr, t0, stream);
+            else launch_summary<false, true>(T, nullptr, t0, stream);
+            if (last_sliced) ktimer.name = "cp_summary_sliced_kernel";
         } else if (inj) {
             launch<true>(T, inj->d_tape, t0, stream);
         } else {
@@ -1237,6 +1512,11 @@ struct ChangepointSampler : SamplerImpl {
         // samples = #{ s in [step0, step0+T) : s % EVERY == 0 }
         const int64_t E = RMN_CP_DIAG_EVERY;
         diag_samples += (step0 + T + E - 1) / E - (step0 + E - 1) / E;
+        if (summary) {
+            // every live chain at each sampled step; ceil(n / every) = #{s in [0, n) : s % every == 0} without overflow
+            auto upto = [&](int64_t n) { return n / sum.every + (n % sum.every != 0); };
+            sum_samples += s->K * (upto(step0 + T) - upto(step0));
+        }
         step0 += T; diag_steps += T;
         return RMN_OK;
     }
@@ -1247,6 +1527,10 @@ struct ChangepointSampler : SamplerImpl {
         RMN_CUDA(cudaMemsetAsync(st.dacc, 0, (size_t)s->K * 8, stream));
         RMN_CUDA(cudaMemsetAsync(st.dovf, 0, (size_t)s->K * 8, stream));
         diag_steps = 0; diag_samples = 0;
+        if (summary) {                  // the summaries cover the same window as the diagnostics
+            RMN_CUDA(cudaMemsetAsync(sum.khist, 0, sum_count_bytes(), stream));
+            sum_samples = 0;
+        }
         return RMN_OK;
     }
     int chain_sums(const double** S1, const double** S2, int64_t* n) override {

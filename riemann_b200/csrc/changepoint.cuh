@@ -74,6 +74,26 @@ __host__ __device__ __forceinline__ int bucket_of(double c, double bscale, doubl
 #endif
 }
 
+// The binary search of run_boundary over any sorted table t of n entries padded with NaN up to 2 * P2 (P2 = the largest
+// power of two <= n): #{i : t_i <= c} for R queries, in [0, n].  The posterior summaries search their grid with it.
+template <int R>
+__device__ __forceinline__ void padded_upper_bound(const double* __restrict__ t, int P2, const double (&c)[R],
+                                                   int (&pos)[R]) {
+    const char* base = (const char*)t;
+    unsigned off[R];
+#pragma unroll
+    for (int r = 0; r < R; ++r) off[r] = 0;
+    for (int step = P2; step > 0; step >>= 1) {
+        double v[R];
+#pragma unroll
+        for (int r = 0; r < R; ++r) v[r] = *(const double*)(base + off[r] + (step - 1) * 8);
+#pragma unroll
+        for (int r = 0; r < R; ++r) if (v[r] <= c[r]) off[r] += 8u * step;
+    }
+#pragma unroll
+    for (int r = 0; r < R; ++r) pos[r] = (int)(off[r] >> 3);
+}
+
 template <bool BUCKETS, int R>
 __device__ __forceinline__ void run_boundary(const CPParams& P, const double* __restrict__ xs,
                                              const double2* __restrict__ bx, const double (&c)[R], int (&pos)[R]) {
@@ -86,19 +106,7 @@ __device__ __forceinline__ void run_boundary(const CPParams& P, const double* __
             pos[r] = bstart[b] + (w.x <= c[r]) + (w.y <= c[r]);
         }
     } else {
-        const char* base = (const char*)xs;
-        unsigned off[R];
-#pragma unroll
-        for (int r = 0; r < R; ++r) off[r] = 0;
-        for (int step = P.P2; step > 0; step >>= 1) {
-            double v[R];
-#pragma unroll
-            for (int r = 0; r < R; ++r) v[r] = *(const double*)(base + off[r] + (step - 1) * 8);
-#pragma unroll
-            for (int r = 0; r < R; ++r) if (v[r] <= c[r]) off[r] += 8u * step;
-        }
-#pragma unroll
-        for (int r = 0; r < R; ++r) pos[r] = (int)(off[r] >> 3);
+        padded_upper_bound<R>(xs, P.P2, c, pos);
     }
 }
 

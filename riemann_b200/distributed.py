@@ -59,6 +59,14 @@ def reduce_block(blk):
     return blk
 
 
+def reduce_counts(t):
+    """Sum an int64 count tensor over ranks, exactly (no-op without an initialised process group)."""
+    import torch.distributed as dist
+    if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
+        dist.all_reduce(t, op=dist.ReduceOp.SUM)
+    return t
+
+
 def summarize_block(b):
     """
     b = [K, n_samples, accepts, overflows, steps, -, sum_c m_c (nd), sum_c m_c^2 (nd), sum_c v_c (nd)].

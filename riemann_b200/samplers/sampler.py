@@ -118,6 +118,8 @@ class Sampler(object):
         self._handle = h
         self.seed, self.chain_offset = int(seed), int(chain_offset)
         self.total_steps = 0
+        self._tempered = _tempering is not None
+        self._summary = None
 
         if move_schedule is not None:
             if move_schedule not in ("group", "chain"):
@@ -531,6 +533,52 @@ class Sampler(object):
         if allreduce and not self.row_sharded:      # row-sharded: every rank holds the SAME K chains, nothing to add up
             blk = reduce_block(blk)
         return summarize_block(blk.cpu().numpy())
+
+    # ------------------------------------------------------------------ posterior summaries (changepoint model)
+    def set_posterior_summary(self, grid, value_range=None, value_bins=128, every=16):
+        """
+        Accumulate posterior summaries on the device from the next run on (rmn_sampler_cp_set_summary): after every MH
+        step whose global index is a multiple of `every`, every chain's state adds to integer histograms of the number
+        of changepoints, of the changepoint locations over the cells of `grid`, and of the posterior predictive
+        ChangepointRegression1D.predict(theta, grid[g]) at every grid point over `value_bins` equal bins of
+        `value_range` = (vlo, vhi) plus an under- and an overflow bin.  No trace is kept.  The counts are reset now and
+        by reset_diagnostics, so they cover the same window as the diagnostics.  grid=None turns the summaries off.
+        Untempered changepoint samplers only.
+        """
+        if not self._is_cp or self._tempered:
+            raise ParameterError("posterior summaries are available for untempered changepoint samplers only")
+        lib = _lib.load()
+        if grid is None:
+            _lib.check(lib.rmn_sampler_cp_set_summary(self._handle, 0, None, 0.0, 0.0, 0, 0))
+            self._summary = None
+            return
+        from ..posterior_summary import check_summary_args
+        g, vlo, vhi, H, every = check_summary_args(grid, value_range, value_bins, every)
+        _lib.check(lib.rmn_sampler_cp_set_summary(self._handle, len(g), _lib.ptr(g), vlo, vhi, H, every))
+        self._summary = (g, vlo, vhi, H)
+
+    def posterior_summary(self, allreduce=True):
+        """
+        The summary counts since the last reset as a PosteriorSummary (riemann_b200/posterior_summary.py): grid,
+        value_edges, khist, cpxhist, yhist, nsamples, and the binned estimates yhat_mean / yhat_quantiles(q).  With
+        torch.distributed initialised the int64 counts are summed over the ranks (their chains are disjoint shards).
+        """
+        if self._summary is None:
+            raise ParameterError("no posterior summary is set (set_posterior_summary)")
+        from ..distributed import reduce_counts
+        from ..posterior_summary import PosteriorSummary
+        torch, (g, vlo, vhi, H) = self._torch, self._summary
+        G, L = len(g), _lib.CP_LANES
+        buf = torch.zeros(1 + L + (G + 1) + G * (H + 2), dtype=torch.int64, device="cuda")
+        ns = C.c_int64()
+        _lib.check(_lib.load().rmn_sampler_cp_get_summary(
+            self._handle, C.c_void_p(buf.data_ptr() + 8), C.c_void_p(buf.data_ptr() + 8 * (1 + L)),
+            C.c_void_p(buf.data_ptr() + 8 * (2 + L + G)), C.byref(ns), _lib.stream_ptr()))
+        buf[0] = ns.value
+        if allreduce:
+            buf = reduce_counts(buf)
+        c = buf.cpu().numpy()
+        return PosteriorSummary(g, vlo, vhi, c[1:1 + L], c[1 + L:2 + L + G], c[2 + L + G:].reshape(G, H + 2), c[0])
 
     # ------------------------------------------------------------------ trace wire format (SURVEY 8f N4)
     def save_trace(self, path):
