@@ -356,6 +356,15 @@ int rmn_sampler_cp_set_summary(rmn_sampler_t* s, int G, const double* h_grid, do
 int rmn_sampler_cp_get_summary(rmn_sampler_t* s, int64_t* d_khist, int64_t* d_cpxhist, int64_t* d_yhist,
                                int64_t* h_nsamples, void* stream);
 
+/* The same summaries for a tempered changepoint sampler (rmn_sampler_set_tempering): only the chain of rung `rung`
+ * (inverse temperature h_betas[rung]) of every ladder is sampled, in its state after the step's swaps, so the count of
+ * sampled chain-steps grows by K / nt per sampled step.  Same arguments and checks as rmn_sampler_cp_set_summary plus
+ * 0 <= rung < nt; G = 0 turns the summaries off.  The counts are read with rmn_sampler_cp_get_summary and zeroed by
+ * rmn_sampler_reset_diagnostics; the chains are unchanged bit for bit.  Untempered samplers and other model families:
+ * RMN_ERR_UNSUPPORTED (rmn_sampler_cp_set_summary serves the untempered changepoint sampler, and refuses tempered ones). */
+int rmn_sampler_cp_set_rung_summary(rmn_sampler_t* s, int rung, int G, const double* h_grid, double vlo, double vhi,
+                                    int H, int64_t every);
+
 /* Number of kernel launches this handle has enqueued so far. */
 int64_t rmn_sampler_launch_count(const rmn_sampler_t* s);
 

@@ -538,6 +538,12 @@ extern "C" int rmn_sampler_cp_set_summary(rmn_sampler_t* s, int G, const double*
     return s->impl->cp_set_summary(G, h_grid, vlo, vhi, H, every);
 }
 
+extern "C" int rmn_sampler_cp_set_rung_summary(rmn_sampler_t* s, int rung, int G, const double* h_grid, double vlo,
+                                               double vhi, int H, int64_t every) {
+    RMN_REQUIRE(s && s->impl, "rmn_sampler_cp_set_rung_summary: null sampler");
+    return s->impl->cp_set_rung_summary(rung, G, h_grid, vlo, vhi, H, every);
+}
+
 extern "C" int rmn_sampler_cp_get_summary(rmn_sampler_t* s, int64_t* d_khist, int64_t* d_cpxhist, int64_t* d_yhist,
                                           int64_t* h_nsamples, void* stream) {
     NvtxRange nvtx_("rmn_sampler_cp_get_summary");

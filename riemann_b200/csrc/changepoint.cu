@@ -387,14 +387,15 @@ __device__ __forceinline__ void summary_sample(const CPSummary& S, unsigned long
 // TEMPER: the ladder layout and the swap moves of cp_tempered_kernel (tp, usel_tape); every addition sits under
 // `if constexpr`, so the untempered instantiations are unchanged.
 // SUMMARY: the posterior summaries of the cp_summary kernels (sp, and ssum = the block's shared counters, see CPSummary),
-// likewise under `if constexpr`.
+// likewise under `if constexpr`.  TEMPER and SUMMARY together (cp_tempered_summary_kernel): only the chains of rung
+// `rung` are sampled.
 template <bool INJ, int DATA, int GL, bool GUARD, bool TEMPER = false, typename IT = int64_t, bool SUMMARY = false>
 __device__ __forceinline__ void cp_block(const CPParams& P, const double* __restrict__ xs, CPState st,
                                          int64_t K, int64_t t_begin, IT nt, int64_t step0, uint64_t seed,
                                          int64_t chain_offset, const double* __restrict__ tape, const rmn_trace_t& tr,
                                          int shared_mv, int64_t blk, const CPTemper* tp = nullptr,
                                          const double* __restrict__ usel_tape = nullptr, const CPSummary* sp = nullptr,
-                                         unsigned long long* ssum = nullptr) {
+                                         unsigned long long* ssum = nullptr, int rung = 0) {
     // iterations [t_begin, t_begin + nt) of the launch for the 128 / GL chains of block `blk`; the chain state is read from and
     // written back to global memory (L2-coherent loads: in the time-sliced kernel another SM wrote it)
     constexpr int EPL = Geo<GL>::EPL;
@@ -467,6 +468,11 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
     }
     double beta = 1.0;                                // this rung's inverse temperature
     if constexpr (TEMPER) beta = tp->betas[min(ti, tp->nt - 1)];
+    // the tempered summary kernel reads it and the rung from slots of the group in shared memory: at 128 registers the
+    // three they take across the T loop are what the summary sampling would spill
+    __shared__ double s_beta[(TEMPER && SUMMARY) ? 128 / GL : 1];
+    __shared__ int s_ti[(TEMPER && SUMMARY) ? 128 / GL : 1];
+    if constexpr (TEMPER && SUMMARY) { s_beta[g] = beta; s_ti[g] = ti; }
     // diagnostics sums: lane l, slot s holds functional l + GL*s of the chain.  They stay in shared memory for the
     // launch (no registers across the T loop) and every sample is added to the running sum in time order, so the sums
     // do not depend on how the launch is sliced.
@@ -561,14 +567,17 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
         bool is_init = false, is_part = false, regular = true;
         if constexpr (TEMPER) {
             const double usel = INJ ? usel_tape[t * K + c] : u01_fast(rk.block(step, (uint32_t)(2 * GL + lane)).x);
-            const bool want = live && lane == 0 && ti < tp->nt - 1 && !(usel > tp->pswap);
-            const int base = ((threadIdx.x & 31) / GL) & ~(tp->S - 1);      // the ladder's first group in the warp
+            const int ri = SUMMARY ? s_ti[g] : ti;      // this group's rung
+            const bool want = live && lane == 0 && ri < tp->nt - 1 && !(usel > tp->pswap);
+            // the ladder's first group in the warp (the summary kernel: the group's index in the warp minus its rung,
+            // from the shared slot, so that the shift below is not held across the T loop)
+            const int base = SUMMARY ? ((threadIdx.x & 31) / GL) - ri : ((threadIdx.x & 31) / GL) & ~(tp->S - 1);
             const unsigned wb = __ballot_sync(FULL, want) >> (base * GL);
             unsigned init = 0;
             for (int b = 0; b < tp->nt - 1; ++b)
                 if (((wb >> (b * GL)) & 1u) && !(b > 0 && ((init >> (b - 1)) & 1u))) init |= 1u << b;
-            is_init = live && ((init >> ti) & 1u);
-            is_part = live && ti > 0 && ((init >> (ti - 1)) & 1u);
+            is_init = live && ((init >> ri) & 1u);
+            is_part = live && ri > 0 && ((init >> (ri - 1)) & 1u);
             regular = !is_init && !is_part;
         }
         // What the warp as a whole needs this step (warp-uniform).  With a shared move schedule all chains of the
@@ -724,7 +733,7 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
             // TemperedModel (ptsampler.py:33-37): combine(log_prior, beta * log_likelihood); beta = 0 times -inf is nan -> -inf
             nll = cp_assemble(P, kk, sss, nvt, nlg, nsig, nls2, 1);
             nlpr = cp_assemble(P, kk, sss, nvt, nlg, nsig, nls2, 2);
-            lpn = combine_logpost(nlpr, __dmul_rn(beta, nll));
+            lpn = combine_logpost(nlpr, __dmul_rn((TEMPER && SUMMARY) ? s_beta[g] : beta, nll));
         } else {
             lpn = cp_assemble(P, kk, sss, nvt, nlg, nsig, nls2, 0);
         }
@@ -756,9 +765,10 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
                 const int go = is_init ? g + 1 : (is_part ? g - 1 : g);         // the partner's slot
                 const double ll_i = s_ll[g], lpr_i = s_lpr[g];
                 const double ll_o = s_ll[go], lpr_o = s_lpr[go], ss_o = s_ss[go], vt_o = s_vt[go], lg_o = s_lg[go];
-                const double beta_o = tp->betas[min(ti + 1, tp->nt - 1)];
+                const int ri = SUMMARY ? s_ti[g] : ti;
+                const double beta_o = tp->betas[min(ri + 1, tp->nt - 1)];
                 const double lp_jj = __shfl_down_sync(FULL, lp, GL);
-                const double lp_ij = combine_logpost(lpr_o, __dmul_rn(beta, ll_o));      // model_i at theta_j
+                const double lp_ij = combine_logpost(lpr_o, __dmul_rn((TEMPER && SUMMARY) ? s_beta[g] : beta, ll_o));   // model_i at theta_j
                 const double lp_ji = combine_logpost(lpr_i, __dmul_rn(beta_o, ll_i));    // model_j at theta_i
                 const double x = exp((lp_ji + lp_ij) - (lp + lp_jj));
                 const double mhr = (x < 1.0) ? x : 1.0;                                  // Python min(1, x): nan -> 1
@@ -816,7 +826,10 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
             if ((long long)step == s_snext[threadIdx.x]) {  // warp-uniform
                 s_snext[threadIdx.x] += sp->every;
                 __syncwarp();                               // the rows as the other lanes accepted them
-                summary_sample<GL>(*sp, ssum, s_cx, s_cv, lane, k, s_chain[g] >= 0);
+                // tempered: the group's rung is its index in the ladder slot (a block holds whole slots); the state is
+                // the one after this step's swaps
+                const bool sampled = s_chain[g] >= 0 && (!TEMPER || (g & (tp->S - 1)) == rung);
+                summary_sample<GL>(*sp, ssum, s_cx, s_cv, lane, k, sampled);
                 __syncwarp();                               // every lane has read the rows before the next step writes
             }
         }
@@ -1042,6 +1055,31 @@ cp_tempered_kernel(const __grid_constant__ CPParams P, const __grid_constant__ C
     }
     cp_block<INJ, DATA, 4, true, true>(P, xs, st, K, 0, T, step0, seed, chain_offset, tape, tr, shared_mv, blockIdx.x,
                                        &TP, usel);
+}
+
+// cp_tempered_kernel with the posterior summaries of rung `rung` of every ladder compiled in (rmn_sampler_cp_set_rung_summary):
+// the groups of that rung are sampled after the step's swaps, the others pass `live` = false to summary_sample (the
+// sampled-step test stays warp-uniform).  `rung` is an argument of its own, so CPTemper and CPSummary, and with them the
+// parameter layout of the other kernels, stay as they are.  Dynamic shared memory as in cp_summary_kernel.  The chains
+// are those of cp_tempered_kernel bit for bit.
+template <bool INJ, int DATA>
+__global__ void __launch_bounds__(128, RMN_CP_MINBLOCKS)
+cp_tempered_summary_kernel(const __grid_constant__ CPParams P, const __grid_constant__ CPTemper TP,
+                           const __grid_constant__ CPSummary SP, int rung, const double* __restrict__ gdata, CPState st,
+                           int64_t K, int64_t T, int64_t step0, uint64_t seed, int64_t chain_offset,
+                           const double* __restrict__ tape, const double* __restrict__ usel, rmn_trace_t tr,
+                           int shared_mv) {
+    extern __shared__ double smem[];
+    const double* xs = gdata;
+    const int n = (DATA != 0) ? P.XP + 2 * P.M + 2 + ((DATA == 2) ? P.G * 5 / 2 : 0) : 0;
+    if (DATA != 0) {
+        for (int i = threadIdx.x; i < n; i += blockDim.x) smem[i] = gdata[i];
+        __syncthreads();
+        xs = smem;
+    }
+    cp_block<INJ, DATA, 4, true, true, int64_t, true>(P, xs, st, K, 0, T, step0, seed, chain_offset, tape, tr, shared_mv,
+                                                       blockIdx.x, &TP, usel, &SP,
+                                                       reinterpret_cast<unsigned long long*>(smem + n), rung);
 }
 
 // evaluate n states given in the canonical layout (pointwise parity entry + set_state); tempered (tp != nullptr): the
@@ -1373,11 +1411,12 @@ struct ChangepointSampler : SamplerImpl {
     CPSummary sum{};
     bool summary = false;
     int64_t sum_samples = 0;        // sampled chain-steps since the last reset
+    int sum_rung = -1;              // tempered: the rung whose chains are sampled (rmn_sampler_cp_set_rung_summary)
     size_t sum_smem() const { return (size_t)summary_counters(sum.G, sum.H) * 8; }
     void free_summary() {
         if (sum.xg) cudaFree((void*)sum.xg);
         if (sum.khist) cudaFree(sum.khist);
-        sum = CPSummary{}; summary = false; sum_samples = 0;
+        sum = CPSummary{}; summary = false; sum_samples = 0; sum_rung = -1;
     }
     size_t sum_count_bytes() const { return ((size_t)LANES + sum.G + 1 + (size_t)sum.G * (sum.H + 2)) * 8; }
     int cp_set_summary(int G, const double* grid, double vlo, double vhi, int H, int64_t every) override {
@@ -1387,16 +1426,51 @@ struct ChangepointSampler : SamplerImpl {
                           tempered ? " (this sampler is tempered)" : " (RMN_CP_GL selects another width)");
             return RMN_ERR_UNSUPPORTED;
         }
-        RMN_REQUIRE(G >= 1 && G <= 1024 && grid, "rmn_sampler_cp_set_summary: need 1 <= G <= 1024 grid points (got %d)", G);
-        for (int i = 0; i < G; ++i) {
-            RMN_REQUIRE(isfinite(grid[i]), "rmn_sampler_cp_set_summary: grid point %d is not finite", i);
-            RMN_REQUIRE(i == 0 || grid[i] > grid[i - 1], "rmn_sampler_cp_set_summary: the grid must be strictly increasing");
+        const int e = alloc_summary("rmn_sampler_cp_set_summary", G, grid, vlo, vhi, H, every);
+        if (e != RMN_OK) return e;
+        if (use_smem) {
+            const size_t b = smem_bytes + sum_smem();
+            const void* kf[] = {(const void*)cp_summary_kernel<false, 1, true>, (const void*)cp_summary_kernel<false, 1, false>,
+                                (const void*)cp_summary_kernel<true, 1, true>, (const void*)cp_summary_kernel<false, 2, true>,
+                                (const void*)cp_summary_kernel<false, 2, false>, (const void*)cp_summary_kernel<true, 2, true>,
+                                (const void*)cp_summary_sliced_kernel<1, true>, (const void*)cp_summary_sliced_kernel<1, false>,
+                                (const void*)cp_summary_sliced_kernel<2, true>, (const void*)cp_summary_sliced_kernel<2, false>};
+            for (const void* f : kf) RMN_CUDA(raise_smem(f, b));
         }
-        RMN_REQUIRE(H >= 1 && H <= 1024, "rmn_sampler_cp_set_summary: need 1 <= H <= 1024 value bins (got %d)", H);
+        return RMN_OK;
+    }
+    // tempered samplers: the summaries of the chains of one rung of every ladder (cp_tempered_summary_kernel)
+    int cp_set_rung_summary(int rung, int G, const double* grid, double vlo, double vhi, int H, int64_t every) override {
+        if (!tempered) {
+            rmn_set_error("rung summaries run on tempered changepoint samplers only (rmn_sampler_cp_set_summary serves "
+                          "untempered ones)");
+            return RMN_ERR_UNSUPPORTED;
+        }
+        if (G == 0) { free_summary(); return RMN_OK; }
+        RMN_REQUIRE(rung >= 0 && rung < tp.nt, "rmn_sampler_cp_set_rung_summary: need 0 <= rung < %d (got %d)", tp.nt, rung);
+        const int e = alloc_summary("rmn_sampler_cp_set_rung_summary", G, grid, vlo, vhi, H, every);
+        if (e != RMN_OK) return e;
+        sum_rung = rung;
+        if (use_smem) {
+            const size_t b = smem_bytes + sum_smem();
+            const void* kf[] = {(const void*)cp_tempered_summary_kernel<false, 1>, (const void*)cp_tempered_summary_kernel<true, 1>,
+                                (const void*)cp_tempered_summary_kernel<false, 2>, (const void*)cp_tempered_summary_kernel<true, 2>};
+            for (const void* f : kf) RMN_CUDA(raise_smem(f, b));
+        }
+        return RMN_OK;
+    }
+    // the checks and buffers common to both entries (fn: the entry's name in the error messages); resets the counts
+    int alloc_summary(const char* fn, int G, const double* grid, double vlo, double vhi, int H, int64_t every) {
+        RMN_REQUIRE(G >= 1 && G <= 1024 && grid, "%s: need 1 <= G <= 1024 grid points (got %d)", fn, G);
+        for (int i = 0; i < G; ++i) {
+            RMN_REQUIRE(isfinite(grid[i]), "%s: grid point %d is not finite", fn, i);
+            RMN_REQUIRE(i == 0 || grid[i] > grid[i - 1], "%s: the grid must be strictly increasing", fn);
+        }
+        RMN_REQUIRE(H >= 1 && H <= 1024, "%s: need 1 <= H <= 1024 value bins (got %d)", fn, H);
         const double inv = (double)H / (vhi - vlo);
         RMN_REQUIRE(isfinite(vlo) && isfinite(vhi) && vlo < vhi && isfinite(inv) && inv > 0.0,
-                    "rmn_sampler_cp_set_summary: need a finite value range vlo < vhi");
-        RMN_REQUIRE(every >= 1 && every <= ((int64_t)1 << 62), "rmn_sampler_cp_set_summary: need 1 <= every <= 2^62");
+                    "%s: need a finite value range vlo < vhi", fn);
+        RMN_REQUIRE(every >= 1 && every <= ((int64_t)1 << 62), "%s: need 1 <= every <= 2^62", fn);
         free_summary();
         CPSummary q{};
         q.G = G; q.H = H; q.vlo = vlo; q.inv = inv; q.every = every;
@@ -1410,7 +1484,7 @@ struct ChangepointSampler : SamplerImpl {
         if (cudaMalloc(&d_xg, tab.size() * 8) != cudaSuccess || cudaMalloc(&d_cnt, sum_count_bytes()) != cudaSuccess) {
             if (d_xg) cudaFree(d_xg);
             sum = CPSummary{};
-            rmn_set_error("rmn_sampler_cp_set_summary: device allocation failed");
+            rmn_set_error("%s: device allocation failed", fn);
             return RMN_ERR_CUDA;
         }
         sum.xg = d_xg;
@@ -1418,15 +1492,6 @@ struct ChangepointSampler : SamplerImpl {
         summary = true;
         RMN_CUDA(cudaMemcpy(d_xg, tab.data(), tab.size() * 8, cudaMemcpyHostToDevice));
         RMN_CUDA(cudaMemset(d_cnt, 0, sum_count_bytes()));
-        if (use_smem) {
-            const size_t b = smem_bytes + sum_smem();
-            const void* kf[] = {(const void*)cp_summary_kernel<false, 1, true>, (const void*)cp_summary_kernel<false, 1, false>,
-                                (const void*)cp_summary_kernel<true, 1, true>, (const void*)cp_summary_kernel<false, 2, true>,
-                                (const void*)cp_summary_kernel<false, 2, false>, (const void*)cp_summary_kernel<true, 2, true>,
-                                (const void*)cp_summary_sliced_kernel<1, true>, (const void*)cp_summary_sliced_kernel<1, false>,
-                                (const void*)cp_summary_sliced_kernel<2, true>, (const void*)cp_summary_sliced_kernel<2, false>};
-            for (const void* f : kf) RMN_CUDA(raise_smem(f, b));
-        }
         return RMN_OK;
     }
     int cp_get_summary(int64_t* d_khist, int64_t* d_cpxhist, int64_t* d_yhist, int64_t* h_nsamples,
@@ -1470,6 +1535,19 @@ struct ChangepointSampler : SamplerImpl {
         const unsigned g = (unsigned)(((L + head) * tp.S * 4 + 127) / 128);
         const double* tape = INJ ? inj->d_tape : nullptr;
         const double* usel = INJ ? inj->d_usel : nullptr;
+        if (summary) {
+            const size_t ss = sum_smem();
+            if (use_smem && P.G > 0)
+                cp_tempered_summary_kernel<INJ, 2><<<g, 128, smem_bytes + ss, stream>>>(
+                    P, tp, sum, sum_rung, s->model->d_cpdata, st, s->K, T, step0, s->seed, s->chain_offset, tape, usel, t0, sh);
+            else if (use_smem)
+                cp_tempered_summary_kernel<INJ, 1><<<g, 128, smem_bytes + ss, stream>>>(
+                    P, tp, sum, sum_rung, s->model->d_cpdata, st, s->K, T, step0, s->seed, s->chain_offset, tape, usel, t0, sh);
+            else
+                cp_tempered_summary_kernel<INJ, 0><<<g, 128, ss, stream>>>(
+                    P, tp, sum, sum_rung, s->model->d_cpdata, st, s->K, T, step0, s->seed, s->chain_offset, tape, usel, t0, sh);
+            return;
+        }
         if (use_smem && P.G > 0)
             cp_tempered_kernel<INJ, 2><<<g, 128, smem_bytes, stream>>>(
                 P, tp, s->model->d_cpdata, st, s->K, T, step0, s->seed, s->chain_offset, tape, usel, t0, sh);
@@ -1486,11 +1564,12 @@ struct ChangepointSampler : SamplerImpl {
         if (t0.thin <= 0) t0.thin = 1;
         if (inj) RMN_REQUIRE(inj->d_tape, "injected changepoint run needs d_tape");
         if (inj && tempered) RMN_REQUIRE(inj->d_usel, "injected tempered run needs d_usel (selection uniforms)");
-        if (summary && tempered) {
-            rmn_set_error("posterior summaries run on the untempered changepoint sampler only");
+        if (summary && tempered && sum_rung < 0) {
+            rmn_set_error("posterior summaries of a tempered sampler are those of one rung (rmn_sampler_cp_set_rung_summary)");
             return RMN_ERR_UNSUPPORTED;
         }
-        ktimer.begin(tempered ? "cp_tempered_kernel" : (summary ? "cp_summary_kernel" : "changepoint_kernel"), stream);
+        ktimer.begin(tempered ? (summary ? "cp_tempered_summary_kernel" : "cp_tempered_kernel")
+                              : (summary ? "cp_summary_kernel" : "changepoint_kernel"), stream);
         if (tempered) {
             if (inj) launch_tempered<true>(T, inj, t0, stream);
             else launch_tempered<false>(T, nullptr, t0, stream);
@@ -1513,9 +1592,10 @@ struct ChangepointSampler : SamplerImpl {
         const int64_t E = RMN_CP_DIAG_EVERY;
         diag_samples += (step0 + T + E - 1) / E - (step0 + E - 1) / E;
         if (summary) {
-            // every live chain at each sampled step; ceil(n / every) = #{s in [0, n) : s % every == 0} without overflow
+            // every live chain (tempered: one per ladder, the chain of rung sum_rung) at each sampled step;
+            // ceil(n / every) = #{s in [0, n) : s % every == 0} without overflow
             auto upto = [&](int64_t n) { return n / sum.every + (n % sum.every != 0); };
-            sum_samples += s->K * (upto(step0 + T) - upto(step0));
+            sum_samples += (tempered ? s->K / tp.nt : s->K) * (upto(step0 + T) - upto(step0));
         }
         step0 += T; diag_steps += T;
         return RMN_OK;

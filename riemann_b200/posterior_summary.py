@@ -1,7 +1,8 @@
 """
-Posterior summaries of the changepoint sampler, accumulated on the device (rmn_sampler_cp_set_summary): integer
-histograms of the number of changepoints, of the changepoint locations on a grid, and of the posterior predictive
-ŷ(x) = ChangepointRegression1D.predict(theta, x) at every grid point, binned on a value range.  The counts are exact and
+Posterior summaries of the changepoint sampler, accumulated on the device (rmn_sampler_cp_set_summary; for one rung of
+PTSampler's tempering ladders, rmn_sampler_cp_set_rung_summary): integer histograms of the number of changepoints, of
+the changepoint locations on a grid, and of the posterior predictive ŷ(x) = ChangepointRegression1D.predict(theta, x)
+at every grid point, binned on a value range.  The counts are exact and
 do not depend on how a run is split into calls, kernels, time slices or chain shards; the means and quantiles derived
 from them here are binned estimates.
 """
@@ -36,7 +37,7 @@ def check_summary_args(grid, value_range, value_bins, every):
 
 class PosteriorSummary(object):
     """
-    Counts since the last reset (Sampler.posterior_summary):
+    Counts since the last reset (Sampler.posterior_summary, PTSampler.posterior_summary):
       grid [G], value_edges [H + 1] (bin b = 1..H of yhist covers [value_edges[b-1], value_edges[b])),
       khist [16] (number of changepoints 0..15), cpxhist [G + 1] (cell i holds changepoints x with
       grid[i-1] <= x < grid[i], cell 0 those below grid[0] and cell G those at or above grid[-1]),

@@ -26,8 +26,10 @@ ChangepointRegression1DProp on the changepoint model).
 """
 import numpy as np
 
+from .. import _lib
 from ..models.changepoint import ChangepointParams, ChangepointRegression1D, unpack_state
 from ..models.model import Model
+from ..posterior_summary import check_summary_args
 from ..sampling_errors import ParameterError
 from .sampler import ChangepointTrace, Sampler
 
@@ -104,6 +106,7 @@ class PTSampler(object):
                 raise ParameterError("theta0 must be (d,), (K, d) or (K*Nt, d)")
         self._sampler = Sampler(model, proposal, th0, K=self.K * self.Nt, seed=seed, chain_offset=chain_offset * self.Nt,
                                 _tempering=(self.betas, Pswap), move_schedule=move_schedule)
+        self._summary, self.summary_rung = None, None
         self.d = self._sampler.d
         self._thetas, self._logpost = [], []
         self._take_record(0)
@@ -170,6 +173,50 @@ class PTSampler(object):
     def sample(self):
         self.run(1)
         return [s.current_state() for s in self.samplers]
+
+    def reset_diagnostics(self):
+        """Zero the device accumulators of every rung: the diagnostics and the posterior-summary counts."""
+        self._sampler.reset_diagnostics()
+
+    # ------------------------------------------------------------------ posterior summaries (changepoint model)
+    def set_posterior_summary(self, grid, value_range=None, value_bins=128, every=16, rung=0):
+        """
+        Accumulate the posterior summaries of `Sampler.set_posterior_summary` (riemann_b200/posterior_summary.py) for the
+        chains of ONE temperature, inverse temperature betas[rung], of every ladder (rmn_sampler_cp_set_rung_summary):
+        after every PT step whose global index is a multiple of `every`, each ladder's rung-`rung` state -- as it
+        stands after that step's swaps -- adds to the integer histograms of the number of changepoints, of the
+        changepoint locations over the cells of `grid`, and of ChangepointRegression1D.predict(theta, grid[g]) over
+        `value_bins` bins of `value_range` = (vlo, vhi) plus an under- and an overflow bin.  No trace is kept.  The
+        default rung 0 is the beta = betas[0] chain, the one this sampler exposes as `_chain_thetas` and whose moments
+        `diagnostics()` reports; the other rungs sample tempered distributions.  The counts are reset now and by
+        reset_diagnostics.  grid=None turns the summaries off.  Changepoint model only; the chains are unchanged bit
+        for bit.
+        """
+        if not self._is_cp:
+            raise ParameterError("posterior summaries are available on the changepoint model only")
+        lib = _lib.load()
+        if grid is None:
+            _lib.check(lib.rmn_sampler_cp_set_rung_summary(self._sampler._handle, 0, 0, None, 0.0, 0.0, 0, 0))
+            self._summary = None
+            return
+        if isinstance(rung, bool) or int(rung) != rung or not 0 <= int(rung) < self.Nt:
+            raise ParameterError("rung must be an integer in 0..{} (got {})".format(self.Nt - 1, rung))
+        g, vlo, vhi, H, every = check_summary_args(grid, value_range, value_bins, every)
+        _lib.check(lib.rmn_sampler_cp_set_rung_summary(self._sampler._handle, int(rung), len(g), _lib.ptr(g), vlo, vhi,
+                                                       H, every))
+        self._summary = (g, vlo, vhi, H)
+        self.summary_rung = int(rung)
+
+    def posterior_summary(self, allreduce=True):
+        """
+        The summary counts of rung `summary_rung` (0: the beta = betas[0] chains of `_chain_thetas` and `diagnostics()`)
+        since the last reset, as a PosteriorSummary; nsamples counts ladders x sampled steps.  With torch.distributed
+        initialised the int64 counts are summed over the ranks: ladders on different ranks are disjoint replicas, so
+        the sum is the pooled summary.
+        """
+        if self._summary is None:
+            raise ParameterError("no posterior summary is set (set_posterior_summary)")
+        return self._sampler._read_summary(self._summary, allreduce)
 
     def diagnostics(self, allreduce=True):
         """Posterior summaries of the beta = betas[0] chains ONLY (one per ladder): the device accumulators hold every

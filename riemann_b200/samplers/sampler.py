@@ -543,7 +543,7 @@ class Sampler(object):
         ChangepointRegression1D.predict(theta, grid[g]) at every grid point over `value_bins` equal bins of
         `value_range` = (vlo, vhi) plus an under- and an overflow bin.  No trace is kept.  The counts are reset now and
         by reset_diagnostics, so they cover the same window as the diagnostics.  grid=None turns the summaries off.
-        Untempered changepoint samplers only.
+        Untempered changepoint samplers only (PTSampler.set_posterior_summary serves one rung of a tempering ladder).
         """
         if not self._is_cp or self._tempered:
             raise ParameterError("posterior summaries are available for untempered changepoint samplers only")
@@ -565,9 +565,14 @@ class Sampler(object):
         """
         if self._summary is None:
             raise ParameterError("no posterior summary is set (set_posterior_summary)")
+        return self._read_summary(self._summary, allreduce)
+
+    def _read_summary(self, spec, allreduce):
+        """The device counts (rmn_sampler_cp_get_summary) as a PosteriorSummary; spec = (grid, vlo, vhi, H) as set.
+        Shared by posterior_summary and PTSampler.posterior_summary."""
         from ..distributed import reduce_counts
         from ..posterior_summary import PosteriorSummary
-        torch, (g, vlo, vhi, H) = self._torch, self._summary
+        torch, (g, vlo, vhi, H) = self._torch, spec
         G, L = len(g), _lib.CP_LANES
         buf = torch.zeros(1 + L + (G + 1) + G * (H + 2), dtype=torch.int64, device="cuda")
         ns = C.c_int64()
