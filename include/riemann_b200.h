@@ -241,7 +241,8 @@ int rmn_sampler_get_adaptcov(rmn_sampler_t* s, double* d_L, void* stream);
  * takes a within-chain MH step or, with probability pswap and sequentially along the ladder exactly as :102-125,
  * proposes a swap with its lower neighbour.  K and chain_offset must be multiples of nt (2..32, 2..8 on the changepoint
  * model); non-adaptive RW / pCN proposals, or the changepoint proposal.
- * Call before rmn_sampler_set_state. */
+ * Call before rmn_sampler_set_state.  On the changepoint model the kernel also counts swap acceptance per pair and the
+ * replicas' round trips along the ladder: rmn_sampler_cp_get_swap_stats. */
 int rmn_sampler_set_tempering(rmn_sampler_t* s, int nt, const double* h_betas, double pswap);
 
 /* = emcee.autocorr.integrated_time(chain) as called at examples/test_randomwalk.py:42 ("steps per independent sample"),
@@ -364,6 +365,20 @@ int rmn_sampler_cp_get_summary(rmn_sampler_t* s, int64_t* d_khist, int64_t* d_cp
  * RMN_ERR_UNSUPPORTED (rmn_sampler_cp_set_summary serves the untempered changepoint sampler, and refuses tempered ones). */
 int rmn_sampler_cp_set_rung_summary(rmn_sampler_t* s, int rung, int G, const double* h_grid, double vlo, double vhi,
                                     int H, int64_t every);
+
+/* Swap statistics of a tempered changepoint sampler (rmn_sampler_set_tempering) since the last
+ * rmn_sampler_reset_diagnostics, pooled over its ladders, int64 device arrays (any may be NULL):
+ *   d_proposed[nt-1], d_accepted[nt-1]  swaps initiated by rung i with rung i+1 / taken;
+ *   d_up[nt], d_down[nt]                at every step s with s % RMN_CP_DIAG_EVERY == 0, chains at rung i whose
+ *                                       replica last touched rung 0 / rung nt-1;
+ *   d_round_trips[1]                    replicas that went from rung 0 to rung nt-1 and back to rung 0.
+ * A replica's direction travels with its state; rmn_sampler_cp_set_state starts the walk (rung 0 up, rung nt-1 down,
+ * the others neither), and rmn_sampler_reset_diagnostics zeroes the counts but keeps the directions, so a trip in
+ * progress still completes.  Integer counts: identical for any split of a run into calls and any sharding of the
+ * ladders.  Enqueued on `stream`.  The chains are unchanged by the counting.  Untempered samplers and other model
+ * families: RMN_ERR_UNSUPPORTED. */
+int rmn_sampler_cp_get_swap_stats(rmn_sampler_t* s, int64_t* d_proposed, int64_t* d_accepted, int64_t* d_up,
+                                  int64_t* d_down, int64_t* d_round_trips, void* stream);
 
 /* Number of kernel launches this handle has enqueued so far. */
 int64_t rmn_sampler_launch_count(const rmn_sampler_t* s);

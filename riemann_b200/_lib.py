@@ -84,6 +84,7 @@ SIGNATURES = {
     "rmn_sampler_cp_set_summary": (_I, [_P, _I, _P, _D, _D, _I, _L]),
     "rmn_sampler_cp_get_summary": (_I, [_P, _P, _P, _P, _P, _P]),
     "rmn_sampler_cp_set_rung_summary": (_I, [_P, _I, _I, _P, _D, _D, _I, _L]),
+    "rmn_sampler_cp_get_swap_stats": (_I, [_P, _P, _P, _P, _P, _P, _P]),
     "rmn_sampler_set_tempering": (_I, [_P, _I, _P, _D]),
     "rmn_autocorr_tau": (_I, [_P, _L, _L, _L, _D, _P, _P, _P]),
     "rmn_nccl_unique_id": (_I, [_P, C.c_size_t]),

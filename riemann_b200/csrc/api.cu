@@ -551,6 +551,12 @@ extern "C" int rmn_sampler_cp_get_summary(rmn_sampler_t* s, int64_t* d_khist, in
     return s->impl->cp_get_summary(d_khist, d_cpxhist, d_yhist, h_nsamples, (cudaStream_t)stream);
 }
 
+extern "C" int rmn_sampler_cp_get_swap_stats(rmn_sampler_t* s, int64_t* d_proposed, int64_t* d_accepted, int64_t* d_up,
+                                             int64_t* d_down, int64_t* d_round_trips, void* stream) {
+    RMN_REQUIRE(s && s->impl, "rmn_sampler_cp_get_swap_stats: null sampler");
+    return s->impl->cp_get_swap_stats(d_proposed, d_accepted, d_up, d_down, d_round_trips, (cudaStream_t)stream);
+}
+
 extern "C" int rmn_sampler_chain_moments(rmn_sampler_t* s, double* d_mean, double* d_var, void* stream) {
     RMN_REQUIRE(s && s->impl, "rmn_sampler_chain_moments: null sampler");
     const double *S1 = nullptr, *S2 = nullptr;

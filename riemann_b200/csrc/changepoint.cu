@@ -317,7 +317,20 @@ struct CPTemper {
     double pswap;
     int nt;                     // temperatures, 2..8
     int S;                      // groups a ladder occupies: the power of two >= nt
+    uint8_t* dir;               // [K] direction label of the replica each chain holds (CP_DIR_*), in the workspace
+    unsigned long long* swaps;  // [CP_SWAP_COUNTERS] swap statistics since the last reset (rmn_sampler_cp_get_swap_stats)
 };
+// Swap statistics, pooled over the ladders.  A replica's label is UP once it last touched rung 0 and DOWN once it last
+// touched rung nt-1 (NONE before either); it travels with the state on every swap, and a DOWN replica that arrives at
+// rung 0 completes a round trip.  Counters: proposed [7] | accepted [7] (pair i, i+1, i = the initiator's rung) |
+// up [8] | down [8] (chains at rung i by label, every RMN_CP_DIAG_EVERY-th step after its swaps) | round trips [1].
+enum : uint8_t { CP_DIR_NONE = 0, CP_DIR_UP = 1, CP_DIR_DOWN = 2 };
+// in the kernel's shared slot of a group the label sits beside two flags of the group itself, which stay when the label moves
+constexpr int CP_DIR_MASK = 3, CP_RUNG_FIRST = 4, CP_RUNG_LAST = 8;
+constexpr int CP_SW_PROP = 0, CP_SW_ACC = 7, CP_SW_UP = 14, CP_SW_DOWN = 22, CP_SW_RT = 30, CP_SWAP_COUNTERS = 31;
+// the per-group counters of the kernel: swaps it initiated / took as initiator, round trips completed at it (rung 0),
+// samples of its label
+constexpr int CP_G_PROP = 0, CP_G_ACC = 1, CP_G_RT = 2, CP_G_UP = 3, CP_G_DOWN = 4, CP_G_COUNTERS = 5;
 
 // Posterior summaries (rmn_sampler_cp_set_summary), given only to the cp_summary kernels.  After every step s with
 // s % every == 0 each live chain's state adds, with i_j = #{g : xg[g] <= cpx[j]} and the prediction on the grid
@@ -446,6 +459,18 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
     const int g = threadIdx.x / GL;
     __shared__ int64_t s_chain[128 / GL];             // the chain the group writes back at the end, -1: none
     s_chain[g] = live ? c : -1;
+    // tempered: the label of the replica the group holds (dead slots and idle rungs: NONE, so they never count) and the
+    // group's swap counters (CP_G_*).  A group keeps its rung for the launch, so lane 0 counts in its own slots with plain
+    // adds -- no atomics in the T loop (a 64-bit shared atomic is a compare-and-swap loop) -- and the block adds them up
+    // by rung at the end.
+    __shared__ uint8_t s_dir[TEMPER ? 128 / GL : 1];
+    __shared__ unsigned long long s_sw[TEMPER ? CP_G_COUNTERS : 1][TEMPER ? 128 / GL : 1];
+    if constexpr (TEMPER) {
+        s_dir[g] = live ? (__ldcg(tp->dir + c) | ((ti == 0) ? CP_RUNG_FIRST : 0) | ((ti == tp->nt - 1) ? CP_RUNG_LAST : 0))
+                        : CP_DIR_NONE;
+#pragma unroll
+        for (int q = 0; q < CP_G_COUNTERS; ++q) s_sw[q][g] = 0;
+    }
     {
         double cx[EPL], cv[EPL];
         int bu[EPL];
@@ -777,6 +802,22 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
                 const double lp_ji_prev = __shfl_up_sync(FULL, lp_ji, GL);
                 const bool take = is_init ? sw : (is_part && sw_prev);
                 const double lp_o = is_init ? lp_ij : lp_ji_prev;
+                // swap statistics.  The labels move by shuffle: every lane has read its own group's label before any
+                // lane leaves the shuffle, so the new one can be written at once, and nothing of this stays live across
+                // the exchange of the rows below
+                {
+                    const int dl = s_dir[g];
+                    const int dd = __shfl_down_sync(FULL, dl, GL), du = __shfl_up_sync(FULL, dl, GL);
+                    const int din = (is_init ? dd : du) & CP_DIR_MASK;    // the partner's replica, as it arrives here
+                    if (lane == 0) {
+                        if (is_init) s_sw[CP_G_PROP][g] += 1;
+                        if (sw) s_sw[CP_G_ACC][g] += 1;
+                        if (take && (dl & CP_RUNG_FIRST) && din == CP_DIR_DOWN) s_sw[CP_G_RT][g] += 1;   // back at rung 0
+                    }
+                    if (take)
+                        s_dir[g] = (dl & ~CP_DIR_MASK) |
+                                   ((dl & CP_RUNG_FIRST) ? CP_DIR_UP : ((dl & CP_RUNG_LAST) ? CP_DIR_DOWN : din));
+                }
                 const int tq = go * GL + lane;                // the partner's slots (its own for a non-participant)
                 double ox[EPL], ov[EPL];
                 int ob[EPL];
@@ -803,6 +844,10 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
 
         if ((step % RMN_CP_DIAG_EVERY) == 0) {              // thinned accumulation (warp-uniform)
             __syncwarp();                                   // the rows as the other lanes accepted them
+            if constexpr (TEMPER) {                         // the flow histogram, after this step's swaps
+                const int d = s_dir[g] & CP_DIR_MASK;
+                if (lane == 0 && d != CP_DIR_NONE) s_sw[(d == CP_DIR_UP) ? CP_G_UP : CP_G_DOWN][g] += 1;
+            }
             const int kd = __reduce_max_sync(FULL, k);      // (an accepted birth may have raised the extent)
             double f[NS];
 #pragma unroll
@@ -869,6 +914,7 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
             st.lp[c] = lp;
             st.dacc[c] = __ldcg(st.dacc + c) + s_nacc[threadIdx.x];
             st.dovf[c] = __ldcg(st.dovf + c) + s_novf[threadIdx.x];
+            if constexpr (TEMPER) tp->dir[c] = s_dir[g] & CP_DIR_MASK;
         }
 #pragma unroll
         for (int s = 0; s < NS; ++s) {
@@ -882,9 +928,27 @@ __device__ __forceinline__ void cp_block(const CPParams& P, const double* __rest
     if constexpr (SUMMARY) {
         __syncthreads();                                // every warp's last sample is in the shared counters
         const int n1 = LANES, n2 = LANES + sp->G + 1;
-        for (int i = threadIdx.x; i < summary_counters(sp->G, sp->H); i += blockDim.x) {
+        // tempered: the block size as the literal it always is (the slots above are sized for 128 threads), so that
+        // blockDim.x is not held across the T loop -- at 128 registers the summary kernel would spill it
+        for (int i = threadIdx.x; i < summary_counters(sp->G, sp->H); i += (TEMPER ? 128u : blockDim.x)) {
             const unsigned long long v = ssum[i];
             if (v) atomicAdd((i < n1) ? sp->khist + i : ((i < n2) ? sp->cpxhist + (i - n1) : sp->D + (i - n2)), v);
+        }
+    }
+    if constexpr (TEMPER) {
+        __syncthreads();                                // every group's last count is in its slots
+        // thread j adds up counter j of CPTemper::swaps over the block's groups of its rung (group g is rung g & (S-1):
+        // a block holds whole ladder slots)
+        const int j = threadIdx.x;
+        if (j < CP_SWAP_COUNTERS) {
+            const int q = (j < CP_SW_ACC) ? CP_G_PROP : (j < CP_SW_UP) ? CP_G_ACC : (j < CP_SW_DOWN) ? CP_G_UP
+                        : (j < CP_SW_RT) ? CP_G_DOWN : CP_G_RT;
+            const int r = (j < CP_SW_ACC) ? j : (j < CP_SW_UP) ? j - CP_SW_ACC : (j < CP_SW_DOWN) ? j - CP_SW_UP
+                        : (j < CP_SW_RT) ? j - CP_SW_DOWN : 0;
+            unsigned long long v = 0;
+            if (r < tp->nt)
+                for (int gg = r; gg < 128 / GL; gg += tp->S) v += s_sw[q][gg];
+            if (v) atomicAdd(tp->swaps + j, v);
         }
     }
 }
@@ -1083,7 +1147,7 @@ cp_tempered_summary_kernel(const __grid_constant__ CPParams P, const __grid_cons
 }
 
 // evaluate n states given in the canonical layout (pointwise parity entry + set_state); tempered (tp != nullptr): the
-// carried log-posterior combine(log_prior, betas[c % nt] * log_likelihood)
+// carried log-posterior combine(log_prior, betas[c % nt] * log_likelihood), and the replica labels are initialised
 template <bool TEMPER>
 __device__ __forceinline__ void cp_eval_body(const CPParams& P, const double* __restrict__ gdata, int which,
                                              int64_t n, const int32_t* __restrict__ kin, const double* __restrict__ cpx,
@@ -1110,7 +1174,14 @@ __device__ __forceinline__ void cp_eval_body(const CPParams& P, const double* __
         const double lpr = cp_assemble(P, k, cp_ss_over_s2(ss, sig[c]), vt, lg, sig[c], ls2, 2);
         v = combine_logpost(lpr, __dmul_rn(tp->betas[c % tp->nt], v));
     }
-    if (live && lane == 0) out[c] = v;
+    if (live && lane == 0) {
+        out[c] = v;
+        // set_state starts the replica walk: the replica at rung 0 moves up, the one at rung nt-1 down
+        if constexpr (TEMPER) {
+            const int i = (int)(c % tp->nt);
+            tp->dir[c] = (i == 0) ? CP_DIR_UP : ((i == tp->nt - 1) ? CP_DIR_DOWN : CP_DIR_NONE);
+        }
+    }
 }
 
 __global__ void __launch_bounds__(128)
@@ -1207,9 +1278,12 @@ struct ChangepointSampler : SamplerImpl {
     }
     size_t workspace_bytes() const override {
         const size_t K = (size_t)s->K;
+        // the replica labels of tempering (one byte per chain) for every sampler: the size is asked before
+        // rmn_sampler_set_tempering
         return align256(K * 4) + 2 * align256(K * LANES * 8) + 4 * align256(K * 8) +
-               2 * align256(RMN_CP_NDIAG * K * 8) + 256;
+               2 * align256(RMN_CP_NDIAG * K * 8) + align256(K) + 256;
     }
+    uint8_t* d_dir = nullptr;       // [K] replica labels (CPTemper::dir), in the workspace
     int bind(void* ws) override {
         const size_t K = (size_t)s->K;
         char* p = (char*)ws;
@@ -1222,6 +1296,7 @@ struct ChangepointSampler : SamplerImpl {
         st.dovf = (long long*)p; p += align256(K * 8);
         st.S1 = (double*)p; p += align256(RMN_CP_NDIAG * K * 8);
         st.S2 = (double*)p; p += align256(RMN_CP_NDIAG * K * 8);
+        d_dir = (uint8_t*)p; p += align256(K);
         RMN_CUDA(cudaMemset(ws, 0, workspace_bytes()));
         if (use_smem) {
             RMN_CUDA(set_smem_attr<4>());
@@ -1286,7 +1361,37 @@ struct ChangepointSampler : SamplerImpl {
         }
         t.nt = nt; t.pswap = pswap; t.S = 1;
         while (t.S < nt) t.S *= 2;
+        if (!d_swaps && cudaMalloc(&d_swaps, CP_SWAP_COUNTERS * 8) != cudaSuccess) {
+            d_swaps = nullptr;
+            rmn_set_error("set_tempering: device allocation failed");
+            return RMN_ERR_CUDA;
+        }
+        RMN_CUDA(cudaMemset(d_swaps, 0, CP_SWAP_COUNTERS * 8));
+        // the replica walk starts here (rung 0 UP, rung nt-1 DOWN), and again at every set_state (cp_eval_tempered_kernel)
+        std::vector<uint8_t> lab((size_t)s->K);
+        for (int64_t c = 0; c < s->K; ++c)
+            lab[c] = (c % nt == 0) ? CP_DIR_UP : ((c % nt == nt - 1) ? CP_DIR_DOWN : CP_DIR_NONE);
+        RMN_CUDA(cudaMemcpy(d_dir, lab.data(), lab.size(), cudaMemcpyHostToDevice));
+        t.dir = d_dir; t.swaps = d_swaps;
         tp = t; tempered = true;
+        return RMN_OK;
+    }
+    unsigned long long* d_swaps = nullptr;      // the swap statistics (CPTemper::swaps), owned by the handle
+    int cp_get_swap_stats(int64_t* d_proposed, int64_t* d_accepted, int64_t* d_up, int64_t* d_down,
+                          int64_t* d_round_trips, cudaStream_t stream) override {
+        if (!tempered) {
+            rmn_set_error("swap statistics are counted for tempered changepoint samplers only (rmn_sampler_set_tempering)");
+            return RMN_ERR_UNSUPPORTED;
+        }
+        const int nt = tp.nt;
+        auto copy = [&](int64_t* dst, int at, int n) {
+            return dst ? cudaMemcpyAsync(dst, d_swaps + at, (size_t)n * 8, cudaMemcpyDeviceToDevice, stream) : cudaSuccess;
+        };
+        RMN_CUDA(copy(d_proposed, CP_SW_PROP, nt - 1));
+        RMN_CUDA(copy(d_accepted, CP_SW_ACC, nt - 1));
+        RMN_CUDA(copy(d_up, CP_SW_UP, nt));
+        RMN_CUDA(copy(d_down, CP_SW_DOWN, nt));
+        RMN_CUDA(copy(d_round_trips, CP_SW_RT, 1));
         return RMN_OK;
     }
 
@@ -1330,6 +1435,7 @@ struct ChangepointSampler : SamplerImpl {
     int force_guard = 0;            // RMN_CP_GUARD=1: per-chain schedules through the guarded instantiation (A/B)
     ~ChangepointSampler() override {
         if (d_done) cudaFree(d_done);
+        if (d_swaps) cudaFree(d_swaps);
         free_summary();
     }
     bool last_sliced = false;       // which kernel the last plain launch used (the timer label is corrected after the launch)
@@ -1611,6 +1717,8 @@ struct ChangepointSampler : SamplerImpl {
             RMN_CUDA(cudaMemsetAsync(sum.khist, 0, sum_count_bytes(), stream));
             sum_samples = 0;
         }
+        // the swap counts too; the replica labels are state of the walk and stay, so a trip in progress still completes
+        if (tempered) RMN_CUDA(cudaMemsetAsync(d_swaps, 0, CP_SWAP_COUNTERS * 8, stream));
         return RMN_OK;
     }
     int chain_sums(const double** S1, const double** S2, int64_t* n) override {

@@ -287,6 +287,7 @@ struct SamplerImpl {
     virtual int cp_set_summary(int, const double*, double, double, int, int64_t) { return unsupported("posterior summaries (changepoint samplers only)"); }
     virtual int cp_set_rung_summary(int, int, const double*, double, double, int, int64_t) { return unsupported("rung posterior summaries (tempered changepoint samplers only)"); }
     virtual int cp_get_summary(int64_t*, int64_t*, int64_t*, int64_t*, cudaStream_t) { return unsupported("posterior summaries (changepoint samplers only)"); }
+    virtual int cp_get_swap_stats(int64_t*, int64_t*, int64_t*, int64_t*, int64_t*, cudaStream_t) { return unsupported("swap statistics (tempered changepoint samplers only)"); }
     // raw per-chain diagnostics sums S1, S2 [nd][K] (chain fastest) and the number of samples behind them
     virtual int chain_sums(const double** S1, const double** S2, int64_t* nsamples) { return unsupported("per-chain moments"); }
     virtual int diag_dim() const = 0;

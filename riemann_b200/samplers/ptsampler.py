@@ -24,6 +24,8 @@ The reference shares ONE proposal object between all temperatures (:81), so only
 sense; the device engine enforces that (MetropolisRandomWalk, pCN; Gaussian models of any dimension, logistic model;
 ChangepointRegression1DProp on the changepoint model).
 """
+import ctypes as C
+
 import numpy as np
 
 from .. import _lib
@@ -71,6 +73,36 @@ class _TemperatureView(object):
     def current_state(self):
         th, lp = self._pt._history_of(self._i)
         return th[-1], lp[-1]
+
+
+class SwapStatistics(object):
+    """Swap statistics of the changepoint tempering ladders since the last reset (PTSampler.swap_statistics), pooled
+    over the ladders: int64 counts and the rates derived from them.
+
+    proposed[i], accepted[i]  (Nt-1,)  swaps rung i initiated with rung i+1 / swaps taken
+    acceptance                (Nt-1,)  accepted / proposed (nan where nothing was proposed)
+    up[i], down[i]            (Nt,)    at every step s with s % 16 == 0 (the diagnostics' cadence, after the step's
+                                       swaps), chains at rung i whose replica last touched rung 0 / rung Nt-1
+    up_fraction               (Nt,)    up / (up + down) (nan where neither): the fraction of replicas moving up, whose
+                                       steep drops show where the ladder needs another temperature (Katzgraber et
+                                       al. 2006); 1 at rung 0 and 0 at rung Nt-1 by construction
+    round_trips                        replicas that went from rung 0 to rung Nt-1 and back to rung 0
+    ladders, steps                     the ladders counted and the PT steps per chain since the reset, so that
+                                       round_trips / (ladders * steps) is the round-trip rate per ladder-step
+    """
+
+    def __init__(self, proposed, accepted, up, down, round_trips, ladders, steps):
+        self.proposed, self.accepted = proposed, accepted
+        self.up, self.down = up, down
+        self.round_trips, self.ladders, self.steps = int(round_trips), int(ladders), int(steps)
+        self.acceptance = np.where(proposed > 0, accepted / np.maximum(proposed, 1), np.nan)
+        n = up + down
+        self.up_fraction = np.where(n > 0, up / np.maximum(n, 1), np.nan)
+
+    def __repr__(self):
+        return "SwapStatistics(acceptance={}, round_trips={}, up_fraction={}, ladders={}, steps={})".format(
+            np.round(self.acceptance, 4).tolist(), self.round_trips, np.round(self.up_fraction, 4).tolist(),
+            self.ladders, self.steps)
 
 
 class PTSampler(object):
@@ -175,8 +207,37 @@ class PTSampler(object):
         return [s.current_state() for s in self.samplers]
 
     def reset_diagnostics(self):
-        """Zero the device accumulators of every rung: the diagnostics and the posterior-summary counts."""
+        """Zero the device accumulators of every rung: the diagnostics, the posterior-summary counts and, on the
+        changepoint model, the swap counts of `swap_statistics` (the replicas' directions stay, so a round trip in
+        progress still completes)."""
         self._sampler.reset_diagnostics()
+
+    # ------------------------------------------------------------------ swap statistics (changepoint model)
+    def swap_statistics(self, allreduce=True):
+        """
+        How the ladders mix since the last reset, counted in the tempered kernel (rmn_sampler_cp_get_swap_stats), as a
+        SwapStatistics: per pair of neighbouring rungs the swaps proposed and accepted, the replicas' round trips
+        from rung 0 to rung Nt-1 and back, and per rung the up / down flow histogram.  A replica's direction travels
+        with its state; set_state starts the walk (rung 0 up, rung Nt-1 down).  With torch.distributed initialised
+        the int64 counts are summed over the ranks (their ladders are disjoint).  Changepoint model only; the chains
+        are unchanged by the counting.
+        """
+        if not self._is_cp:
+            raise ParameterError("swap statistics are counted on the changepoint model only")
+        torch, nt = self._sampler._torch, self.Nt
+        # [ladders | proposed (nt-1) | accepted (nt-1) | up (nt) | down (nt) | round trips]
+        buf = torch.zeros(1 + 2 * (nt - 1) + 2 * nt + 1, dtype=torch.int64, device="cuda")
+        at = lambda i: C.c_void_p(buf.data_ptr() + 8 * i)
+        _lib.check(_lib.load().rmn_sampler_cp_get_swap_stats(
+            self._sampler._handle, at(1), at(nt), at(2 * nt - 1), at(3 * nt - 1), at(4 * nt - 1), _lib.stream_ptr()))
+        buf[0] = self.K
+        steps = int(self._sampler.diagnostics_block()[4].item())       # PT steps per chain since the reset
+        if allreduce:
+            from ..distributed import reduce_counts
+            buf = reduce_counts(buf)
+        c = buf.cpu().numpy()
+        return SwapStatistics(c[1:nt], c[nt:2 * nt - 1], c[2 * nt - 1:3 * nt - 1], c[3 * nt - 1:4 * nt - 1],
+                              c[4 * nt - 1], c[0], steps)
 
     # ------------------------------------------------------------------ posterior summaries (changepoint model)
     def set_posterior_summary(self, grid, value_range=None, value_bins=128, every=16, rung=0):
@@ -224,7 +285,9 @@ class PTSampler(object):
         per-chain moments (`Sampler.chain_moments`), rank-local (`allreduce` is accepted for interface symmetry:
         ladders on other ranks are independent replicas, combine their summaries on the host if needed).
         `accept_rate` is that of the flat engine -- accepted within-chain moves per chain-step over all temperatures,
-        a swap step counting as no move -- and is reported as `accept_rate_all_rungs`; `swap_fraction` = Pswap."""
+        a swap step counting as no move -- and is reported as `accept_rate_all_rungs`; `swap_fraction` = Pswap.
+        On the changepoint model `swap_acceptance` is the accepted fraction of the swaps proposed between rung i and
+        i+1 (`swap_statistics`)."""
         from ..distributed import summarize_block
         flat = self._sampler.diagnostics(allreduce=False)
         m, v = self._sampler.chain_moments()                      # [nd, K * Nt], chain fastest
@@ -240,4 +303,6 @@ class PTSampler(object):
         out["accept_rate_all_rungs"] = flat["accept_rate"]
         out["swap_fraction"] = float(self.Pswap)
         out["temperatures"] = self.Nt
+        if self._is_cp:                                           # per pair of neighbouring rungs, rank-local like the rest
+            out["swap_acceptance"] = self.swap_statistics(allreduce=False).acceptance
         return out

@@ -5,7 +5,9 @@ Prints the card's name, power limit and max SM clock, then:
     8,192 ladders x 8; CUDA events around the kernel launch, a warm-up first, every timed run >= 1 s, 3 runs per
     configuration alternated.  Chain-steps/s over all rungs and beta = 1 chain-steps/s.
   * mixing: 512 ladders x 5 against 512 untempered chains, tau of k and sigma at rung 0 from thinned traces
-    (riemann_b200.diagnostics.integrated_time_chains), ESS per beta = 1 chain-step and per second.
+    (riemann_b200.diagnostics.integrated_time_chains), ESS per beta = 1 chain-step and per second; for the ladders
+    also the swap statistics after the burn-in (PTSampler.swap_statistics): acceptance per pair of neighbouring
+    rungs, round trips per ladder per 1,000 steps and the up-moving fraction per rung.
 
     python scripts/bench_cp_tempering.py [--runs 3] [--min-seconds 1.0]
 """
@@ -90,6 +92,7 @@ def mixing(dm, dp, th0, burn=6000, T=40000, thin=40):
     for kind in (("plain", 512), ("pt", 512, 5)):
         obj, flat, beta1 = make(kind, dm, dp, th0, seed=3)
         flat.run(burn, trace=False)
+        flat.reset_diagnostics()                     # the swap statistics cover the 2 T steps after the burn-in
         import time
         import torch
         torch.cuda.synchronize()
@@ -104,11 +107,18 @@ def mixing(dm, dp, th0, burn=6000, T=40000, thin=40):
         sig = tr.sig[1:, ::nt]
         tau = integrated_time_chains(np.stack([k, sig], axis=2)) * thin     # in MH steps
         ess_per_step = 1.0 / tau                     # per beta = 1 chain-step
-        out.append(dict(config="untempered" if kind[0] == "plain" else "tempered x {}".format(nt),
-                        tau_k=float(tau[0]), tau_sig=float(tau[1]),
-                        ess_per_beta1_chain_step=[float(v) for v in ess_per_step],
-                        seconds_for_T=dt_plain,
-                        ess_per_s=[float(beta1 * T / dt_plain / t) for t in tau]))
+        rec = dict(config="untempered" if kind[0] == "plain" else "tempered x {}".format(nt),
+                   tau_k=float(tau[0]), tau_sig=float(tau[1]),
+                   ess_per_beta1_chain_step=[float(v) for v in ess_per_step],
+                   seconds_for_T=dt_plain,
+                   ess_per_s=[float(beta1 * T / dt_plain / t) for t in tau])
+        if kind[0] == "pt":
+            sw = obj.swap_statistics(allreduce=False)
+            rec.update(swap_steps=sw.steps, swap_acceptance=[float(v) for v in sw.acceptance],
+                       round_trips=sw.round_trips,
+                       round_trips_per_ladder_per_1000_steps=1000.0 * sw.round_trips / (sw.ladders * sw.steps),
+                       up_fraction=[float(v) for v in sw.up_fraction])
+        out.append(rec)
     return out
 
 
